@@ -323,6 +323,32 @@ def synthetic_values_device(torch, cols, n, device, col0=0):
     return torch.where(ge, z + ((1 << 32) - 1), z).contiguous()
 
 
+DUMP_SEED, DUMP_BYTES = 0x706C6F6E6B7932, 32 << 20
+
+
+def u64_halves(a):
+    """u64 -> float64 [..., 2] = (low 32 bits, high 32 bits): exact, which a u64 -> float cast of a field element is not."""
+    a = np.asarray(a).view(np.uint64)
+    return np.stack([a & np.uint64(0xFFFFFFFF), a >> np.uint64(32)], axis=-1).astype(np.float64)
+
+
+def dump_outputs(out_dir, cap_host, coeffs_dev):
+    """What the last timed step handed its caller, as .npy files: the whole cap and, when the step returns coefficients
+    (1.13 GB at the default shape), every coefficient column at a fixed, seeded sample of rows, with those row indices."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "cap.npy"), u64_halves(cap_host))
+    if coeffs_dev is None:
+        return
+    cols, n = coeffs_dev.shape
+    k = max(1, min(n, DUMP_BYTES // (16 * cols)))
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=k, replace=False))
+    sample = coeffs_dev.index_select(1, torch.from_numpy(rows).to(coeffs_dev.device)).cpu().numpy()
+    np.save(os.path.join(out_dir, "coeffs_sample.npy"), u64_halves(sample))
+    np.save(os.path.join(out_dir, "coeffs_sample_rows.npy"), rows.astype(np.float64))
+
+
 _RESULT_FD = None
 
 
@@ -361,7 +387,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-proof-trace", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float64; each u64 field element as its "
+                         "low and high 32 bits along the last axis): the cap and a seeded sample of the coefficients")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -473,6 +504,8 @@ def main():
     ms_per_step = dev_ms / args.steps
     value = cells * args.steps / (dev_ms * 1e-3)
     cap_host = cap.cpu().numpy().view(np.uint64)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, cap_host, coeffs_dev if world == 1 else None)
 
     # ---- e2e: HOST (pinned) buffers through the same C-ABI call -------------------------------------
     e2e = None
