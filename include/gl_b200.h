@@ -409,6 +409,26 @@ int gl_quotient_polys(gl_ctx *ctx, const gl_circuit *circuit, const gl_gate *gat
                       const uint64_t *public_inputs_hash, const uint64_t *betas, const uint64_t *gammas,
                       const uint64_t *alphas, uint64_t *chunks_out, int space);
 
+/* ---- plonky2::plonk::prover all_wires_permutation_partial_products / wires_permutation_partial_products_and_zs ----------
+ * (SURVEY 3.2 step 5), on the resident oracles; reached from every data.prove(pw).  Reads degree_bits, num_wires,
+ * num_routed_wires (R), num_constants, num_challenges (nch <= 4) and quotient_degree_factor (deg, a power of two) of
+ * `circuit`.  The routed wire values (columns [0, R) of `wires`) and the sigma values (columns [num_constants,
+ * num_constants + R) of `constants_sigmas`) are recovered on the device from the coefficients the two commits hold (commits
+ * of from_values or from_coeffs, blinded or not; unsharded, same degree, nch * ceil(R / deg) <= 64).  k_is [R], betas /
+ * gammas [nch]: host.
+ * zs_partial_products_out [nch * ceil(R / deg)][2^degree_bits] in `space`: values on the subgroup, canonical, laid out as
+ * the prover commits them (Z_0 .. Z_{nch-1}, then the ceil(R / deg) - 1 partial products of challenge 0, 1, ..) -- what
+ * gl_quotient_polys reads; a GL_DEVICE buffer goes straight into gl_commit_from_values(.., GL_DEVICE).
+ * grand_products_out [nch] (host, may be NULL): per challenge the product of the row ratios over all rows, 1 exactly when
+ * the witness satisfies every copy constraint.  A product other than 1 is not an error: the call returns GL_OK with every
+ * column written, as the prover does not panic there (the proof is simply invalid).  This is the one deliberate
+ * difference from the CPU restatement glo_permutation_zs (oracle/gl_oracle.c), which stops at the first challenge whose
+ * product is not 1 and fails.  A zero denominator
+ * wire + beta * sigma + gamma at some row returns GL_E_ARG (upstream's batch_multiplicative_inverse panics). */
+int gl_permutation_zs(gl_ctx *ctx, const gl_circuit *circuit, const uint64_t *k_is, gl_commit *constants_sigmas,
+                      gl_commit *wires, const uint64_t *betas, const uint64_t *gammas, uint64_t *zs_partial_products_out,
+                      int space, uint64_t *grand_products_out);
+
 /* ---- P10: fri_proof_of_work ------------------------------------------------------------------- */
 /* Smallest w >= 0 such that permute(state with state[input_pos] = w)[7] (the last rate lane, as
  * `duplex_state.squeeze().last()`) has >= min_leading_zeros leading zero bits.  Upstream's rayon

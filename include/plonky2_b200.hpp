@@ -769,6 +769,31 @@ inline std::vector<std::vector<F>> compute_quotient_polys(const Context& c, cons
     return out;
 }
 
+// plonky2::plonk::prover all_wires_permutation_partial_products on the two resident commits (gl_permutation_zs): returns
+// the num_challenges * ceil(num_routed_wires / quotient_degree_factor) columns of values on the subgroup (Z_0 .. Z_{nch-1},
+// then the partial products of challenge 0, 1, ..) and, per challenge, the product of the row ratios over all rows
+// (1 exactly when the witness satisfies every copy constraint).
+struct PermutationZs {
+    std::vector<std::vector<F>> zs_partial_products;
+    std::vector<F> grand_products;
+};
+inline PermutationZs all_wires_permutation_partial_products(const Context& c, const gl_circuit& circuit, const std::vector<F>& k_is,
+                                                            const PolynomialBatch& constants_sigmas, const PolynomialBatch& wires,
+                                                            const std::vector<F>& betas, const std::vector<F>& gammas) {
+    if (k_is.size() < circuit.num_routed_wires || betas.size() < circuit.num_challenges || gammas.size() < circuit.num_challenges)
+        throw Panic(GL_E_ARG, "all_wires_permutation_partial_products: fewer k_is / betas / gammas than the circuit needs");
+    const uint32_t deg = circuit.quotient_degree_factor ? circuit.quotient_degree_factor : 1;
+    const size_t n = (size_t)1 << circuit.degree_bits;
+    const size_t cols = (size_t)circuit.num_challenges * ((circuit.num_routed_wires + deg - 1) / deg);
+    std::vector<F> flat(cols * n);
+    PermutationZs out;
+    out.grand_products.assign(circuit.num_challenges, 0);
+    c.check(gl_permutation_zs(c.raw(), &circuit, k_is.data(), constants_sigmas.raw_handle(), wires.raw_handle(), betas.data(),
+                              gammas.data(), flat.data(), GL_HOST, out.grand_products.data()));
+    for (size_t i = 0; i < cols; i++) out.zs_partial_products.emplace_back(flat.begin() + i * n, flat.begin() + (i + 1) * n);
+    return out;
+}
+
 // One commit sharded over the GPUs of a box (gl_group_*: NCCL behind the C ABI); this process holds every rank.
 class Group {
    public:

@@ -8,7 +8,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libgl_b200.so")
-SOURCES = ["gl_b200.cu", "ntt_kernels.cu", "ntt_tma.cu", "hash_kernels.cu", "fri_kernels.cu", "host_staging.cu", "quotient_kernels.cu"]
+SOURCES = ["gl_b200.cu", "ntt_kernels.cu", "ntt_tma.cu", "hash_kernels.cu", "fri_kernels.cu", "host_staging.cu", "quotient_kernels.cu",
+           "permutation_kernels.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -32,6 +32,7 @@
 #include "hash_kernels.h"
 #include "host_staging.h"
 #include "ntt_kernels.h"
+#include "permutation_kernels.h"
 #include "poseidon_constants.h"
 #include "quotient_kernels.h"
 #include "smt_kernels.h"
@@ -2271,6 +2272,90 @@ extern "C" int gl_quotient_polys(gl_ctx* ctx, const gl_circuit* cd, const gl_gat
     TRY(transform_natural(ctx, (u64*)d_vals, lg_n + qdb, nch, true, nullptr, post));
     TRY(copy_out(ctx, chunks_out, d_vals, (size_t)nch * lde_size * 8, space));
     return finish(ctx);
+}
+
+// ------------------------------------------------------------------------------------------------
+// all_wires_permutation_partial_products: Z and the partial products, from the coefficients the two commits hold
+// ------------------------------------------------------------------------------------------------
+extern "C" int gl_permutation_zs(gl_ctx* ctx, const gl_circuit* cd, const uint64_t* k_is, gl_commit* constants_sigmas,
+                                 gl_commit* wires, const uint64_t* betas, const uint64_t* gammas,
+                                 uint64_t* zs_partial_products_out, int space, uint64_t* grand_products_out) {
+    if (!ctx) return GL_E_ARG;
+    if (!cd || !k_is || !constants_sigmas || !wires || !betas || !gammas || !zs_partial_products_out)
+        return fail(ctx, GL_E_ARG, "gl_permutation_zs: NULL argument");
+    if (space != GL_HOST && space != GL_DEVICE) return fail(ctx, GL_E_ARG, "gl_permutation_zs: bad space");
+    const uint32_t nch = cd->num_challenges, R = cd->num_routed_wires, deg = cd->quotient_degree_factor;
+    if (nch == 0 || nch > PERM_MAX_CHALLENGES || R == 0 || R > cd->num_wires || !is_pow2(deg))
+        return fail(ctx, GL_E_ARG, "gl_permutation_zs: unsupported circuit geometry");
+    const uint32_t chunks = (R + deg - 1) / deg;
+    if (nch * chunks > PERM_MAX_SLOTS)
+        return fail(ctx, GL_E_ARG, "gl_permutation_zs: num_challenges * ceil(num_routed_wires / quotient_degree_factor) > 64");
+    for (gl_commit* h : {constants_sigmas, wires}) {
+        if (h->ctx != ctx || !h->finished || !h->coeffs)
+            return fail(ctx, GL_E_STATE, "gl_permutation_zs: oracle is not a finished polynomial commit of this ctx");
+        if (h->shard_count != 1) return fail(ctx, GL_E_ARG, "gl_permutation_zs: sharded oracles are not supported");
+    }
+    if (constants_sigmas->c != cd->num_constants + R || wires->c != cd->num_wires)
+        return fail(ctx, GL_E_ARG, "gl_permutation_zs: column counts do not match the circuit description");
+    if (wires->log_n != constants_sigmas->log_n || wires->log_n != cd->degree_bits)
+        return fail(ctx, GL_E_ARG, "gl_permutation_zs: oracles of different degree");
+    Guard g(ctx);
+    const uint32_t lg_n = cd->degree_bits;
+    const u64 n = (u64)1 << lg_n;
+    const uint32_t nblocks = (uint32_t)((n + PERM_BLOCK - 1) / PERM_BLOCK);
+    // small device state (scratch slot 0): k_is [R] | CTA products [nch][nblocks] | grand products [4] | zero flag
+    std::vector<u64> kt(R);
+    for (uint32_t j = 0; j < R; j++) kt[j] = glh::canon(k_is[j]);
+    const size_t small_words = R + (size_t)nch * nblocks + PERM_MAX_CHALLENGES + 1;
+    void* d_small;
+    TRY(scratch_get(ctx, 0, small_words * 8, &d_small));
+    u64* d_k = (u64*)d_small;
+    u64* d_cta = d_k + R;
+    u64* d_grand = d_cta + (size_t)nch * nblocks;
+    unsigned* d_flag = (unsigned*)(d_grand + PERM_MAX_CHALLENGES);
+    CK(cudaMemcpyAsync(d_k, kt.data(), R * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemsetAsync(d_flag, 0, sizeof(unsigned), ctx->stream));
+    const u64* xtab;
+    TRY(pow_table(ctx, glh::root_of_unity(lg_n), &xtab));
+    void* d_out = zs_partial_products_out;
+    const size_t out_bytes = (size_t)nch * chunks * n * 8;
+    if (space == GL_HOST) TRY(scratch_get(ctx, 4, out_bytes, &d_out));
+    // the routed wire and sigma values: forward transforms of the coefficient columns (the salt of a blinded commit
+    // lives only in its leaves).  The transforms run through scratch slot 1.
+    const size_t rec_bytes = (size_t)2 * R * n * 8;
+    u64* d_rec;
+    TRY(dev_alloc(ctx, rec_bytes, &d_rec));
+    int rc = transform_natural(ctx, d_rec, lg_n, R, false, nullptr, nullptr, wires->coeffs);
+    if (rc == GL_OK)
+        rc = transform_natural(ctx, d_rec + (size_t)R * n, lg_n, R, false, nullptr, nullptr,
+                               constants_sigmas->coeffs + (size_t)cd->num_constants * n);
+    u64 grand[PERM_MAX_CHALLENGES];
+    unsigned zero_den = 0;
+    if (rc == GL_OK) {
+        perm_args a;
+        memset(&a, 0, sizeof a);
+        a.wires = d_rec; a.sigmas = d_rec + (size_t)R * n; a.k_is = d_k; a.xtab = xtab;
+        a.out = (u64*)d_out; a.cta = d_cta; a.grand = d_grand; a.zero_den = d_flag;
+        a.n = n; a.R = R; a.deg = deg; a.chunks = chunks; a.nch = nch; a.nblocks = nblocks;
+        for (uint32_t c = 0; c < nch; c++) { a.betas[c] = glh::canon(betas[c]); a.gammas[c] = glh::canon(gammas[c]); }
+        cudaError_t e = launch_permutation_zs(a, ctx->stream);
+        if (e != cudaSuccess) rc = cuda_fail(ctx, e, "launch_permutation_zs");
+    }
+    if (rc == GL_OK) {
+        cudaError_t e = cudaMemcpyAsync(grand, d_grand, nch * 8, cudaMemcpyDeviceToHost, ctx->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(&zero_den, d_flag, sizeof zero_den, cudaMemcpyDeviceToHost, ctx->stream);
+        if (e != cudaSuccess) rc = cuda_fail(ctx, e, "download grand products");
+    }
+    if (rc == GL_OK && space == GL_HOST) rc = copy_out(ctx, zs_partial_products_out, d_out, out_bytes, GL_HOST);
+    if (rc == GL_OK) rc = finish(ctx);
+    dev_release(ctx, d_rec, rec_bytes);
+    if (rc != GL_OK) return rc;
+    if (zero_den)
+        return fail(ctx, GL_E_ARG, "gl_permutation_zs: wire + beta * sigma + gamma is zero at some row "
+                                   "(batch_multiplicative_inverse of a zero denominator)");
+    if (grand_products_out)
+        for (uint32_t c = 0; c < nch; c++) grand_products_out[c] = grand[c];
+    return GL_OK;
 }
 
 extern "C" int gl_pow_grind(gl_ctx* ctx, const uint64_t state[12], uint32_t input_pos, uint32_t min_leading_zeros,

@@ -158,6 +158,23 @@ GL_D u64 gl_sub(u64 a, u64 b) {
 GL_D u64 gl_canon(u64 x) { return x >= GL_P ? x - GL_P : x; }
 GL_D u64 gl_neg(u64 a) { return gl_sub(0, a); }
 
+// a * b + c + d with ONE reduction: (2^64 - 1)^2 + 2 (2^64 - 1) = 2^128 - 1, so the sum fits 128 bits
+GL_D u64 gl_mad2(u64 a, u64 b, u64 c, u64 d) {
+    unsigned __int128 p = (unsigned __int128)a * b;
+    p += c;
+    p += d;
+    return gl_reduce128((u64)p, (u64)(p >> 64));
+}
+// base^e from the host's 3 x 1024 power table of base (e < 2^30)
+GL_D u64 gl_powtab(const u64* __restrict__ tab, u64 e) {
+    u64 r = __ldg(tab + (e & 1023));
+    if (e >> 10) {
+        r = gl_mul(r, __ldg(tab + 1024 + ((e >> 10) & 1023)));
+        if (e >> 20) r = gl_mul(r, __ldg(tab + 2048 + ((e >> 20) & 1023)));
+    }
+    return r;
+}
+
 GL_D u64 gl_pow(u64 a, u64 e) {
     u64 r = 1;
     while (e) {

@@ -35,16 +35,6 @@ unsigned quotient_gate_constraints(const gl_gate& g) {
 
 GL_D u64 q_inv(u64 a) { return gl_pow(a, GL_P - 2); }
 
-// base^e from a 3 x 1024 table (e < 2^30)
-GL_D u64 q_powtab(const u64* __restrict__ tab, u64 e) {
-    u64 r = __ldg(tab + (e & 1023));
-    if (e >> 10) {
-        r = gl_mul(r, __ldg(tab + 1024 + ((e >> 10) & 1023)));
-        if (e >> 20) r = gl_mul(r, __ldg(tab + 2048 + ((e >> 20) & 1023)));
-    }
-    return r;
-}
-
 // ---- 160-bit unreduced accumulators ---------------------------------------------------------------------------------------
 // The alpha-weighted sums of a gate's constraints and the binary / base-4 recompositions of its bit wires are sums of
 // hundreds of products: they are accumulated as plain integers (five 32-bit limbs, carry chains) and reduced mod p once,
@@ -70,13 +60,6 @@ GL_D void acc_horner(acc160& c, u64 v) {
         : "=r"(c.w0), "=r"(c.w1), "=r"(c.w2), "=r"(c.w3), "=r"(c.w4)
         : "r"(n0), "r"(n1), "r"(n2), "r"(n3), "r"(n4), "r"((u32)v), "r"((u32)(v >> 32)));
 }
-// a * b + c + d with ONE reduction: (2^64 - 1)^2 + 2 (2^64 - 1) = 2^128 - 1, so the sum fits 128 bits
-GL_D u64 q_mad2(u64 a, u64 b, u64 c, u64 d) {
-    unsigned __int128 p = (unsigned __int128)a * b;
-    p += c;
-    p += d;
-    return gl_reduce128((u64)p, (u64)(p >> 64));
-}
 // w0 + w1 phi + w2 phi^2 + w3 phi^3 + w4 phi^4, phi = 2^32: phi^2 = phi - 1, phi^3 = -1, phi^4 = -phi
 GL_D u64 acc_reduce(const acc160& c) {
     const u64 r = gl_reduce128(gl_pack(c.w0, c.w1), gl_pack(c.w2, c.w3));
@@ -90,7 +73,7 @@ __global__ void __launch_bounds__(Q_BLOCK) k_quotient(const quotient_args a) {
     const u64 i = a.lg_lde ? (__brevll(p) >> (64 - a.lg_lde)) : 0;      // natural index of this leaf
     const u64 i_next = (i + ((u64)1 << a.qdb)) & (lde_size - 1);
     const u64 p_next = a.lg_lde ? (__brevll(i_next) >> (64 - a.lg_lde)) : 0;
-    const u64 x = gl_mul(7, q_powtab(a.xtab, i));                       // shifted_x = coset_shift * w^i
+    const u64 x = gl_mul(7, gl_powtab(a.xtab, i));                       // shifted_x = coset_shift * w^i
     const unsigned nch = a.nch;
     const u64* __restrict__ W = a.wires + p;
     const u64* __restrict__ CS = a.cs + p;
@@ -119,8 +102,8 @@ __global__ void __launch_bounds__(Q_BLOCK) k_quotient(const quotient_args a) {
             for (unsigned j = q * a.deg; j < j1; j++) {
                 const u64 wv = W[(u64)j * a.w_ld];
                 const u64 sg = CS[(u64)(a.num_constants + j) * a.cs_ld];
-                num = gl_mul(num, q_mad2(bx, __ldg(a.k_is + j), wv, gamma));    // wire + beta * k_i * x + gamma
-                den = gl_mul(den, q_mad2(beta, sg, wv, gamma));                 // wire + beta * sigma + gamma
+                num = gl_mul(num, gl_mad2(bx, __ldg(a.k_is + j), wv, gamma));    // wire + beta * k_i * x + gamma
+                den = gl_mul(den, gl_mad2(beta, sg, wv, gamma));                 // wire + beta * sigma + gamma
             }
             const u64 next = q == a.chunks - 1 ? ZN[(u64)c * a.z_ld] : pp[(u64)q * a.z_ld];
             const u64 term = gl_sub(gl_mul(prev, num), gl_mul(next, den));

@@ -650,6 +650,35 @@ def compute_quotient_polys(circuit, gates, k_is, constants_sigmas: "PolynomialBa
     return out
 
 
+def permutation_zs(circuit, k_is, constants_sigmas: "PolynomialBatch", wires: "PolynomialBatch", betas, gammas, out=None,
+                   ctx=None):
+    """all_wires_permutation_partial_products (prover step 3): the Z and partial-product columns, values on the subgroup,
+    [num_challenges * ceil(num_routed_wires / quotient_degree_factor)][n] in the order the prover commits them, computed from
+    the coefficients the two resident commits hold.  circuit: the same tuple as compute_quotient_polys takes.  out: None (a
+    new numpy array), a numpy array, a torch CUDA tensor or a DeviceBuffer (the columns stay on the device and go straight
+    into PolynomialBatch.from_values).  Returns (zs, grand_products): grand_products[c] is 1 exactly when the witness
+    satisfies every copy constraint; a product other than 1 is returned, not raised."""
+    ctx = _ctx(ctx)
+    cd = N.Circuit(*[int(v) for v in circuit])
+    k, b, g = _h(k_is), _h(betas), _h(gammas)
+    nch = cd.num_challenges
+    if len(b) < nch or len(g) < nch:
+        raise GlPanic(N.GL_E_ARG, "permutation_zs: fewer betas / gammas than num_challenges")
+    if len(k) < cd.num_routed_wires:
+        raise GlPanic(N.GL_E_ARG, "permutation_zs: fewer k_is than num_routed_wires")
+    deg = max(cd.quotient_degree_factor, 1)
+    shape = (nch * -(-cd.num_routed_wires // deg), 1 << cd.degree_bits)
+    if out is None:
+        out = np.empty(shape, dtype=np.uint64)
+    o = _Buf(out, writable=True)
+    if o.nbytes < shape[0] * shape[1] * 8:
+        raise GlPanic(N.GL_E_ARG, "permutation_zs: output buffer too small")
+    grand = np.zeros(max(nch, 1), dtype=np.uint64)
+    ctx.check(ctx._lib.gl_permutation_zs(ctx._h, C.byref(cd), k.ctypes.data, constants_sigmas._h, wires._h, b.ctypes.data,
+                                         g.ctypes.data, o.ptr, o.space, grand.ctypes.data))
+    return out, grand[:nch]
+
+
 # ------------------------------------------------------------------------------------------------
 # gl_group: one commit sharded over several GPUs, NCCL behind the C ABI (SURVEY 8e)
 # ------------------------------------------------------------------------------------------------

@@ -109,6 +109,10 @@ extern "C" {
                              constants_sigmas: *mut gl_commit, wires: *mut gl_commit, zs_partial_products: *mut gl_commit,
                              public_inputs_hash: *const u64, betas: *const u64, gammas: *const u64, alphas: *const u64,
                              chunks_out: *mut u64, space: c_int) -> c_int;
+    // all_wires_permutation_partial_products on the resident oracles (plonk/prover.rs, before the Z commit)
+    pub fn gl_permutation_zs(ctx: *mut gl_ctx, circuit: *const gl_circuit, k_is: *const u64, constants_sigmas: *mut gl_commit,
+                             wires: *mut gl_commit, betas: *const u64, gammas: *const u64, zs_partial_products_out: *mut u64,
+                             space: c_int, grand_products_out: *mut u64) -> c_int;
     // N1 in one call: prove_openings + fri_proof with the transcript on the device; fork-version switches
     pub fn gl_ctx_set_compat(ctx: *mut gl_ctx, flags: u32) -> c_int;
     pub fn gl_fri_proof_words(prm: *const gl_fri_params, oracle_columns: *const u32, num_oracles: u32, degree_bits: u32,
