@@ -109,7 +109,31 @@ GL_D u64 gl_mul(u64 a, u64 b) {
     unsigned __int128 p = (unsigned __int128)a * b;
     return gl_reduce128((u64)p, (u64)(p >> 64));
 }
-GL_D u64 gl_sqr(u64 a) { return gl_mul(a, a); }
+// a^2 = l + 2^32 (m + m) + 2^64 h with l = a0^2, m = a0 a1, h = a1^2 (a = a0 + 2^32 a1): three wide products instead of
+// gl_mul's four; the cross product enters the carry chain twice instead of being shifted.  No partial sum exceeds a^2.
+GL_D u64 gl_sqr(u64 a) {
+    u32 r0, r1, r2, r3;
+    asm("{\n\t"
+        ".reg .u32 a0, a1, l1, m0, m1, h0, h1;\n\t"
+        ".reg .u64 l, m, h;\n\t"
+        "mov.b64 {a0, a1}, %4;\n\t"
+        "mul.wide.u32 l, a0, a0;\n\t"
+        "mul.wide.u32 m, a0, a1;\n\t"
+        "mul.wide.u32 h, a1, a1;\n\t"
+        "mov.b64 {%0, l1}, l;\n\t"
+        "mov.b64 {m0, m1}, m;\n\t"
+        "mov.b64 {h0, h1}, h;\n\t"
+        "add.cc.u32 %1, l1, m0;\n\t"
+        "addc.cc.u32 %2, h0, m1;\n\t"
+        "addc.u32 %3, h1, 0;\n\t"
+        "add.cc.u32 %1, %1, m0;\n\t"
+        "addc.cc.u32 %2, %2, m1;\n\t"
+        "addc.u32 %3, %3, 0;\n\t"
+        "}"
+        : "=&r"(r0), "=&r"(r1), "=&r"(r2), "=&r"(r3)
+        : "l"(a));
+    return gl_reduce128(gl_pack(r0, r1), gl_pack(r2, r3));
+}
 
 // a + b where b is canonical (< p): one wrap correction suffices
 GL_D u64 gl_add_c(u64 a, u64 b_canonical) {

@@ -24,12 +24,7 @@ int gl_poseidon_upload_constants(const u64* rc360) {
     static u64 split[(POSEIDON_ROUNDS + 1) * POSEIDON_WIDTH * 2];
     static u64 pk[(POSEIDON_PARTIAL / 2) * POSEIDON_WIDTH * 2];
     static const int circ[12] = {17, 15, 41, 16, 2, 28, 13, 13, 39, 18, 34, 20};
-#ifdef POSEIDON_SPLIT_SBOX
-    const bool signed_sbox = true;
-#else
-    const bool signed_sbox = false;
-#endif
-    poseidon_constants::linear_layer_tables(rc360, circ, 8, signed_sbox, split, pk);
+    poseidon_constants::linear_layer_tables(rc360, circ, 8, true, split, pk, POSEIDON_HANDOFF_BIAS);
     e = cudaMemcpyToSymbol(c_poseidon_rc_split, split, sizeof(split));
     if (e != cudaSuccess) return (int)e;
     return (int)cudaMemcpyToSymbol(c_poseidon_pair_k, pk, sizeof(pk));

@@ -8,7 +8,8 @@
 // B200 mapping (measured pipe rates: profiles/r1_pipe_peaks.json).  IMAD.WIDE.U32 issues at ~51
 // lanes/clk/SM and does not overlap with ALU work, so the two halves of a round go to different
 // pipes:
-//   * S-box x^7: four 64x64 products = IMAD.WIDE.U32 on the FMA-heavy pipe + shift-reduction on ALU.
+//   * S-box x^7: four 64x64 products (two of them squares of three 32x32 products each) = IMAD.WIDE.U32 on the
+//     FMA-heavy pipe + shift-reduction on ALU; the last product is handed to the linear layer unreduced.
 //   * MDS layer: on the FP64 pipe (B200 keeps full-rate DFMA).  A 32-bit half x of a lane is
 //     reinterpreted as the double with bit pattern (hi = 0, lo = x), i.e. the denormal x * 2^-1074.
 //     The circulant entries are <= 41 and each row sums to 264, so sum_i c_i * x_i < 2^42 stays below
@@ -36,39 +37,39 @@ __constant__ u64 c_poseidon_rc[POSEIDON_ROUNDS * POSEIDON_WIDTH];
 __constant__ double2 c_poseidon_rc_split[(POSEIDON_ROUNDS + 1) * POSEIDON_WIDTH];
 
 #ifdef __CUDACC__
-GL_D u64 poseidon_sbox(u64 x) {
-    u64 x2 = gl_sqr(x);
-    u64 x4 = gl_sqr(x2);
-    u64 x3 = gl_mul(x2, x);
-    return gl_mul(x3, x4);
-}
-
 GL_D double u32_as_denormal(u32 x) { return __hiloint2double(0, (int)x); }
 GL_D u64 double_bits(double d) { return (u64)__double_as_longlong(d); }
 
-#ifndef POSEIDON_NO_SPLIT_SBOX
-#define POSEIDON_SPLIT_SBOX 1
-#endif
-#ifdef POSEIDON_SPLIT_SBOX
-// x^7 handed to the FP64 linear layer without the last modular reduction: the 128-bit product x^3 * x^4 =
-// r0 + r1 phi + r2 phi^2 + r3 phi^3 (phi = 2^32, phi^2 = phi - 1, phi^3 = -1) is (r0 - r2 - r3) + (r1 + r2) phi, and
-// the two coefficients are formed by three exact FP64 additions on the limbs' denormal images: dl in (-2^33, 2^32),
-// dh in [0, 2^33).  The linear layers are exact on signed integers below 2^52; the constants they add carry an offset
-// that is a multiple of p and makes every sum positive again (POSEIDON_OFF_*), so the fold is unchanged.
+// x^7 handed to the FP64 linear layers without the last modular reduction.  The 128-bit product x^3 * x^4 =
+// r0 + r1 phi + r2 phi^2 + r3 phi^3 (phi = 2^32, phi^2 = phi - 1, phi^3 = -1 mod p) is (r0 - r2 - r3) + (r1 + r2) phi.  Both
+// coefficients are formed as 64-bit integers by carry chains (IADD3 / IADD3.X), and their bit patterns ARE the doubles the
+// layers read (integers below 2^52 are exact denormals, no move or FP64 add is needed):
+//   dl = r0 - r2 - r3 + POSEIDON_HANDOFF_BIAS in [2, 3 * 2^32),  dh = r1 + r2 in [0, 2^33).
+// The bias keeps dl non-negative; the layers' constant tables take it back out (poseidon_constants.h: linear_layer_tables),
+// so every accumulator the fold sees is the same integer as with the signed coefficient r0 - r2 - r3.
+#define POSEIDON_HANDOFF_BIAS (1ULL << 33)
 GL_D void poseidon_sbox_split(u64 x, double& dl, double& dh) {
     const u64 x2 = gl_sqr(x), x4 = gl_sqr(x2), x3 = gl_mul(x2, x);
     const unsigned __int128 p = (unsigned __int128)x3 * x4;
     const u64 lo = (u64)p, hi = (u64)(p >> 64);
-    const double r0 = u32_as_denormal((u32)lo), r1 = u32_as_denormal((u32)(lo >> 32));
-    const double r2 = u32_as_denormal((u32)hi), r3 = u32_as_denormal((u32)(hi >> 32));
-    dl = (r0 - r2) - r3;
-    dh = r1 + r2;
+    u32 l0, l1, h0, h1;
+    asm("{\n\t"
+        "sub.cc.u32 %0, %4, %6;\n\t"      // dl = (2 phi + r0) - r2 - r3, subtract family only
+        "subc.u32 %1, 2, 0;\n\t"
+        "sub.cc.u32 %0, %0, %7;\n\t"
+        "subc.u32 %1, %1, 0;\n\t"
+        "add.cc.u32 %2, %5, %6;\n\t"      // dh = r1 + r2
+        "addc.u32 %3, 0, 0;\n\t"
+        "}"
+        : "=&r"(l0), "=&r"(l1), "=&r"(h0), "=&r"(h1)
+        : "r"((u32)lo), "r"((u32)(lo >> 32)), "r"((u32)hi), "r"((u32)(hi >> 32)));
+    dl = __longlong_as_double((long long)gl_pack(l0, l1));
+    dh = __longlong_as_double((long long)gl_pack(h0, h1));
 }
-#endif
-// (the offsets live in the constant tables: poseidon_constants.h, linear_layer_tables(signed_sbox = true).  Exactness: every
-// operand is an integer multiple of 2^-1074, so FP64 sums and products are exact while they stay below 2^53: a full
-// round's layer sees |inputs| < 2^33 and peaks below 2^44; the fused pair's CIRC^2 form sees lane 0 in (-2^33, 2^32) and the
-// other lanes in [0, 2^32) and peaks below 2^49, its outputs landing in [0, 2^50) after the 2^48 offset.)
+// (exactness: every operand is an integer multiple of 2^-1074, so FP64 sums and products are exact while they stay below
+// 2^53 in magnitude.  A full round's layer sees inputs in [0, 3 * 2^32); the fused pair's CIRC^2 form sees lane 0 in
+// [0, 3 * 2^32) and the other lanes in [0, 2^32).  tests/test_poseidon_schedule_model_cpu.py bounds every intermediate
+// exactly: all stay below 2^51.)
 
 // MDS entries: M[r][j] = CIRC[(j - r) mod 12] + (r == j ? DIAG[r] : 0)
 __host__ __device__ constexpr int poseidon_mds_entry(int r, int j) {
@@ -87,23 +88,27 @@ __host__ __device__ constexpr int poseidon_pair_entry(int r, int j) {
 // (a = 4 + 2 * pair), split in 32-bit-half sums like c_poseidon_rc_split.
 __constant__ double2 c_poseidon_pair_k[(POSEIDON_PARTIAL / 2) * POSEIDON_WIDTH];
 
-GL_D u64 poseidon_fold(double al, double ah);
+// value = A + 2^32 B with A, B < 2^50 (integer bit patterns); bh = B >> 32 < 2^18, b0 = B mod 2^32.  2^64 = 2^32 - 1 (mod p):
+//   A + 2^32 B = (A - bh) + 2^32 (bh + b0)  (mod p),
+// one carry chain without a multiply.  A - bh does not borrow: the tables keep A >= 2^40 (their positive offsets).  The sum
+// is below 2^64 + 2^51, so it wraps at most once; the wrap c is folded back as c * (2^32 - 1) = c * 2^32 - c, which cannot
+// wrap again (the wrapped sum is below 2^51).
 GL_D u64 poseidon_fold(double al, double ah) {
-    // value = A + 2^32 * B with A, B < 2^50 (integer bit patterns).  2^64 = 2^32 - 1 (mod p):
-    //   t = A + (B >> 32) * (2^32 - 1)  (< 2^51, one IMAD.WIDE);  y = t + (B mod 2^32) * 2^32 wraps at most once
-    u64 A = double_bits(al), B = double_bits(ah);
-    u64 t = A + (u64)(u32)(B >> 32) * GL_EPS;
-    u32 t0 = (u32)t, t1 = (u32)(t >> 32), b0 = (u32)B, y0, y1;
+    const u64 A = double_bits(al), B = double_bits(ah);
+    u32 y0, y1;
     asm("{\n\t"
-        ".reg .u32 m;\n\t"
-        "add.cc.u32 %1, %3, %4;\n\t"
-        "addc.u32 m, 0, 0;\n\t"          // carry (add family only)
-        "neg.s32 m, m;\n\t"              // carry * (2^32 - 1)
-        "add.cc.u32 %0, %2, m;\n\t"
-        "addc.u32 %1, %1, 0;\n\t"
+        ".reg .u32 t, c;\n\t"
+        "add.u32 t, %3, %5;\n\t"          // A1 + bh < 2^19
+        "sub.cc.u32 %0, %2, %5;\n\t"      // A0 - bh
+        "subc.u32 t, t, 0;\n\t"
+        "add.cc.u32 %1, t, %4;\n\t"       // + b0: the wrap
+        "addc.u32 c, 0, 0;\n\t"
+        "add.u32 t, %1, c;\n\t"           // + c * 2^32 (no carry: after a wrap the high word is < 2^19)
+        "sub.cc.u32 %0, %0, c;\n\t"       // - c
+        "subc.u32 %1, t, 0;\n\t"
         "}"
         : "=&r"(y0), "=&r"(y1)
-        : "r"(t0), "r"(t1), "r"(b0));
+        : "r"((u32)A), "r"((u32)(A >> 32)), "r"((u32)B), "r"((u32)(B >> 32)));
     return gl_pack(y0, y1);
 }
 
@@ -170,13 +175,7 @@ GL_D void poseidon_full_round(u64 s[12], const double2* __restrict__ rc) {
     double dl[12], dh[12], yl[12], yh[12];
 #pragma unroll
     for (int j = 0; j < 12; j++) {
-#ifdef POSEIDON_SPLIT_SBOX
         poseidon_sbox_split(s[j], dl[j], dh[j]);
-#else
-        const u64 x = poseidon_sbox(s[j]);
-        dl[j] = u32_as_denormal((u32)x);
-        dh[j] = u32_as_denormal((u32)(x >> 32));
-#endif
     }
     poseidon_circ12<0>(dl, yl);
     poseidon_circ12<0>(dh, yh);
@@ -210,23 +209,12 @@ GL_D void poseidon_partial_pair(u64 s[12], int pair) {
         yl = __fma_rn((double)poseidon_mds_entry(0, j), dl[j], yl);
         yh = __fma_rn((double)poseidon_mds_entry(0, j), dh[j], yh);
     }
-#ifdef POSEIDON_SPLIT_SBOX
     poseidon_sbox_split(s[0], dl[0], dh[0]);
-#else
-    const u64 x0 = poseidon_sbox(s[0]);
-    dl[0] = u32_as_denormal((u32)x0);
-    dh[0] = u32_as_denormal((u32)(x0 >> 32));
-#endif
     yl = __fma_rn((double)poseidon_mds_entry(0, 0), dl[0], yl);      // Yraw
     yh = __fma_rn((double)poseidon_mds_entry(0, 0), dh[0], yh);
     const double2 ky = c_poseidon_rc_split[(POSEIDON_FULL_HALF + 2 * pair + 1) * 12];
-#ifdef POSEIDON_SPLIT_SBOX
     double gl, gh;
     poseidon_sbox_split(poseidon_fold(yl + ky.x, yh + ky.y), gl, gh);
-#else
-    const u64 sigma = poseidon_sbox(poseidon_fold(yl + ky.x, yh + ky.y));
-    const double gl = u32_as_denormal((u32)sigma), gh = u32_as_denormal((u32)(sigma >> 32));
-#endif
     double zl[12], zh[12];
     poseidon_circ12<1>(dl, zl);
     poseidon_circ12<1>(dh, zh);

@@ -85,8 +85,12 @@ inline bool generate(uint64_t* rc) {
 // can be as low as -2^33; every constant a sum with such a term meets then carries an offset that is 0 mod p and makes
 // the low accumulator positive: value = A + 2^32 B, p = 1 + 2^32 (2^32 - 1), so (A, B) += (2^e + k, k (2^32 - 1) - 2^(e-32))
 // with k = 1 (e = 42: one linear layer, gain <= 280) or k = 2^16 (e = 48: the fused pair, gain < 2^14.1 on lane 0).
+// handoff_bias: the device's S-box hands over r0 - r2 - r3 + handoff_bias (non-negative) instead of the signed coefficient,
+// so each low (A) entry loses handoff_bias times the total weight of the S-box outputs in its row.  Every accumulator the
+// fold sees is then the same integer as with the signed coefficients (handoff_bias = 0 describes that schedule).
 inline void linear_layer_tables(const uint64_t* rc, const int mds_circ[12], int mds_diag0, bool signed_sbox,
-                                uint64_t* split /* [31 * 12 * 2] */, uint64_t* pair_k /* [11 * 12 * 2] */) {
+                                uint64_t* split /* [31 * 12 * 2] */, uint64_t* pair_k /* [11 * 12 * 2] */,
+                                uint64_t handoff_bias = 0) {
     auto entry = [&](int r, int j) { return mds_circ[(j - r + 12) % 12] + ((r == 0 && j == 0) ? mds_diag0 : 0); };
     for (int i = 0; i < 31 * 12; i++) {
         const uint64_t v = i < 360 ? rc[i] : 0;
@@ -100,7 +104,10 @@ inline void linear_layer_tables(const uint64_t* rc, const int mds_circ[12], int 
             const bool lane0_only = round >= 5 && round <= 25 && (round & 1);                   // y0 of a fused pair
             for (int lane = 0; lane < 12; lane++)
                 if (full_layer || (lane0_only && lane == 0)) {
-                    split[2 * (round * 12 + lane)] += offA;
+                    // a full round's row sees all twelve S-box outputs, y0 of a pair only lane 0's
+                    uint64_t weight = 0;
+                    for (int j = 0; j < (full_layer ? 12 : 1); j++) weight += (uint64_t)entry(lane, j);
+                    split[2 * (round * 12 + lane)] += offA - handoff_bias * weight;
                     split[2 * (round * 12 + lane) + 1] += offB;
                 }
         }
@@ -115,7 +122,11 @@ inline void linear_layer_tables(const uint64_t* rc, const int mds_circ[12], int 
                 hi += (uint64_t)entry(lane, i) * (r1[i] >> 32);
             }
             if (signed_sbox) {
-                lo += (1ULL << 48) + (1ULL << 16);
+                // the S-box outputs of the pair reach row `lane` as N[lane][0] x~_0 (N = M M' without the lane-0 path:
+                // CIRC^2 x~ + col0(CIRC) (8 x~_0 - Yraw) on the device) and M[lane][0] sigma
+                uint64_t weight = (uint64_t)entry(lane, 0);
+                for (int i = 1; i < 12; i++) weight += (uint64_t)entry(lane, i) * (uint64_t)entry(i, 0);
+                lo += (1ULL << 48) + (1ULL << 16) - handoff_bias * weight;
                 hi += (1ULL << 16) * 0xFFFFFFFFULL - (1ULL << 16);
             }
             pair_k[(pair * 12 + lane) * 2] = lo;

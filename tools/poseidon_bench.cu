@@ -93,40 +93,54 @@ __global__ void k_circ_extremes(const u64* halves, int cases, int* bad) {
         if (double_bits(y1[r]) != c1[r] || double_bits(y2[r]) != c2[r]) atomicAdd(bad, 1);
 }
 
-// The same check for the SIGNED inputs of the split S-box: lanes in (-2^33, 2^32) for one layer (SQ = 0); lane 0 in that
-// range and lanes 1..11 in [0, 2^32) for the fused pair (SQ = 1).  v[t][i] = (a, b): the lane is denormal(a) - 2 denormal(b).
-__global__ void k_circ_signed(const u32* ab, int cases, int* bad) {
+// The same check for the inputs the S-box hand-off gives the layers: lanes in [0, 3 * 2^32) (dl = r0 - r2 - r3 + 2^33) for one
+// layer (SQ = 0); lane 0 in that range and lanes 1..11 in [0, 2^32) for the fused pair (SQ = 1).  ab[t][i] = (a, b): the
+// lane is a + 2 b, formed as an integer bit pattern the way poseidon_sbox_split forms it.
+__global__ void k_circ_handoff(const u32* ab, int cases, int* bad) {
     int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= cases) return;
     const u32* h = ab + 24 * t;
     const int C[12] = {17, 15, 41, 16, 2, 28, 13, 13, 39, 18, 34, 20};
     for (int sq = 0; sq < 2; sq++) {
         double x[12], y[12];
-        long long xi[12], c1[12], c2[12];
+        u64 xi[12], c1[12], c2[12];
         for (int i = 0; i < 12; i++) {
-            const bool sgn = sq == 0 || i == 0;
-            const double a = u32_as_denormal(h[2 * i]), b = u32_as_denormal(h[2 * i + 1]);
-            x[i] = sgn ? (a - b) - b : a;
-            xi[i] = sgn ? (long long)h[2 * i] - 2 * (long long)h[2 * i + 1] : (long long)h[2 * i];
+            xi[i] = (sq == 0 || i == 0) ? (u64)h[2 * i] + 2 * (u64)h[2 * i + 1] : (u64)h[2 * i];
+            x[i] = __longlong_as_double((long long)xi[i]);
         }
         if (sq == 0) poseidon_circ12<0>(x, y);
         else poseidon_circ12<1>(x, y);
         for (int r = 0; r < 12; r++) {
-            long long acc = 0;
-            for (int i = 0; i < 12; i++) acc += (long long)C[i] * xi[(i + r) % 12];
+            u64 acc = 0;
+            for (int i = 0; i < 12; i++) acc += (u64)C[i] * xi[(i + r) % 12];
             c1[r] = acc;
         }
         for (int r = 0; r < 12; r++) {
-            long long acc = 0;
-            for (int i = 0; i < 12; i++) acc += (long long)C[i] * c1[(i + r) % 12];
+            u64 acc = 0;
+            for (int i = 0; i < 12; i++) acc += (u64)C[i] * c1[(i + r) % 12];
             c2[r] = acc;
         }
-        for (int r = 0; r < 12; r++) {
-            // y is an integer multiple of 2^-1074 below 2^53 in magnitude: scale it up exactly and compare as an integer
-            const long long got = (long long)((y[r] * 0x1p537) * 0x1p537);
-            if (got != (sq ? c2[r] : c1[r])) atomicAdd(bad, 1);
-        }
+        for (int r = 0; r < 12; r++)
+            if (double_bits(y[r]) != (sq ? c2[r] : c1[r])) atomicAdd(bad, 1);
     }
+}
+
+// The integer forms at their extremes against 128-bit arithmetic: the S-box hand-off (dl - 2^33 + 2^32 dh = x^7 mod p) and
+// the fold (A + 2^32 B mod p for A in [2^18, 2^50), B in [0, 2^50), the range the tables guarantee).  w[t] = (x, A, B).
+__global__ void k_forms(const u64* w, int cases, int* bad) {
+    int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= cases) return;
+    typedef unsigned __int128 u128;
+    const u64 x = w[3 * t], A = w[3 * t + 1], B = w[3 * t + 2];
+    double dl, dh;
+    poseidon_sbox_split(x, dl, dh);
+    u64 x7 = 1;
+    for (int i = 0; i < 7; i++) x7 = (u64)((u128)x7 * (x % GL_P) % GL_P);
+    const u64 l = double_bits(dl), h = double_bits(dh);
+    if (l < 2 || l >= (3ULL << 32) || h >= (1ULL << 33)) atomicAdd(bad, 1);
+    if ((u64)(((u128)l + ((u128)h << 32) + (u128)GL_P * 4 - POSEIDON_HANDOFF_BIAS) % GL_P) != x7) atomicAdd(bad, 1);
+    const u64 y = poseidon_fold(__longlong_as_double((long long)A), __longlong_as_double((long long)B));
+    if (y % GL_P != (u64)(((u128)A + ((u128)B << 32)) % GL_P)) atomicAdd(bad, 1);
 }
 
 int main() {
@@ -135,12 +149,7 @@ int main() {
     cudaMemcpyToSymbol(c_poseidon_rc, rc, sizeof rc);
     static u64 split[31 * 12 * 2], pk[11 * 12 * 2];
     static const int circ[12] = {17, 15, 41, 16, 2, 28, 13, 13, 39, 18, 34, 20};
-#ifdef POSEIDON_SPLIT_SBOX
-    const bool signed_sbox = true;
-#else
-    const bool signed_sbox = false;
-#endif
-    poseidon_constants::linear_layer_tables(rc, circ, 8, signed_sbox, split, pk);
+    poseidon_constants::linear_layer_tables(rc, circ, 8, true, split, pk, POSEIDON_HANDOFF_BIAS);
     cudaMemcpyToSymbol(c_poseidon_rc_split, split, sizeof split);
     cudaMemcpyToSymbol(c_poseidon_pair_k, pk, sizeof pk);
     u64 h[12], *d;
@@ -194,11 +203,12 @@ int main() {
             for (int i = 0; i < 24; i++) {
                 st ^= st << 13; st ^= st >> 7; st ^= st << 17;
                 u32 v = (u32)st;
-                const int mode = t & 7;   // extremes of a - 2b: all most negative, all most positive, alternating, random
-                if (mode == 0) v = (i & 1) ? 0xFFFFFFFFu : 0u;
-                else if (mode == 1) v = (i & 1) ? 0u : 0xFFFFFFFFu;
-                else if (mode == 2) v = (((i >> 1) + (t >> 3)) & 1) ? ((i & 1) ? 0xFFFFFFFFu : 0u) : ((i & 1) ? 0u : 0xFFFFFFFFu);
-                else if (mode == 3 && (st >> 40) % 3 == 0) v = 0xFFFFFFFFu;
+                const int mode = t & 7;   // all limbs max, all zero, alternating lanes, one-hot lane, random with extremes
+                if (mode == 0) v = 0xFFFFFFFFu;
+                else if (mode == 1) v = 0;
+                else if (mode == 2) v = (((i >> 1) + (t >> 3)) & 1) ? 0xFFFFFFFFu : 0u;
+                else if (mode == 3) v = ((i >> 1) == (t >> 3) % 12) ? 0xFFFFFFFFu : 0u;
+                else if (mode == 4 && (st >> 40) % 3 == 0) v = 0xFFFFFFFFu;
                 hh[(size_t)t * 24 + i] = v;
             }
         u32* dh;
@@ -207,11 +217,43 @@ int main() {
         cudaMalloc(&dbad, 4);
         cudaMemcpy(dh, hh, (size_t)cases * 96, cudaMemcpyHostToDevice);
         cudaMemset(dbad, 0, 4);
-        k_circ_signed<<<cases / 128, 128>>>(dh, cases, dbad);
+        k_circ_handoff<<<cases / 128, 128>>>(dh, cases, dbad);
         cudaMemcpy(&hbad, dbad, 4, cudaMemcpyDeviceToHost);
-        printf("{\"circ12_signed_cases\": %d, \"mismatches\": %d}\n", cases, hbad);
+        printf("{\"circ12_handoff_cases\": %d, \"mismatches\": %d}\n", cases, hbad);
         ok &= hbad == 0;
         free(hh);
+    }
+    {
+        const int cases = 1 << 16;
+        u64* hw = (u64*)malloc((size_t)cases * 24);
+        u64 st = 0x2545F4914F6CDD1DULL;
+        const u64 X[6] = {0, 1, GL_P - 1, 0xFFFFFFFFFFFFFFFFULL, 0xFFFFFFFF00000000ULL, 0xFFFFFFFFULL};
+        const u64 AMIN = 1ULL << 18, AMAX = (1ULL << 50) - 1, BMAX = (1ULL << 50) - 1;
+        for (int t = 0; t < cases; t++) {
+            u64 r[3];
+            for (int k = 0; k < 3; k++) { st ^= st << 13; st ^= st >> 7; st ^= st << 17; r[k] = st; }
+            const int mode = t & 7;   // extremes of x, A, B (b0 = 0xffffffff, bh max, A at both ends), then random
+            u64 x = r[0], A = AMIN + r[1] % (AMAX - AMIN + 1), B = r[2] & BMAX;
+            if (mode < 6) x = X[mode];
+            if (mode == 0) { A = AMAX; B = BMAX; }
+            else if (mode == 1) { A = AMIN; B = BMAX; }
+            else if (mode == 2) { A = AMIN; B = 0; }
+            else if (mode == 3) { A = AMAX; B = 0xFFFFFFFFULL; }
+            else if (mode == 4) { A = AMIN; B = BMAX & ~0xFFFFFFFFULL; }
+            else if (mode == 5) B |= 0xFFFFFFFFULL;
+            hw[3 * t] = x; hw[3 * t + 1] = A; hw[3 * t + 2] = B;
+        }
+        u64* dw;
+        int *dbad, hbad = 0;
+        cudaMalloc(&dw, (size_t)cases * 24);
+        cudaMalloc(&dbad, 4);
+        cudaMemcpy(dw, hw, (size_t)cases * 24, cudaMemcpyHostToDevice);
+        cudaMemset(dbad, 0, 4);
+        k_forms<<<cases / 128, 128>>>(dw, cases, dbad);
+        cudaMemcpy(&hbad, dbad, 4, cudaMemcpyDeviceToHost);
+        printf("{\"handoff_fold_cases\": %d, \"mismatches\": %d}\n", cases, hbad);
+        ok &= hbad == 0;
+        free(hw);
     }
     cudaDeviceProp p;
     cudaGetDeviceProperties(&p, 0);
