@@ -19,6 +19,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <map>
+#include <memory>
 #include <random>
 #include <mutex>
 #include <new>
@@ -63,7 +64,6 @@ struct gl_ctx {
     std::map<std::tuple<int, uint64_t, uint64_t, uint64_t>, u64*> tables;
     DevBuf scratch[6];
     std::mutex mu;
-    int live_commits = 0;
     // freed commit buffers, kept for the next commit of the same geometry (cudaMalloc/cudaFree of
     // multi-GB blocks cost milliseconds and serialise the device)
     std::multimap<size_t, void*> pool;
@@ -79,31 +79,6 @@ struct gl_ctx {
     bool ev_valid = false;
     float phase_ms[GL_PHASES] = {};
 };
-
-struct gl_commit {
-    gl_ctx* ctx = nullptr;
-    uint32_t log_n = 0, c = 0, rate_bits = 0, cap_height = 0;
-    uint32_t salt = 0;         // blinding: SALT_SIZE = 4 random columns after the c polynomial columns of every leaf
-    uint32_t shard_index = 0, shard_count = 1;
-    uint64_t n_local = 0;      // leaves held here
-    uint64_t leaf_begin = 0;   // global index of the first local leaf
-    uint32_t cap_local_bits = 0;
-    u64* coeffs = nullptr;     // [c][n]
-    u64* lde = nullptr;        // [c + salt][n_local]
-    u64* digests = nullptr;    // [2*(n_local - 2^cap_local_bits)][4]
-    u64* cap = nullptr;        // [2^cap_local_bits][4]
-    uint64_t num_digests = 0;
-    size_t coeffs_bytes = 0, lde_bytes = 0, digests_bytes = 0, cap_bytes = 0;
-    uint32_t cols_added = 0;   // gl_commit_begin / add_coeffs / finish
-    bool finished = true;
-    // GL_COMMIT_STREAM_HASH: leaves are absorbed 8 polynomials at a time as the blocks arrive
-    bool stream_hash = false;
-    uint32_t next_col = 0, hashed_cols = 0;
-    u64* hstate = nullptr;     // [12][n_local] sponge states between blocks
-    size_t hstate_bytes = 0;
-};
-
-static inline uint32_t leaf_len(const gl_commit* h) { return h->c + h->salt; }   // MerkleTree.leaves[i].len()
 
 static int fail(gl_ctx* ctx, int code, const std::string& msg) {
     if (ctx) ctx->err = msg;
@@ -208,6 +183,68 @@ static void dev_release(gl_ctx* ctx, void* p, size_t bytes) {
     ctx->pool.emplace(bytes, p);
     ctx->pool_bytes += bytes;
 }
+
+// The one owner of a pooled block: the block goes back to the pool when the owner is reset or dies.  An owner dies
+// with the ctx's mutex held and its device current (declare it after the Guard).
+class PoolBuf {
+  public:
+    PoolBuf() = default;
+    PoolBuf(const PoolBuf&) = delete;
+    PoolBuf& operator=(const PoolBuf&) = delete;
+    PoolBuf(PoolBuf&& o) noexcept : ctx_(o.ctx_), p_(o.p_), bytes_(o.bytes_) { o.p_ = nullptr; }
+    PoolBuf& operator=(PoolBuf&& o) noexcept {
+        if (this != &o) {
+            reset();
+            ctx_ = o.ctx_;
+            p_ = o.p_;
+            bytes_ = o.bytes_;
+            o.p_ = nullptr;
+        }
+        return *this;
+    }
+    ~PoolBuf() { reset(); }
+    int alloc(gl_ctx* ctx, size_t bytes) {
+        reset();
+        TRY(dev_alloc(ctx, bytes, &p_));
+        ctx_ = ctx;
+        bytes_ = bytes;
+        return GL_OK;
+    }
+    void reset() {
+        dev_release(ctx_, p_, bytes_);
+        p_ = nullptr;
+    }
+    u64* get() const { return p_; }
+    size_t bytes() const { return bytes_; }
+
+  private:
+    gl_ctx* ctx_ = nullptr;
+    u64* p_ = nullptr;
+    size_t bytes_ = 0;
+};
+
+struct gl_commit {
+    gl_ctx* ctx = nullptr;
+    uint32_t log_n = 0, c = 0, rate_bits = 0, cap_height = 0;
+    uint32_t salt = 0;         // blinding: SALT_SIZE = 4 random columns after the c polynomial columns of every leaf
+    uint32_t shard_index = 0, shard_count = 1;
+    uint64_t n_local = 0;      // leaves held here
+    uint64_t leaf_begin = 0;   // global index of the first local leaf
+    uint32_t cap_local_bits = 0;
+    PoolBuf coeffs;            // [c][n]
+    PoolBuf lde;               // [c + salt][n_local]
+    PoolBuf digests;           // [2*(n_local - 2^cap_local_bits)][4]
+    PoolBuf cap;               // [2^cap_local_bits][4]
+    uint64_t num_digests = 0;
+    uint32_t cols_added = 0;   // gl_commit_begin / add_coeffs / finish
+    bool finished = true;
+    // GL_COMMIT_STREAM_HASH: leaves are absorbed 8 polynomials at a time as the blocks arrive
+    bool stream_hash = false;
+    uint32_t next_col = 0, hashed_cols = 0;
+    PoolBuf hstate;            // [12][n_local] sponge states between blocks
+};
+
+static inline uint32_t leaf_len(const gl_commit* h) { return h->c + h->salt; }   // MerkleTree.leaves[i].len()
 
 // Host <-> device copies of caller buffers.  Page-able memory of a megabyte or more is staged through
 // page-locked rings by helper threads (host_staging.h); small or page-locked buffers go straight to the DMA engine.
@@ -626,20 +663,20 @@ extern "C" int gl_ctx_create(int device, gl_ctx** out) {
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&ctx->d2h_stream, cudaStreamNonBlocking);
     if (e != cudaSuccess) {
         int rc = cuda_fail(nullptr, e, "gl_ctx_create");
-        delete ctx;
+        gl_ctx_destroy(ctx);
         return rc;
     }
     for (auto& ev : ctx->ev) cudaEventCreate(&ev);
     cudaEventCreateWithFlags(&ctx->dl_ev, cudaEventDisableTiming);
     uint64_t rc360[360];
     if (!poseidon_constants::generate(rc360)) {
-        delete ctx;
+        gl_ctx_destroy(ctx);
         return fail(nullptr, GL_E_STATE, "gl_ctx_create: derived Poseidon round constants fail their fingerprint");
     }
     int up = gl_poseidon_upload_constants(rc360);
     if (up != 0) {
         int rc = cuda_fail(nullptr, (cudaError_t)up, "upload Poseidon constants");
-        delete ctx;
+        gl_ctx_destroy(ctx);
         return rc;
     }
     int st = gl_field_selftest(ctx->stream);
@@ -663,7 +700,7 @@ extern "C" void gl_ctx_destroy(gl_ctx* ctx) {
     if (!ctx) return;
     {
         Guard g(ctx);
-        cudaStreamSynchronize(ctx->stream);
+        if (ctx->stream) cudaStreamSynchronize(ctx->stream);
         delete ctx->downloader;   // joins the worker
         ctx->h2d_ring.destroy();
         if (ctx->dl_ev) cudaEventDestroy(ctx->dl_ev);
@@ -677,7 +714,7 @@ extern "C" void gl_ctx_destroy(gl_ctx* ctx) {
         for (auto& ev : ctx->pipe_ev) cudaEventDestroy(ev);
         if (ctx->h2d_stream) cudaStreamDestroy(ctx->h2d_stream);
         if (ctx->d2h_stream) cudaStreamDestroy(ctx->d2h_stream);
-        cudaStreamDestroy(ctx->stream);
+        if (ctx->stream) cudaStreamDestroy(ctx->stream);
     }
     delete ctx;
 }
@@ -999,48 +1036,32 @@ static int smt_events_run(gl_ctx* ctx, const u64* dk, const u64* dv, uint64_t m,
     q.bit = (uint8_t*)(p0 + o_keys) + 4 * m;   // m bytes
     u64* d_off = (u64*)(p0 + o_off);
     // per-event sibling rows while sweeping: [m][stride][4]; counts (u32 [m + 1]) reuse the radix-sort double buffer
-    const size_t sib_bytes = (size_t)m * q.stride * 32;
-    u64* d_sib = nullptr;
-    TRY(dev_alloc(ctx, sib_bytes, &d_sib));
-    q.sib = d_sib;
+    PoolBuf d_sib;
+    TRY(d_sib.alloc(ctx, (size_t)m * q.stride * 32));
+    q.sib = d_sib.get();
     uint32_t* counts = (uint32_t*)b.rk_alt;   // m * 8 bytes >= (m + 1) * 4
     rc = smt_proofs_sweep(q, dmax, hist, counts, b.sort_tmp, tmp_bytes, ctx->stream);
     if (rc == 0) rc = smt_proofs_offsets(counts, d_off, m, b.sort_tmp, tmp_bytes, ctx->stream);
-    if (rc) {
-        cudaStreamSynchronize(ctx->stream);
-        dev_release(ctx, d_sib, sib_bytes);
-        return cuda_fail(ctx, (cudaError_t)rc, name);
-    }
+    if (rc) return cuda_fail(ctx, (cudaError_t)rc, name);
     u64 total = 0;
     cudaError_t e = cudaMemcpyAsync(&total, d_off + m, 8, cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) {
-        dev_release(ctx, d_sib, sib_bytes);
-        return cuda_fail(ctx, e, name);
-    }
+    if (e != cudaSuccess) return cuda_fail(ctx, e, name);
     *num_siblings_out = total;
-    int out_rc = GL_OK;
-    u64* d_pool = nullptr;
-    size_t pool_bytes = 0;
+    PoolBuf d_pool;
     if (sib_pool_out && total <= sib_cap && total) {
         if (space == GL_DEVICE) {
             smt_proofs_gather(q, d_off, sib_cap, sib_pool_out, ctx->stream);
         } else {
-            pool_bytes = (size_t)total * 32;
-            out_rc = dev_alloc(ctx, pool_bytes, &d_pool);
-            if (out_rc == GL_OK) {
-                smt_proofs_gather(q, d_off, total, d_pool, ctx->stream);
-                out_rc = copy_out(ctx, sib_pool_out, d_pool, pool_bytes, GL_HOST);
-            }
+            TRY(d_pool.alloc(ctx, (size_t)total * 32));
+            smt_proofs_gather(q, d_off, total, d_pool.get(), ctx->stream);
+            TRY(copy_out(ctx, sib_pool_out, d_pool.get(), d_pool.bytes(), GL_HOST));
         }
     }
-    if (out_rc == GL_OK) out_rc = copy_out(ctx, hdr_out, p0 + o_hdr, hdr_bytes, space);
+    TRY(copy_out(ctx, hdr_out, p0 + o_hdr, hdr_bytes, space));
     // in find mode the sets have no siblings, so the offsets of the queries start at 0
-    if (out_rc == GL_OK) out_rc = copy_out(ctx, sib_off_out, d_off + (m - n_out), (n_out + 1) * 8, space);
-    int frc = finish(ctx);
-    dev_release(ctx, d_sib, sib_bytes);
-    if (d_pool) dev_release(ctx, d_pool, pool_bytes);
-    return out_rc != GL_OK ? out_rc : frc;
+    TRY(copy_out(ctx, sib_off_out, d_off + (m - n_out), (n_out + 1) * 8, space));
+    return finish(ctx);
 }
 
 // N2, second half: the process proofs of m successive `set` calls on an empty tree (smt_proofs.cu)
@@ -1179,16 +1200,23 @@ extern "C" int gl_coset_ifft_batch(gl_ctx* ctx, uint64_t* data, uint32_t log_n, 
 // ------------------------------------------------------------------------------------------------
 // PolynomialBatch::from_values / from_coeffs
 // ------------------------------------------------------------------------------------------------
-static void commit_release(gl_commit* h) {
-    if (!h) return;
-    dev_release(h->ctx, h->coeffs, h->coeffs_bytes);
-    dev_release(h->ctx, h->lde, h->lde_bytes);
-    dev_release(h->ctx, h->digests, h->digests_bytes);
-    dev_release(h->ctx, h->cap, h->cap_bytes);
-    if (h->hstate) dev_release(h->ctx, h->hstate, h->hstate_bytes);
-    delete h;
-}
 static void mark(gl_ctx* ctx, int i) { cudaEventRecord(ctx->ev[i], ctx->stream); }
+
+// end of a successful commit: the streaming hash state goes back to the pool, the phase times are kept
+static void commit_done(gl_ctx* ctx, gl_commit* h) {
+    h->hstate.reset();
+    for (int i = 0; i < GL_PHASES; i++) cudaEventElapsedTime(&ctx->phase_ms[i], ctx->ev[i], ctx->ev[i + 1]);
+    ctx->ev_valid = true;
+}
+
+// A failed commit may still have copies in flight on the PCIe streams, which are not ordered with ctx->stream: every
+// stream drains before the handle, and with it its blocks, is dropped.
+static void quiesce(gl_ctx* ctx) {
+    cudaStreamSynchronize(ctx->stream);
+    cudaStreamSynchronize(ctx->h2d_stream);
+    cudaStreamSynchronize(ctx->d2h_stream);
+    cudaGetLastError();
+}
 
 static int commit_check(gl_ctx* ctx, uint32_t log_n, uint32_t c, uint32_t rate_bits, uint32_t cap_height,
                         const char* name) {
@@ -1202,22 +1230,24 @@ static int commit_check(gl_ctx* ctx, uint32_t log_n, uint32_t c, uint32_t rate_b
     return GL_OK;
 }
 
-// h->coeffs already holds the coefficients on the device
-// geometry + device buffers of the LDE / digests / cap
-static int commit_prepare(gl_ctx* ctx, gl_commit* h) {
+// A polynomial commit of the ctx's shard with every block allocated: `coeff_cols` >= c coefficient columns, the LDE,
+// the digests and the cap
+static int commit_new(gl_ctx* ctx, uint32_t log_n, uint32_t c, uint32_t rate_bits, uint32_t cap_height, uint32_t salt,
+                      uint32_t coeff_cols, std::unique_ptr<gl_commit>* out) {
+    std::unique_ptr<gl_commit> h(new (std::nothrow) gl_commit());
+    if (!h) return fail(ctx, GL_E_OOM, "host allocation failed");
+    h->ctx = ctx; h->log_n = log_n; h->c = c; h->rate_bits = rate_bits; h->cap_height = cap_height; h->salt = salt;
+    h->shard_index = ctx->shard_index; h->shard_count = ctx->shard_count;
     const unsigned lc = ilog2(h->shard_count);
-    const u64 n = (u64)1 << h->log_n;
-    const uint32_t blocks = (1u << h->rate_bits) >> lc;
-    h->n_local = n * blocks;
+    h->n_local = ((u64)1 << log_n) * ((1u << rate_bits) >> lc);
     h->leaf_begin = (u64)h->shard_index * h->n_local;
-    h->cap_local_bits = h->cap_height - lc;
+    h->cap_local_bits = cap_height - lc;
     h->num_digests = 2 * (h->n_local - ((u64)1 << h->cap_local_bits));
-    h->lde_bytes = (size_t)leaf_len(h) * h->n_local * 8;
-    h->digests_bytes = h->num_digests * 32;
-    h->cap_bytes = (size_t)32 << h->cap_local_bits;
-    TRY(dev_alloc(ctx, h->lde_bytes, &h->lde));
-    TRY(dev_alloc(ctx, h->digests_bytes, &h->digests));
-    TRY(dev_alloc(ctx, h->cap_bytes, &h->cap));
+    TRY(h->coeffs.alloc(ctx, ((size_t)coeff_cols << log_n) * 8));
+    TRY(h->lde.alloc(ctx, (size_t)leaf_len(h.get()) * h->n_local * 8));
+    TRY(h->digests.alloc(ctx, h->num_digests * 32));
+    TRY(h->cap.alloc(ctx, (size_t)32 << h->cap_local_bits));
+    *out = std::move(h);
     return GL_OK;
 }
 
@@ -1228,8 +1258,8 @@ static int commit_lde_columns(gl_ctx* ctx, gl_commit* h, uint32_t col0, uint32_t
     const u64* pre;
     TRY(coset_tables(ctx, h->log_n, h->rate_bits, h->shard_index, h->shard_count, &pre));
     NttJob j;
-    j.in = h->coeffs + (size_t)col0 * n; j.in_ld = n; j.in_coset_stride = 0;
-    j.out = h->lde + (size_t)col0 * h->n_local; j.out_ld = h->n_local; j.out_coset_stride = n;
+    j.in = h->coeffs.get() + (size_t)col0 * n; j.in_ld = n; j.in_coset_stride = 0;
+    j.out = h->lde.get() + (size_t)col0 * h->n_local; j.out_ld = h->n_local; j.out_coset_stride = n;
     j.L = h->log_n; j.columns = ncols; j.cosets = blocks; j.inverse = false; j.pre_tab = pre;
     j.pre_direct_ok = true;
     j.canonical_out = 1;
@@ -1241,18 +1271,19 @@ static int commit_tree(gl_ctx* ctx, gl_commit* h, uint64_t* cap_out, int space, 
     const unsigned lg_local = h->log_n + h->rate_bits - ilog2(h->shard_count);
     if (h->salt) {
         // lde_values(): `.chain((0..salt_size).map(|_| F::rand_vec(degree << rate_bits)))` -- uniform field elements
-        launch_salt_fill(h->lde + (size_t)h->c * h->n_local, (u64)h->salt * h->n_local, ctx->salt_seed,
+        launch_salt_fill(h->lde.get() + (size_t)h->c * h->n_local, (u64)h->salt * h->n_local, ctx->salt_seed,
                          (ctx->salt_counter++ << 8) | h->shard_index, ctx->stream);
     }
     mark(ctx, 4);
     if (!leaves_hashed)
-        launch_leaf_hash_cols(h->lde, h->n_local, leaf_len(h), lg_local, h->cap_local_bits, h->digests, h->cap, ctx->stream);
+        launch_leaf_hash_cols(h->lde.get(), h->n_local, leaf_len(h), lg_local, h->cap_local_bits, h->digests.get(), h->cap.get(),
+                              ctx->stream);
     mark(ctx, 5);
-    launch_merkle_levels(lg_local, h->cap_local_bits, h->digests, h->cap, ctx->stream);
+    launch_merkle_levels(lg_local, h->cap_local_bits, h->digests.get(), h->cap.get(), ctx->stream);
     mark(ctx, 6);
     if (cap_out) {
         uint64_t* dst = cap_out + 4 * ((size_t)h->shard_index << h->cap_local_bits);
-        TRY(copy_out(ctx, dst, h->cap, h->cap_bytes, space));
+        TRY(copy_out(ctx, dst, h->cap.get(), h->cap.bytes(), space));
     }
     return GL_OK;
 }
@@ -1271,13 +1302,10 @@ static int commit_absorb_block(gl_ctx* ctx, gl_commit* h, uint32_t col0, uint32_
     const uint32_t complete = h->next_col == h->c ? h->c : (h->next_col & ~7u);
     if (complete <= h->hashed_cols) return GL_OK;
     const bool first = h->hashed_cols == 0, last = complete == h->c;
-    if (!h->hstate && !(first && last)) {
-        h->hstate_bytes = (size_t)h->n_local * 12 * 8;
-        TRY(dev_alloc(ctx, h->hstate_bytes, &h->hstate));
-    }
+    if (!h->hstate.get() && !(first && last)) TRY(h->hstate.alloc(ctx, (size_t)h->n_local * 12 * 8));
     const unsigned lg_local = h->log_n + h->rate_bits - ilog2(h->shard_count);
-    launch_leaf_absorb_cols(h->lde, h->n_local, h->hashed_cols, complete, lg_local, h->cap_local_bits, h->hstate, first, last,
-                            h->digests, h->cap, ctx->stream);
+    launch_leaf_absorb_cols(h->lde.get(), h->n_local, h->hashed_cols, complete, lg_local, h->cap_local_bits, h->hstate.get(), first,
+                            last, h->digests.get(), h->cap.get(), ctx->stream);
     h->hashed_cols = complete;
     return GL_OK;
 }
@@ -1336,7 +1364,7 @@ static int commit_pipeline_host(gl_ctx* ctx, gl_commit* h, const HostCols& input
     for (uint32_t b = 0; col0 < h->c; b++) {
         const uint32_t want = b == 0 ? cb0 : cb;
         const uint32_t nc = (col0 + want <= h->c) ? want : h->c - col0;
-        u64* dcol = h->coeffs + (size_t)col0 * n;
+        u64* dcol = h->coeffs.get() + (size_t)col0 * n;
         input.segs(col0, nc, n, segs);
         TRY(h2d_copy(ctx, dcol, segs.data(), segs.size(), ctx->h2d_stream));
         CK(cudaEventRecord(ctx->pipe_ev[2 * b], ctx->h2d_stream));
@@ -1356,6 +1384,38 @@ static int commit_pipeline_host(gl_ctx* ctx, gl_commit* h, const HostCols& input
     return GL_OK;
 }
 
+// copy-in, IFFT, LDE and tree of the freshly allocated commit `h`
+static int commit_build(gl_ctx* ctx, gl_commit* h, const HostCols& input, bool is_values, const HostCols& coeffs_out,
+                        uint64_t* cap_out, int space) {
+    mark(ctx, 0);
+    if (space == GL_HOST) {
+        // phases 1..3 overlap in this mode: their sum is reported as "lde_ntt" (phase 3)
+        mark(ctx, 1);
+        mark(ctx, 2);
+        mark(ctx, 3);
+        h->stream_hash = h->c > 4 && nblocks_host(h) > 1 && !h->salt;   // the salt columns only exist at the end
+        TRY(commit_pipeline_host(ctx, h, input, is_values, coeffs_out));
+    } else {
+        if (!is_values) {
+            cudaError_t e = cudaMemcpyAsync(h->coeffs.get(), input.flat, h->coeffs.bytes(), cudaMemcpyDeviceToDevice, ctx->stream);
+            if (e != cudaSuccess) return cuda_fail(ctx, e, "copy polynomials");
+        }
+        mark(ctx, 1);
+        if (is_values) {
+            // "IFFT": reads the caller's values where they lie, the coefficients land behind the handle
+            TRY(transform_natural(ctx, h->coeffs.get(), h->log_n, h->c, true, nullptr, nullptr, input.flat));
+            mark(ctx, 2);
+            TRY(copy_out(ctx, coeffs_out.flat, h->coeffs.get(), h->coeffs.bytes(), space));
+        } else {
+            mark(ctx, 2);
+        }
+        mark(ctx, 3);
+        TRY(commit_lde_columns(ctx, h, 0, h->c));
+    }
+    TRY(commit_tree(ctx, h, cap_out, space, h->stream_hash && h->hashed_cols == h->c));
+    return finish(ctx);
+}
+
 static int commit_common(gl_ctx* ctx, const HostCols& input, bool is_values, uint32_t log_n, uint32_t c,
                          uint32_t rate_bits, uint32_t cap_height, const HostCols& coeffs_out, uint64_t* cap_out,
                          gl_commit** handle, int space, const char* name, bool blinding = false) {
@@ -1369,65 +1429,19 @@ static int commit_common(gl_ctx* ctx, const HostCols& input, bool is_values, uin
                 return fail(ctx, GL_E_ARG, std::string(name) + ": NULL polynomial pointer");
     }
     Guard g(ctx);
-    gl_commit* h = new (std::nothrow) gl_commit();
-    if (!h) return fail(ctx, GL_E_OOM, "host allocation failed");
-    h->ctx = ctx; h->log_n = log_n; h->c = c; h->rate_bits = rate_bits; h->cap_height = cap_height;
-    h->salt = blinding ? GL_SALT_SIZE : 0;
-    h->shard_index = ctx->shard_index; h->shard_count = ctx->shard_count;
-    const u64 n = (u64)1 << log_n;
-    const size_t poly_bytes = (size_t)c * n * 8;
-    h->coeffs_bytes = poly_bytes;
-    int rc = dev_alloc(ctx, poly_bytes, &h->coeffs);
-    if (rc == GL_OK) rc = commit_prepare(ctx, h);
-    mark(ctx, 0);
-    if (rc == GL_OK && space == GL_HOST) {
-        // phases 1..3 overlap in this mode: their sum is reported as "lde_ntt" (phase 3)
-        mark(ctx, 1);
-        mark(ctx, 2);
-        mark(ctx, 3);
-        h->stream_hash = c > 4 && nblocks_host(h) > 1 && !h->salt;   // the salt columns only exist at the end
-        rc = commit_pipeline_host(ctx, h, input, is_values, coeffs_out);
-    } else if (rc == GL_OK) {
-        if (!is_values) {
-            cudaError_t e = cudaMemcpyAsync(h->coeffs, input.flat, poly_bytes, cudaMemcpyDeviceToDevice, ctx->stream);
-            if (e != cudaSuccess) rc = cuda_fail(ctx, e, "copy polynomials");
-        }
-        mark(ctx, 1);
-        if (rc == GL_OK && is_values) {
-            // "IFFT": reads the caller's values where they lie, the coefficients land behind the handle
-            rc = transform_natural(ctx, h->coeffs, log_n, c, true, nullptr, nullptr, input.flat);
-            mark(ctx, 2);
-            if (rc == GL_OK) rc = copy_out(ctx, coeffs_out.flat, h->coeffs, poly_bytes, space);
-        } else {
-            mark(ctx, 2);
-        }
-        mark(ctx, 3);
-        if (rc == GL_OK) rc = commit_lde_columns(ctx, h, 0, c);
-    }
-    if (rc == GL_OK) rc = commit_tree(ctx, h, cap_out, space, h->stream_hash && h->hashed_cols == h->c);
-    if (rc == GL_OK) rc = finish(ctx);
-    if (h->hstate) {
-        dev_release(ctx, h->hstate, h->hstate_bytes);
-        h->hstate = nullptr;
-    }
+    std::unique_ptr<gl_commit> h;
+    int rc = commit_new(ctx, log_n, c, rate_bits, cap_height, blinding ? GL_SALT_SIZE : 0, c, &h);
+    if (rc == GL_OK) rc = commit_build(ctx, h.get(), input, is_values, coeffs_out, cap_out, space);
     if (space == GL_HOST) {   // coefficient downloads (also after an error: they write into caller memory)
         int rc2 = downloads_wait(ctx);
         if (rc == GL_OK) rc = rc2;
     }
-    if (rc == GL_OK) {
-        for (int i = 0; i < GL_PHASES; i++) cudaEventElapsedTime(&ctx->phase_ms[i], ctx->ev[i], ctx->ev[i + 1]);
-        ctx->ev_valid = true;
-    }
     if (rc != GL_OK) {
-        cudaStreamSynchronize(ctx->stream);
-        cudaStreamSynchronize(ctx->h2d_stream);
-        cudaStreamSynchronize(ctx->d2h_stream);
-        cudaGetLastError();
-        commit_release(h);
+        quiesce(ctx);
         return rc;
     }
-    ctx->live_commits++;
-    *handle = h;
+    commit_done(ctx, h.get());
+    *handle = h.release();
     return GL_OK;
 }
 
@@ -1522,24 +1536,13 @@ extern "C" int gl_commit_begin_ex(gl_ctx* ctx, uint32_t log_n, uint32_t c, uint3
     *handle = nullptr;
     TRY(commit_check(ctx, log_n, c, rate_bits, cap_height, "PolynomialBatch::from_coeffs"));
     Guard g(ctx);
-    gl_commit* h = new (std::nothrow) gl_commit();
-    if (!h) return fail(ctx, GL_E_OOM, "host allocation failed");
-    h->ctx = ctx; h->log_n = log_n; h->c = c; h->rate_bits = rate_bits; h->cap_height = cap_height;
-    h->shard_index = ctx->shard_index; h->shard_count = ctx->shard_count;
-    h->coeffs_bytes = ((size_t)c << log_n) * 8;
+    std::unique_ptr<gl_commit> h;
+    TRY(commit_new(ctx, log_n, c, rate_bits, cap_height, (flags & GL_COMMIT_BLINDING) ? GL_SALT_SIZE : 0, c, &h));
     h->finished = false;
-    h->salt = (flags & GL_COMMIT_BLINDING) ? GL_SALT_SIZE : 0;
     // <= 4 polynomials: hash_or_noop copies, nothing to absorb; salted leaves: the salt columns only exist at the end
     h->stream_hash = (flags & GL_COMMIT_STREAM_HASH) && c > 4 && !h->salt;
-    int rc = dev_alloc(ctx, h->coeffs_bytes, &h->coeffs);
-    if (rc == GL_OK) rc = commit_prepare(ctx, h);
-    if (rc != GL_OK) {
-        commit_release(h);
-        return rc;
-    }
     for (int i = 0; i <= 3; i++) mark(ctx, i);
-    ctx->live_commits++;
-    *handle = h;
+    *handle = h.release();
     return GL_OK;
 }
 extern "C" int gl_commit_add_coeffs(gl_commit* h, uint32_t col0, uint32_t ncols, const uint64_t* coeffs, int space) {
@@ -1549,7 +1552,7 @@ extern "C" int gl_commit_add_coeffs(gl_commit* h, uint32_t col0, uint32_t ncols,
     if (!coeffs || ncols == 0 || col0 + (uint64_t)ncols > h->c) return fail(ctx, GL_E_ARG, "gl_commit_add_coeffs: bad column range");
     Guard g(ctx);
     const u64 n = (u64)1 << h->log_n;
-    CK(cudaMemcpyAsync(h->coeffs + (size_t)col0 * n, coeffs, (size_t)ncols * n * 8,
+    CK(cudaMemcpyAsync(h->coeffs.get() + (size_t)col0 * n, coeffs, (size_t)ncols * n * 8,
                        space == GL_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, ctx->stream));
     TRY(commit_lde_columns(ctx, h, col0, ncols));
     h->cols_added += ncols;
@@ -1565,12 +1568,7 @@ extern "C" int gl_commit_finish(gl_commit* h, uint64_t* cap_out, int space) {
     TRY(commit_tree(ctx, h, cap_out, space, h->stream_hash && h->hashed_cols == h->c));
     TRY(finish(ctx));
     h->finished = true;
-    if (h->hstate) {
-        dev_release(ctx, h->hstate, h->hstate_bytes);
-        h->hstate = nullptr;
-    }
-    for (int i = 0; i < GL_PHASES; i++) cudaEventElapsedTime(&ctx->phase_ms[i], ctx->ev[i], ctx->ev[i + 1]);
-    ctx->ev_valid = true;
+    commit_done(ctx, h);
     return GL_OK;
 }
 
@@ -1579,8 +1577,7 @@ extern "C" void gl_commit_free(gl_commit* h) {
     gl_ctx* ctx = h->ctx;
     Guard g(ctx);
     cudaStreamSynchronize(ctx->stream);
-    ctx->live_commits--;
-    commit_release(h);
+    delete h;
 }
 
 extern "C" int gl_commit_info(const gl_commit* h, uint32_t* log_n, uint32_t* c, uint32_t* rate_bits,
@@ -1598,18 +1595,18 @@ extern "C" int gl_commit_info(const gl_commit* h, uint32_t* log_n, uint32_t* c, 
 extern "C" int gl_commit_device_ptrs(const gl_commit* h, const uint64_t** lde_cols, uint64_t* ld,
                                      const uint64_t** digests) {
     if (!h) return GL_E_ARG;
-    if (lde_cols) *lde_cols = h->lde;
+    if (lde_cols) *lde_cols = h->lde.get();
     if (ld) *ld = h->n_local;
-    if (digests) *digests = h->digests;
+    if (digests) *digests = h->digests.get();
     return GL_OK;
 }
 
 extern "C" int gl_commit_coeffs(gl_commit* h, uint64_t* coeffs_out, int space) {
     if (!h || !coeffs_out) return GL_E_ARG;
     gl_ctx* ctx = h->ctx;
-    if (!h->coeffs) return fail(ctx, GL_E_STATE, "gl_commit_coeffs: this handle has no polynomials (FRI layer tree)");
+    if (!h->coeffs.get()) return fail(ctx, GL_E_STATE, "gl_commit_coeffs: this handle has no polynomials (FRI layer tree)");
     Guard g(ctx);
-    TRY(copy_out(ctx, coeffs_out, h->coeffs, ((size_t)h->c << h->log_n) * 8, space));
+    TRY(copy_out(ctx, coeffs_out, h->coeffs.get(), ((size_t)h->c << h->log_n) * 8, space));
     return finish(ctx);
 }
 
@@ -1617,7 +1614,7 @@ extern "C" int gl_commit_coeffs(gl_commit* h, uint64_t* coeffs_out, int space) {
 extern "C" int gl_commit_eval(gl_commit* h, const uint64_t point[2], uint64_t* values_out, int space) {
     if (!h || !point || !values_out) return GL_E_ARG;
     gl_ctx* ctx = h->ctx;
-    if (!h->coeffs) return fail(ctx, GL_E_STATE, "gl_commit_eval: this handle has no polynomials (FRI layer tree)");
+    if (!h->coeffs.get()) return fail(ctx, GL_E_STATE, "gl_commit_eval: this handle has no polynomials (FRI layer tree)");
     if (!h->finished && h->cols_added != h->c) return fail(ctx, GL_E_STATE, "gl_commit_eval: not every polynomial has been added");
     Guard g(ctx);
     const u64 n = (u64)1 << h->log_n;
@@ -1629,7 +1626,7 @@ extern "C" int gl_commit_eval(gl_commit* h, const uint64_t point[2], uint64_t* v
     TRY(scratch_get(ctx, 0, ((size_t)h->c * chunks + h->c) * 16, &d));
     u64* partial = (u64*)d;
     u64* d_out = space == GL_DEVICE ? values_out : partial + 2 * (size_t)h->c * chunks;
-    launch_eval_at(h->coeffs, n, h->c, zz, z2, z3, partial, d_out, ctx->stream);
+    launch_eval_at(h->coeffs.get(), n, h->c, zz, z2, z3, partial, d_out, ctx->stream);
     if (space == GL_HOST) TRY(copy_out(ctx, values_out, d_out, (size_t)h->c * 16, GL_HOST));
     return finish(ctx);
 }
@@ -1639,16 +1636,16 @@ extern "C" int gl_commit_download(gl_commit* h, uint64_t* leaves_out, uint64_t* 
     gl_ctx* ctx = h->ctx;
     if (!h->finished) return fail(ctx, GL_E_STATE, "gl_commit_download: gl_commit_finish has not run yet");
     Guard g(ctx);
-    if (digests_out) TRY(copy_out(ctx, digests_out, h->digests, h->num_digests * 32, space));
+    if (digests_out) TRY(copy_out(ctx, digests_out, h->digests.get(), h->num_digests * 32, space));
     if (leaves_out) {
         if (space == GL_DEVICE) {
-            launch_transpose_to_rows(h->lde, h->n_local, leaf_len(h), 0, h->n_local, leaves_out, ctx->stream);
+            launch_transpose_to_rows(h->lde.get(), h->n_local, leaf_len(h), 0, h->n_local, leaves_out, ctx->stream);
         } else {
             const u64 chunk = h->n_local < ((u64)1 << 16) ? h->n_local : ((u64)1 << 16);
             void* stage;
             TRY(scratch_get(ctx, 0, (size_t)chunk * leaf_len(h) * 8, &stage));
             for (u64 r0 = 0; r0 < h->n_local; r0 += chunk) {
-                launch_transpose_to_rows(h->lde, h->n_local, leaf_len(h), r0, chunk, (u64*)stage, ctx->stream);
+                launch_transpose_to_rows(h->lde.get(), h->n_local, leaf_len(h), r0, chunk, (u64*)stage, ctx->stream);
                 TRY(copy_out(ctx, leaves_out + (size_t)r0 * leaf_len(h), stage, (size_t)chunk * leaf_len(h) * 8, GL_HOST));
                 CK(cudaStreamSynchronize(ctx->stream));   // `stage` is reused by the next chunk
             }
@@ -1704,7 +1701,7 @@ extern "C" int gl_commit_open(gl_commit* h, const uint64_t* leaf_indices, uint32
             TRY(scratch_get(ctx, 0, (size_t)k * leaf_len(h) * 8, &t));
             d_rows = (u64*)t;
         }
-        launch_gather_rows(h->lde, h->n_local, leaf_len(h), d_idx, k, d_rows, ctx->stream);
+        launch_gather_rows(h->lde.get(), h->n_local, leaf_len(h), d_idx, k, d_rows, ctx->stream);
         TRY(copy_out(ctx, rows_out, d_rows, (size_t)k * leaf_len(h) * 8, space));
     }
     if (paths_out && sub_bits) {
@@ -1714,7 +1711,7 @@ extern "C" int gl_commit_open(gl_commit* h, const uint64_t* leaf_indices, uint32
             TRY(scratch_get(ctx, 1, (size_t)k * sub_bits * 32, &t));
             d_paths = (u64*)t;
         }
-        launch_gather_paths(h->digests, sub_bits, d_idx, k, d_paths, ctx->stream);
+        launch_gather_paths(h->digests.get(), sub_bits, d_idx, k, d_paths, ctx->stream);
         TRY(copy_out(ctx, paths_out, d_paths, (size_t)k * sub_bits * 32, space));
     }
     return finish(ctx);
@@ -1747,7 +1744,7 @@ extern "C" int gl_commit_get_lde_values(gl_commit* h, const uint64_t* indices, u
         TRY(scratch_get(ctx, 0, (size_t)k * h->c * 8, &t));
         d_rows = (u64*)t;
     }
-    launch_gather_rows(h->lde, h->n_local, h->c, d_idx, k, d_rows, ctx->stream);
+    launch_gather_rows(h->lde.get(), h->n_local, h->c, d_idx, k, d_rows, ctx->stream);
     TRY(copy_out(ctx, rows_out, d_rows, (size_t)k * h->c * 8, space));
     return finish(ctx);
 }
@@ -1781,6 +1778,24 @@ extern "C" int gl_fri_layer_tree(gl_ctx* ctx, const uint64_t* values_ext, uint64
     return finish(ctx);
 }
 
+// A FRI layer tree kept on the device: the leaves are the arity-sized cosets of `values` ([2^lg][2] extension
+// elements on the device), 2 << arity_bits columns each, with no polynomials behind the handle
+static int fri_tree_new(gl_ctx* ctx, const u64* values, unsigned lg, unsigned arity_bits, uint32_t cap_height,
+                        std::unique_ptr<gl_commit>* out) {
+    std::unique_ptr<gl_commit> t(new (std::nothrow) gl_commit());
+    if (!t) return fail(ctx, GL_E_OOM, "host allocation failed");
+    t->ctx = ctx; t->log_n = lg - arity_bits; t->c = 2u << arity_bits; t->rate_bits = 0; t->cap_height = cap_height;
+    t->n_local = (u64)1 << t->log_n; t->cap_local_bits = cap_height;
+    t->num_digests = 2 * (t->n_local - ((u64)1 << cap_height));
+    TRY(t->lde.alloc(ctx, (size_t)16 << lg));
+    TRY(t->digests.alloc(ctx, t->num_digests * 32));
+    TRY(t->cap.alloc(ctx, (size_t)32 << cap_height));
+    launch_fri_leaves(values, lg, arity_bits, t->lde.get(), ctx->stream);
+    launch_merkle_cols(t->lde.get(), t->n_local, t->c, t->log_n, cap_height, t->digests.get(), t->cap.get(), ctx->stream);
+    *out = std::move(t);
+    return GL_OK;
+}
+
 extern "C" int gl_fri_layer_commit(gl_ctx* ctx, const uint64_t* values_ext, uint64_t len, uint32_t arity_bits,
                                    uint32_t cap_height, uint64_t* cap_out, gl_commit** handle, int space) {
     if (!ctx) return GL_E_ARG;
@@ -1793,37 +1808,13 @@ extern "C" int gl_fri_layer_commit(gl_ctx* ctx, const uint64_t* values_ext, uint
         return fail(ctx, GL_E_ARG, "MerkleTree::new: cap_height must be at most log2(leaves.len())");
     if (!values_ext) return fail(ctx, GL_E_ARG, "gl_fri_layer_commit: NULL buffer");
     Guard g(ctx);
-    gl_commit* h = new (std::nothrow) gl_commit();
-    if (!h) return fail(ctx, GL_E_OOM, "host allocation failed");
-    h->ctx = ctx;
-    h->log_n = lg - arity_bits;
-    h->c = 2u << arity_bits;
-    h->rate_bits = 0;
-    h->cap_height = cap_height;
-    h->n_local = len >> arity_bits;
-    h->cap_local_bits = cap_height;
-    h->num_digests = 2 * (h->n_local - ((u64)1 << cap_height));
-    h->lde_bytes = len * 16;
-    h->digests_bytes = h->num_digests * 32;
-    h->cap_bytes = (size_t)32 << cap_height;
-    int rc = dev_alloc(ctx, h->lde_bytes, &h->lde);
-    if (rc == GL_OK) rc = dev_alloc(ctx, h->digests_bytes, &h->digests);
-    if (rc == GL_OK) rc = dev_alloc(ctx, h->cap_bytes, &h->cap);
-    const u64* dv = nullptr;
-    if (rc == GL_OK) rc = stage_in(ctx, values_ext, len * 16, space, 0, &dv);
-    if (rc == GL_OK) {
-        launch_fri_leaves(dv, lg, arity_bits, h->lde, ctx->stream);
-        launch_merkle_cols(h->lde, h->n_local, h->c, h->log_n, cap_height, h->digests, h->cap, ctx->stream);
-        rc = copy_out(ctx, cap_out, h->cap, h->cap_bytes, space);
-    }
-    if (rc == GL_OK) rc = finish(ctx);
-    if (rc != GL_OK) {
-        cudaStreamSynchronize(ctx->stream);
-        commit_release(h);
-        return rc;
-    }
-    ctx->live_commits++;
-    *handle = h;
+    const u64* dv;
+    TRY(stage_in(ctx, values_ext, len * 16, space, 0, &dv));
+    std::unique_ptr<gl_commit> h;
+    TRY(fri_tree_new(ctx, dv, lg, arity_bits, cap_height, &h));
+    TRY(copy_out(ctx, cap_out, h->cap.get(), h->cap.bytes(), space));
+    TRY(finish(ctx));
+    *handle = h.release();
     return GL_OK;
 }
 
@@ -1871,7 +1862,7 @@ static int fri_final_poly_device(gl_ctx* ctx, gl_commit* const* oracles, uint32_
         return fail(ctx, GL_E_ARG, "gl_fri_final_poly: NULL or empty argument");
     const uint32_t log_n = oracles[0]->log_n;
     for (uint32_t i = 0; i < num_oracles; i++) {
-        if (!oracles[i] || oracles[i]->ctx != ctx || !oracles[i]->coeffs)
+        if (!oracles[i] || oracles[i]->ctx != ctx || !oracles[i]->coeffs.get())
             return fail(ctx, GL_E_STATE, "gl_fri_final_poly: oracle is not a polynomial commit of this ctx");
         if (oracles[i]->log_n != log_n) return fail(ctx, GL_E_ARG, "gl_fri_final_poly: oracles of different degree");
     }
@@ -1910,7 +1901,7 @@ static int fri_final_poly_device(gl_ctx* ctx, gl_commit* const* oracles, uint32_
         glh::ext cur = {1, 0};
         for (uint32_t j = 0; j < k; j++) {
             const gl_fri_poly& fp = polys[batches[b].first_poly + j];
-            host_tab[j] = (u64)(uintptr_t)(oracles[fp.oracle_index]->coeffs + (size_t)fp.polynomial_index * n);
+            host_tab[j] = (u64)(uintptr_t)(oracles[fp.oracle_index]->coeffs.get() + (size_t)fp.polynomial_index * n);
             host_tab[k + 2 * j] = cur.a;
             host_tab[k + 2 * j + 1] = cur.b;
             cur = glh::ext_mul(cur, al);
@@ -1991,7 +1982,7 @@ extern "C" int gl_fri_prove(gl_ctx* ctx, gl_commit* const* oracles, uint32_t num
         prm->proof_of_work_bits > 48)
         return fail(ctx, GL_E_ARG, "gl_fri_prove: unsupported FRI parameters");
     for (uint32_t i = 0; i < num_oracles; i++)
-        if (!oracles[i] || oracles[i]->ctx != ctx || !oracles[i]->coeffs || !oracles[i]->finished || oracles[i]->shard_count != 1 ||
+        if (!oracles[i] || oracles[i]->ctx != ctx || !oracles[i]->coeffs.get() || !oracles[i]->finished || oracles[i]->shard_count != 1 ||
             oracles[i]->rate_bits != prm->rate_bits || oracles[i]->cap_height != prm->cap_height || oracles[i]->log_n != oracles[0]->log_n)
             return fail(ctx, GL_E_STATE, "gl_fri_prove: every oracle must be a finished, unsharded polynomial commit of this ctx with the FRI config's rate_bits / cap_height");
     const uint32_t degree_bits = oracles[0]->log_n, rate_bits = prm->rate_bits, h = prm->cap_height, rounds = prm->num_query_rounds;
@@ -2008,29 +1999,12 @@ extern "C" int gl_fri_prove(gl_ctx* ctx, gl_commit* const* oracles, uint32_t num
     const uint32_t layers = prm->num_reduction_layers;
     // device state: challenger | alpha/beta scratch [2] | query challenges [rounds] | pow state [12] | pow best | response |
     // cumulative arity bits | query indices [(layers + 1)][rounds]
-    u64* d_state;
-    const size_t state_words = 32 + 2 + rounds + 12 + 2 + GL_FRI_MAX_LAYERS + (size_t)(layers + 1) * rounds;
-    TRY(dev_alloc(ctx, state_words * 8, &d_state));
-    u64* d_proof = nullptr;
-    std::vector<gl_commit*> trees;
-    auto cleanup = [&](int rc) {
-        cudaStreamSynchronize(ctx->stream);
-        for (auto* t : trees) commit_release(t);
-        dev_release(ctx, d_state, state_words * 8);
-        if (d_proof) dev_release(ctx, d_proof, words * 8);
-        return rc;
-    };
-#define FTRY(expr)                         \
-    do {                                   \
-        int rc__ = (expr);                 \
-        if (rc__) return cleanup(rc__);    \
-    } while (0)
-#define FCK(call)                                                            \
-    do {                                                                     \
-        cudaError_t e__ = (call);                                            \
-        if (e__ != cudaSuccess) return cleanup(cuda_fail(ctx, e__, #call));  \
-    } while (0)
-    FTRY(dev_alloc(ctx, words * 8, &d_proof));
+    PoolBuf state, proof;
+    TRY(state.alloc(ctx, (32 + 2 + rounds + 12 + 2 + GL_FRI_MAX_LAYERS + (size_t)(layers + 1) * rounds) * 8));
+    TRY(proof.alloc(ctx, words * 8));
+    u64* d_state = state.get();
+    u64* d_proof = proof.get();
+    std::vector<std::unique_ptr<gl_commit>> trees;
     static_assert(sizeof(gl_challenger) == 29 * 8, "gl_challenger layout");
     gl_challenger* d_ch = (gl_challenger*)d_state;
     u64* d_ab = d_state + 32;
@@ -2040,67 +2014,56 @@ extern "C" int gl_fri_prove(gl_ctx* ctx, gl_commit* const* oracles, uint32_t num
     u64* d_resp = d_pow_state + 13;
     uint32_t* d_cum = (uint32_t*)(d_pow_state + 14);
     u64* d_idx = d_pow_state + 14 + GL_FRI_MAX_LAYERS;
-    FCK(cudaMemcpyAsync(d_ch, challenger, sizeof(gl_challenger), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_ch, challenger, sizeof(gl_challenger), cudaMemcpyHostToDevice, ctx->stream));
     // ---- alpha = challenger.get_extension_challenge(): the only challenge the host needs (power tables of the reduction)
     u64 alpha[2];
     launch_challenger_step(d_ch, nullptr, 0, d_ab, 2, nullptr, ctx->stream);
-    FCK(cudaMemcpyAsync(alpha, d_ab, 16, cudaMemcpyDeviceToHost, ctx->stream));
-    FCK(cudaStreamSynchronize(ctx->stream));
+    CK(cudaMemcpyAsync(alpha, d_ab, 16, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
     u64 *d_coeffs, *d_values;
-    FTRY(fri_final_poly_device(ctx, oracles, num_oracles, batches, num_batches, polys, alpha, rate_bits,
-                               ((prm->flags | ctx->compat) & GL_COMPAT_FRI_FINAL_POLY_TIMES_X) != 0, true, &d_coeffs, &d_values));
+    TRY(fri_final_poly_device(ctx, oracles, num_oracles, batches, num_batches, polys, alpha, rate_bits,
+                              ((prm->flags | ctx->compat) & GL_COMPAT_FRI_FINAL_POLY_TIMES_X) != 0, true, &d_coeffs, &d_values));
     // ---- fri_committed_trees: per layer tree -> observe cap -> beta -> fold -> coset_fft, no host involvement
     u64 len = N;
     unsigned lg = lgN;
     u64 off = 0;                 // write position in the proof buffer
     u64 shift = 7;
     u64 *cur_coeffs = d_coeffs, *cur_values = d_values;
-    u64 *owned_a = nullptr, *owned_b = nullptr;   // folded buffers of the previous layer
-    size_t owned_bytes = 0;
+    PoolBuf folded_coeffs, folded_values;   // the previous layer's fold
     uint32_t cum[GL_FRI_MAX_LAYERS] = {}, acc_bits = 0;
     for (uint32_t l = 0; l < layers; l++) {
         const unsigned ab = prm->reduction_arity_bits[l];
-        gl_commit* t = new (std::nothrow) gl_commit();
-        if (!t) return cleanup(fail(ctx, GL_E_OOM, "host allocation failed"));
-        trees.push_back(t);
-        t->ctx = ctx; t->log_n = lg - ab; t->c = 2u << ab; t->rate_bits = 0; t->cap_height = h;
-        t->n_local = len >> ab; t->cap_local_bits = h;
-        t->num_digests = 2 * (t->n_local - ((u64)1 << h));
-        t->lde_bytes = len * 16; t->digests_bytes = t->num_digests * 32; t->cap_bytes = (size_t)32 << h;
-        FTRY(dev_alloc(ctx, t->lde_bytes, &t->lde));
-        FTRY(dev_alloc(ctx, t->digests_bytes, &t->digests));
-        FTRY(dev_alloc(ctx, t->cap_bytes, &t->cap));
-        launch_fri_leaves(cur_values, lg, ab, t->lde, ctx->stream);
-        launch_merkle_cols(t->lde, t->n_local, t->c, t->log_n, h, t->digests, t->cap, ctx->stream);
-        FCK(cudaMemcpyAsync(d_proof + off, t->cap, t->cap_bytes, cudaMemcpyDeviceToDevice, ctx->stream));
+        std::unique_ptr<gl_commit> t;
+        TRY(fri_tree_new(ctx, cur_values, lg, ab, h, &t));
+        CK(cudaMemcpyAsync(d_proof + off, t->cap.get(), t->cap.bytes(), cudaMemcpyDeviceToDevice, ctx->stream));
         off += 4ull << h;
-        launch_challenger_step(d_ch, t->cap, 4u << h, d_ab, 2, nullptr, ctx->stream);   // observe_cap, beta
+        launch_challenger_step(d_ch, t->cap.get(), 4u << h, d_ab, 2, nullptr, ctx->stream);   // observe_cap, beta
+        trees.push_back(std::move(t));
         shift = glh::pow(shift, (u64)1 << ab);
         const u64 out_len = len >> ab;
-        u64 *n_coeffs, *n_values;
-        FTRY(dev_alloc(ctx, out_len * 16, &n_coeffs));
-        FTRY(dev_alloc(ctx, out_len * 16, &n_values));
+        PoolBuf n_coeffs, n_values;
+        TRY(n_coeffs.alloc(ctx, out_len * 16));
+        TRY(n_values.alloc(ctx, out_len * 16));
         void* dcols;
-        FTRY(scratch_get(ctx, 2, out_len * 16, &dcols));
+        TRY(scratch_get(ctx, 2, out_len * 16, &dcols));
         launch_fri_fold_dev(cur_coeffs, out_len, ab, d_ab, (u64*)dcols, out_len, ctx->stream);
-        launch_interleave2((const u64*)dcols, out_len, out_len, n_coeffs, ctx->stream);
+        launch_interleave2((const u64*)dcols, out_len, out_len, n_coeffs.get(), ctx->stream);
         const u64* pre;
-        FTRY(pow_table(ctx, shift, &pre));
-        FTRY(transform_natural(ctx, (u64*)dcols, lg - ab, 2, false, pre, nullptr));
-        launch_interleave2((const u64*)dcols, out_len, out_len, n_values, ctx->stream);
-        if (owned_a) { dev_release(ctx, owned_a, owned_bytes); dev_release(ctx, owned_b, owned_bytes); }   // stream-ordered reuse
-        owned_a = n_coeffs; owned_b = n_values; owned_bytes = out_len * 16;
-        cur_coeffs = n_coeffs; cur_values = n_values;
+        TRY(pow_table(ctx, shift, &pre));
+        TRY(transform_natural(ctx, (u64*)dcols, lg - ab, 2, false, pre, nullptr));
+        launch_interleave2((const u64*)dcols, out_len, out_len, n_values.get(), ctx->stream);
+        cur_coeffs = n_coeffs.get(); cur_values = n_values.get();
+        folded_coeffs = std::move(n_coeffs);   // the fold before goes back to the pool: stream-ordered reuse
+        folded_values = std::move(n_values);
         len = out_len; lg -= ab;
         acc_bits += ab;
         cum[l] = acc_bits;
     }
     // final_poly: "the coefficients being removed here are always zero"
     const u64 final_len = len >> rate_bits;
-    FCK(cudaMemcpyAsync(d_proof + off, cur_coeffs, final_len * 16, cudaMemcpyDeviceToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_proof + off, cur_coeffs, final_len * 16, cudaMemcpyDeviceToDevice, ctx->stream));
     launch_challenger_step(d_ch, d_proof + off, (uint32_t)(2 * final_len), nullptr, 0, d_pow_state, ctx->stream);
     off += 2 * final_len;
-    if (owned_a) { dev_release(ctx, owned_a, owned_bytes); dev_release(ctx, owned_b, owned_bytes); }
     // ---- fri_proof_of_work: smallest witness; the input position is the number of pending inputs, which the host can count
     uint32_t pending = challenger->input_len;   // replay the buffer lengths of the transcript so far (values stay on the device)
     {
@@ -2112,7 +2075,7 @@ extern "C" int gl_fri_prove(gl_ctx* ctx, gl_commit* const* oracles, uint32_t num
     }
     const unsigned min_lz = prm->proof_of_work_bits;   // + (64 - F::order().bits()) = + 0
     const unsigned long long none = ~0ULL;
-    FCK(cudaMemcpyAsync(d_best, &none, 8, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_best, &none, 8, cudaMemcpyHostToDevice, ctx->stream));
     u64 witness = 0;
     {
         unsigned lg_chunk = min_lz + 2 < 14 ? 14 : (min_lz + 2 > 24 ? 24 : min_lz + 2);
@@ -2122,50 +2085,49 @@ extern "C" int gl_fri_prove(gl_ctx* ctx, gl_commit* const* oracles, uint32_t num
             u64 count = GL_P - start < chunk ? GL_P - start : chunk;
             launch_pow_grind(d_pow_state, pending, 7, min_lz, start, count, d_best, ctx->stream);
             unsigned long long best;
-            FCK(cudaMemcpyAsync(&best, d_best, 8, cudaMemcpyDeviceToHost, ctx->stream));
-            FCK(cudaStreamSynchronize(ctx->stream));
+            CK(cudaMemcpyAsync(&best, d_best, 8, cudaMemcpyDeviceToHost, ctx->stream));
+            CK(cudaStreamSynchronize(ctx->stream));
             if (best != none) { witness = best; found = true; }
             else if (start >= ((u64)1 << 40)) break;
         }
-        if (!found) return cleanup(fail(ctx, GL_E_STATE, "fri_proof_of_work: no witness found"));
+        if (!found) return fail(ctx, GL_E_STATE, "fri_proof_of_work: no witness found");
     }
     // observe the witness, recompute the response with the normal Challenger code (as upstream does), then the query indices
     launch_challenger_step(d_ch, (const u64*)d_best, 1, d_resp, 1, nullptr, ctx->stream);
-    FCK(cudaMemcpyAsync(d_proof + off, d_best, 8, cudaMemcpyDeviceToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_proof + off, d_best, 8, cudaMemcpyDeviceToDevice, ctx->stream));
     off += 1;
     launch_challenger_step(d_ch, nullptr, 0, d_qch, rounds, nullptr, ctx->stream);
-    FCK(cudaMemcpyAsync(d_cum, cum, sizeof cum, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_cum, cum, sizeof cum, cudaMemcpyHostToDevice, ctx->stream));
     uint64_t query_stride = 1;
     for (uint32_t i = 0; i < num_oracles; i++) query_stride += leaf_len(oracles[i]) + 4ull * (lgN - h);
-    for (auto* t : trees) query_stride += t->c + 4ull * (t->log_n - h);
+    for (auto& t : trees) query_stride += t->c + 4ull * (t->log_n - h);
     u64* d_queries = d_proof + off;
     launch_fri_query_indices(d_qch, rounds, lgN, d_cum, layers, d_idx, d_queries, query_stride, ctx->stream);
     u64 qoff = 1;
     for (uint32_t i = 0; i < num_oracles; i++) {
         const gl_commit* o = oracles[i];
-        launch_gather_proof(o->lde, o->n_local, leaf_len(o), o->digests, lgN - h, d_idx, rounds, d_queries + qoff, query_stride, ctx->stream);
+        launch_gather_proof(o->lde.get(), o->n_local, leaf_len(o), o->digests.get(), lgN - h, d_idx, rounds, d_queries + qoff,
+                            query_stride, ctx->stream);
         qoff += leaf_len(o) + 4ull * (lgN - h);
     }
     for (uint32_t l = 0; l < layers; l++) {
-        const gl_commit* t = trees[l];
-        launch_gather_proof(t->lde, t->n_local, t->c, t->digests, t->log_n - h, d_idx + (size_t)(l + 1) * rounds, rounds,
+        const gl_commit* t = trees[l].get();
+        launch_gather_proof(t->lde.get(), t->n_local, t->c, t->digests.get(), t->log_n - h, d_idx + (size_t)(l + 1) * rounds, rounds,
                             d_queries + qoff, query_stride, ctx->stream);
         qoff += t->c + 4ull * (t->log_n - h);
     }
     off += query_stride * rounds;
-    if (off != words) return cleanup(fail(ctx, GL_E_STATE, "gl_fri_prove: internal size mismatch"));
+    if (off != words) return fail(ctx, GL_E_STATE, "gl_fri_prove: internal size mismatch");
     u64 response = 0;
-    FCK(cudaMemcpyAsync(proof_out, d_proof, words * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    FCK(cudaMemcpyAsync(challenger, d_ch, sizeof(gl_challenger), cudaMemcpyDeviceToHost, ctx->stream));
-    FCK(cudaMemcpyAsync(&response, d_resp, 8, cudaMemcpyDeviceToHost, ctx->stream));
-    FCK(cudaStreamSynchronize(ctx->stream));
-    FCK(cudaGetLastError());
+    CK(cudaMemcpyAsync(proof_out, d_proof, words * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(challenger, d_ch, sizeof(gl_challenger), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&response, d_resp, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    CK(cudaGetLastError());
     if (min_lz && (response >> (64 - min_lz)) != 0)
-        return cleanup(fail(ctx, GL_E_STATE, "fri_proof_of_work: response does not have the required leading zeros"));
+        return fail(ctx, GL_E_STATE, "fri_proof_of_work: response does not have the required leading zeros");
     (void)witness;
-    return cleanup(GL_OK);
-#undef FTRY
-#undef FCK
+    return GL_OK;
 }
 
 extern "C" int gl_ctx_set_compat(gl_ctx* ctx, uint32_t flags) {
@@ -2193,7 +2155,7 @@ extern "C" int gl_quotient_polys(gl_ctx* ctx, const gl_circuit* cd, const gl_gat
     const uint32_t qdb = ilog2(deg), lg_n = cd->degree_bits;
     gl_commit* cm[3] = {constants_sigmas, wires, zs_pp};
     for (auto* h : cm) {
-        if (h->ctx != ctx || !h->finished || !h->lde) return fail(ctx, GL_E_STATE, "gl_quotient_polys: oracle is not a finished commit of this ctx");
+        if (h->ctx != ctx || !h->finished || !h->lde.get()) return fail(ctx, GL_E_STATE, "gl_quotient_polys: oracle is not a finished commit of this ctx");
         if (h->log_n != lg_n || h->rate_bits != wires->rate_bits) return fail(ctx, GL_E_ARG, "gl_quotient_polys: oracles of different degree or rate");
         if (h->shard_count != 1) return fail(ctx, GL_E_ARG, "gl_quotient_polys: sharded oracles are not supported");
     }
@@ -2244,9 +2206,9 @@ extern "C" int gl_quotient_polys(gl_ctx* ctx, const gl_circuit* cd, const gl_gat
     CK(cudaMemcpyAsync(d_tab, tab.data(), tab.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
     const u64* xtab;
     TRY(pow_table(ctx, glh::root_of_unity(lg_n + qdb), &xtab));
-    a.cs = constants_sigmas->lde; a.cs_ld = constants_sigmas->n_local;
-    a.wires = wires->lde; a.w_ld = wires->n_local;
-    a.zs = zs_pp->lde; a.z_ld = zs_pp->n_local;
+    a.cs = constants_sigmas->lde.get(); a.cs_ld = constants_sigmas->n_local;
+    a.wires = wires->lde.get(); a.w_ld = wires->n_local;
+    a.zs = zs_pp->lde.get(); a.z_ld = zs_pp->n_local;
     a.lg_lde = lg_n + qdb; a.qdb = qdb; a.nch = nch; a.R = R; a.deg = deg; a.chunks = chunks; a.num_prods = num_prods;
     a.num_constants = cd->num_constants; a.num_selectors = cd->num_selectors; a.num_gates = cd->num_gates;
     a.nterms = nterms; a.gate_term0 = nch * (1 + chunks);
@@ -2291,7 +2253,7 @@ extern "C" int gl_permutation_zs(gl_ctx* ctx, const gl_circuit* cd, const uint64
     if (nch * chunks > PERM_MAX_SLOTS)
         return fail(ctx, GL_E_ARG, "gl_permutation_zs: num_challenges * ceil(num_routed_wires / quotient_degree_factor) > 64");
     for (gl_commit* h : {constants_sigmas, wires}) {
-        if (h->ctx != ctx || !h->finished || !h->coeffs)
+        if (h->ctx != ctx || !h->finished || !h->coeffs.get())
             return fail(ctx, GL_E_STATE, "gl_permutation_zs: oracle is not a finished polynomial commit of this ctx");
         if (h->shard_count != 1) return fail(ctx, GL_E_ARG, "gl_permutation_zs: sharded oracles are not supported");
     }
@@ -2322,34 +2284,27 @@ extern "C" int gl_permutation_zs(gl_ctx* ctx, const gl_circuit* cd, const uint64
     if (space == GL_HOST) TRY(scratch_get(ctx, 4, out_bytes, &d_out));
     // the routed wire and sigma values: forward transforms of the coefficient columns (the salt of a blinded commit
     // lives only in its leaves).  The transforms run through scratch slot 1.
-    const size_t rec_bytes = (size_t)2 * R * n * 8;
-    u64* d_rec;
-    TRY(dev_alloc(ctx, rec_bytes, &d_rec));
-    int rc = transform_natural(ctx, d_rec, lg_n, R, false, nullptr, nullptr, wires->coeffs);
-    if (rc == GL_OK)
-        rc = transform_natural(ctx, d_rec + (size_t)R * n, lg_n, R, false, nullptr, nullptr,
-                               constants_sigmas->coeffs + (size_t)cd->num_constants * n);
+    PoolBuf rec;
+    TRY(rec.alloc(ctx, (size_t)2 * R * n * 8));
+    u64* d_rec = rec.get();
+    TRY(transform_natural(ctx, d_rec, lg_n, R, false, nullptr, nullptr, wires->coeffs.get()));
+    TRY(transform_natural(ctx, d_rec + (size_t)R * n, lg_n, R, false, nullptr, nullptr,
+                          constants_sigmas->coeffs.get() + (size_t)cd->num_constants * n));
+    perm_args a;
+    memset(&a, 0, sizeof a);
+    a.wires = d_rec; a.sigmas = d_rec + (size_t)R * n; a.k_is = d_k; a.xtab = xtab;
+    a.out = (u64*)d_out; a.cta = d_cta; a.grand = d_grand; a.zero_den = d_flag;
+    a.n = n; a.R = R; a.deg = deg; a.chunks = chunks; a.nch = nch; a.nblocks = nblocks;
+    for (uint32_t c = 0; c < nch; c++) { a.betas[c] = glh::canon(betas[c]); a.gammas[c] = glh::canon(gammas[c]); }
+    cudaError_t e = launch_permutation_zs(a, ctx->stream);
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "launch_permutation_zs");
     u64 grand[PERM_MAX_CHALLENGES];
     unsigned zero_den = 0;
-    if (rc == GL_OK) {
-        perm_args a;
-        memset(&a, 0, sizeof a);
-        a.wires = d_rec; a.sigmas = d_rec + (size_t)R * n; a.k_is = d_k; a.xtab = xtab;
-        a.out = (u64*)d_out; a.cta = d_cta; a.grand = d_grand; a.zero_den = d_flag;
-        a.n = n; a.R = R; a.deg = deg; a.chunks = chunks; a.nch = nch; a.nblocks = nblocks;
-        for (uint32_t c = 0; c < nch; c++) { a.betas[c] = glh::canon(betas[c]); a.gammas[c] = glh::canon(gammas[c]); }
-        cudaError_t e = launch_permutation_zs(a, ctx->stream);
-        if (e != cudaSuccess) rc = cuda_fail(ctx, e, "launch_permutation_zs");
-    }
-    if (rc == GL_OK) {
-        cudaError_t e = cudaMemcpyAsync(grand, d_grand, nch * 8, cudaMemcpyDeviceToHost, ctx->stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(&zero_den, d_flag, sizeof zero_den, cudaMemcpyDeviceToHost, ctx->stream);
-        if (e != cudaSuccess) rc = cuda_fail(ctx, e, "download grand products");
-    }
-    if (rc == GL_OK && space == GL_HOST) rc = copy_out(ctx, zs_partial_products_out, d_out, out_bytes, GL_HOST);
-    if (rc == GL_OK) rc = finish(ctx);
-    dev_release(ctx, d_rec, rec_bytes);
-    if (rc != GL_OK) return rc;
+    e = cudaMemcpyAsync(grand, d_grand, nch * 8, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&zero_den, d_flag, sizeof zero_den, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "download grand products");
+    if (space == GL_HOST) TRY(copy_out(ctx, zs_partial_products_out, d_out, out_bytes, GL_HOST));
+    TRY(finish(ctx));
     if (zero_den)
         return fail(ctx, GL_E_ARG, "gl_permutation_zs: wire + beta * sigma + gamma is zero at some row "
                                    "(batch_multiplicative_inverse of a zero denominator)");

@@ -579,48 +579,47 @@ static int group_commit(gl_group* g, const uint64_t* const* inputs, bool is_valu
     int prev = -1;
     cudaGetDevice(&prev);
     struct Restore { int d; ~Restore() { if (d >= 0) cudaSetDevice(d); } } restore{prev};
-    std::vector<gl_commit*> hs(nl, nullptr);
-    auto bail = [&](int rc) {
-        for (uint32_t i = 0; i < nl; i++) {
-            gl_ctx* ctx = g->r[i].ctx;
-            cudaSetDevice(ctx->device);
-            cudaStreamSynchronize(ctx->stream);
-            cudaStreamSynchronize(g->r[i].comm_stream);
-            cudaStreamSynchronize(g->r[i].prep_stream);
-            cudaStreamSynchronize(ctx->h2d_stream);
-            cudaStreamSynchronize(ctx->d2h_stream);
-            cudaGetLastError();
-            if (hs[i]) commit_release(hs[i]);
+    // Handles still held when this function returns belong to a failed commit.  `bail` drops them rank by rank, with the
+    // rank's device current, once nothing the rank queued (its streams, the coefficient downloads) can use their blocks.
+    std::vector<std::unique_ptr<gl_commit>> hs(nl);
+    struct Bail {
+        gl_group* g;
+        std::vector<std::unique_ptr<gl_commit>>& hs;
+        int space;
+        ~Bail() {
+            for (uint32_t i = 0; i < hs.size(); i++) {
+                if (!hs[i]) continue;
+                gl_ctx* ctx = g->r[i].ctx;
+                cudaSetDevice(ctx->device);
+                if (space == GL_HOST) downloads_wait(ctx);
+                cudaStreamSynchronize(g->r[i].comm_stream);
+                cudaStreamSynchronize(g->r[i].prep_stream);
+                quiesce(ctx);
+                hs[i].reset();
+            }
         }
-        return rc;
-    };
+    } bail{g, hs, space};
     // ---- allocate
     for (uint32_t i = 0; i < nl; i++) {
         gl_group_rank& rk = g->r[i];
         gl_ctx* ctx = rk.ctx;
         GCK(g, cudaSetDevice(ctx->device));
-        gl_commit* h = new (std::nothrow) gl_commit();
-        if (!h) return bail(gfail(g, GL_E_OOM, "host allocation failed"));
-        hs[i] = h;
-        h->ctx = ctx; h->log_n = log_n; h->c = c; h->rate_bits = rate_bits; h->cap_height = cap_height;
-        h->salt = (flags & GL_COMMIT_BLINDING) ? GL_SALT_SIZE : 0;   // every rank salts its own leaves
-        h->shard_index = ctx->shard_index; h->shard_count = ctx->shard_count;
-        h->coeffs_bytes = (size_t)plan.cpad * n * 8;
-        int rc = dev_alloc(ctx, h->coeffs_bytes, &h->coeffs);
-        if (rc == GL_OK) rc = commit_prepare(ctx, h);
-        if (rc != GL_OK) return bail(gfail(g, rc, ctx->err));
+        // every rank salts its own leaves
+        GTRY(g, ctx, commit_new(ctx, log_n, c, rate_bits, cap_height, (flags & GL_COMMIT_BLINDING) ? GL_SALT_SIZE : 0, plan.cpad,
+                                &hs[i]));
+        gl_commit* h = hs[i].get();
         h->stream_hash = (flags & GL_COMMIT_STREAM_HASH) && c > 4 && !h->salt;
         while (rk.ev.size() < 2 * (size_t)plan.rounds + 2) {
             cudaEvent_t e;
             cudaError_t ce = cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
-            if (ce != cudaSuccess) return bail(gfail(g, GL_E_CUDA, cudaGetErrorString(ce)));
+            if (ce != cudaSuccess) return gfail(g, GL_E_CUDA, cudaGetErrorString(ce));
             rk.ev.push_back(e);
         }
         if (rk.cap_all_bytes < cap_bytes) {
             if (rk.cap_all) cudaFree(rk.cap_all);
             rk.cap_all = nullptr;
             cudaError_t ce = cudaMalloc(&rk.cap_all, cap_bytes);
-            if (ce != cudaSuccess) return bail(gfail(g, GL_E_OOM, cudaGetErrorString(ce)));
+            if (ce != cudaSuccess) return gfail(g, GL_E_OOM, cudaGetErrorString(ce));
             rk.cap_all_bytes = cap_bytes;
         }
         // the padding columns of the last round take part in the gather: keep them defined
@@ -629,7 +628,7 @@ static int group_commit(gl_group* g, const uint64_t* const* inputs, bool is_valu
             const uint32_t j = plan.rounds - 1;
             const uint32_t own0 = plan.base[j] + (g->rank0 + i) * plan.w[j], own1 = own0 + plan.w[j];
             const uint32_t z0 = own0 > c ? own0 : c;
-            if (own1 > z0) cudaMemsetAsync(h->coeffs + (size_t)z0 * n, 0, (size_t)(own1 - z0) * n * 8, ctx->stream);
+            if (own1 > z0) cudaMemsetAsync(h->coeffs.get() + (size_t)z0 * n, 0, (size_t)(own1 - z0) * n * 8, ctx->stream);
         }
         for (int e = 0; e <= 3; e++) mark(ctx, e);
     }
@@ -637,7 +636,7 @@ static int group_commit(gl_group* g, const uint64_t* const* inputs, bool is_valu
     auto lde_round = [&](uint32_t i, uint32_t j) -> int {
         gl_group_rank& rk = g->r[i];
         gl_ctx* ctx = rk.ctx;
-        gl_commit* h = hs[i];
+        gl_commit* h = hs[i].get();
         cudaSetDevice(ctx->device);
         cudaError_t ce = cudaStreamWaitEvent(ctx->stream, rk.ev[2 * j + 1], 0);
         if (ce != cudaSuccess) return gfail(g, GL_E_CUDA, cudaGetErrorString(ce));
@@ -656,7 +655,7 @@ static int group_commit(gl_group* g, const uint64_t* const* inputs, bool is_valu
         for (uint32_t i = 0; i < nl; i++) {
             gl_group_rank& rk = g->r[i];
             gl_ctx* ctx = rk.ctx;
-            gl_commit* h = hs[i];
+            gl_commit* h = hs[i].get();
             GCK(g, cudaSetDevice(ctx->device));
             const uint32_t own0 = plan.base[j] + (g->rank0 + i) * plan.w[j];
             const uint32_t o0 = clampc(own0, c), o1 = clampc(own0 + plan.w[j], c);
@@ -670,31 +669,26 @@ static int group_commit(gl_group* g, const uint64_t* const* inputs, bool is_valu
             } on_prep(ctx, rk.prep_stream);
             if (j == 0) cudaStreamWaitEvent(rk.prep_stream, ctx->ev[3], 0);   // buffers allocated / padded on the main stream
             if (o1 > o0) {
-                u64* dcol = h->coeffs + (size_t)o0 * n;
+                u64* dcol = h->coeffs.get() + (size_t)o0 * n;
                 const size_t bytes = (size_t)(o1 - o0) * n * 8;
                 if (space == GL_DEVICE) {
                     cudaError_t ce = cudaMemcpyAsync(dcol, inputs[i] + (size_t)o0 * n, bytes, cudaMemcpyDeviceToDevice, ctx->stream);
-                    if (ce != cudaSuccess) return bail(gfail(g, GL_E_CUDA, cudaGetErrorString(ce)));
+                    if (ce != cudaSuccess) return gfail(g, GL_E_CUDA, cudaGetErrorString(ce));
                 } else {
                     if (j == 0) cudaStreamWaitEvent(ctx->h2d_stream, ctx->ev[0], 0);
-                    int rc = h2d_copy(ctx, dcol, inputs[i] + (size_t)o0 * n, bytes, ctx->h2d_stream);
-                    if (rc != GL_OK) return bail(gfail(g, rc, ctx->err));
+                    GTRY(g, ctx, h2d_copy(ctx, dcol, inputs[i] + (size_t)o0 * n, bytes, ctx->h2d_stream));
                     cudaEventRecord(rk.ev[2 * j], ctx->h2d_stream);
                     cudaStreamWaitEvent(ctx->stream, rk.ev[2 * j], 0);
                     trace[i].mark("up" + std::to_string(j), ctx->h2d_stream);
                 }
-                if (is_values) {
-                    int rc = transform_natural(ctx, dcol, log_n, o1 - o0, true, nullptr, nullptr);   // "IFFT" of this rank's columns
-                    if (rc != GL_OK) return bail(gfail(g, rc, ctx->err));
-                }
+                if (is_values)   // "IFFT" of this rank's columns
+                    GTRY(g, ctx, transform_natural(ctx, dcol, log_n, o1 - o0, true, nullptr, nullptr));
             }
             cudaEventRecord(rk.ev[2 * j], ctx->stream);
             trace[i].mark("ifft" + std::to_string(j), ctx->stream);
-            if (o1 > o0 && is_values && coeffs_out && coeffs_out[i] && space == GL_HOST) {
-                int rc = d2h_copy(ctx, {staging::HostSeg{coeffs_out[i] + (size_t)o0 * n, (size_t)(o1 - o0) * n * 8}},
-                                  h->coeffs + (size_t)o0 * n, rk.ev[2 * j]);
-                if (rc != GL_OK) return bail(gfail(g, rc, ctx->err));
-            }
+            if (o1 > o0 && is_values && coeffs_out && coeffs_out[i] && space == GL_HOST)
+                GTRY(g, ctx, d2h_copy(ctx, {staging::HostSeg{coeffs_out[i] + (size_t)o0 * n, (size_t)(o1 - o0) * n * 8}},
+                                      h->coeffs.get() + (size_t)o0 * n, rk.ev[2 * j]));
             cudaStreamWaitEvent(rk.comm_stream, rk.ev[2 * j], 0);
         }
         if (p2p) {
@@ -703,17 +697,17 @@ static int group_commit(gl_group* g, const uint64_t* const* inputs, bool is_valu
             for (uint32_t i = 0; i < nl; i++) {
                 gl_group_rank& rk = g->r[i];
                 cudaSetDevice(rk.ctx->device);
-                u64* base = hs[i]->coeffs + (size_t)plan.base[j] * n;
+                u64* base = hs[i]->coeffs.get() + (size_t)plan.base[j] * n;
                 cudaError_t ce = cudaMemcpyAsync(rk.xbuf + xoff[j], base + (size_t)(g->rank0 + i) * count, count * 8,
                                                  cudaMemcpyDeviceToDevice, rk.comm_stream);
-                if (ce != cudaSuccess) return bail(gfail(g, GL_E_CUDA, cudaGetErrorString(ce)));
+                if (ce != cudaSuccess) return gfail(g, GL_E_CUDA, cudaGetErrorString(ce));
                 k_group_signal<<<1, 1, 0, rk.comm_stream>>>(rk.xbuf + j, g->epoch);
                 ++g_gl_launches;
             }
             for (uint32_t i = 0; i < nl; i++) {
                 gl_group_rank& rk = g->r[i];
                 cudaSetDevice(rk.ctx->device);
-                u64* base = hs[i]->coeffs + (size_t)plan.base[j] * n;
+                u64* base = hs[i]->coeffs.get() + (size_t)plan.base[j] * n;
                 // 56 CTAs x 256 threads x 4 x 16 B = 0.9 MB of loads in flight per GPU: at 8 GPUs 28 CTAs cost 1.2 ms of a
                 // commit, 126 cost 0.3 ms (they crowd the hashing), 56 are the best of the three
                 static const unsigned pull_ctas = getenv("GL_B200_GROUP_PULL_CTAS") ? (unsigned)atoi(getenv("GL_B200_GROUP_PULL_CTAS")) : 56u;
@@ -726,12 +720,12 @@ static int group_commit(gl_group* g, const uint64_t* const* inputs, bool is_valu
             for (uint32_t i = 0; i < nl; i++) {
                 gl_group_rank& rk = g->r[i];
                 cudaSetDevice(rk.ctx->device);
-                u64* base = hs[i]->coeffs + (size_t)plan.base[j] * n;
+                u64* base = hs[i]->coeffs.get() + (size_t)plan.base[j] * n;
                 const size_t count = (size_t)plan.w[j] * n;
                 ncclResult_t r = a->AllGather(base + (size_t)(g->rank0 + i) * count, base, count, ncclUint64, rk.comm, rk.comm_stream);
                 if (r != ncclSuccess) {
                     if (nl > 1) a->GroupEnd();
-                    return bail(gfail(g, GL_E_NCCL, std::string("ncclAllGather: ") + a->GetErrorString(r)));
+                    return gfail(g, GL_E_NCCL, std::string("ncclAllGather: ") + a->GetErrorString(r));
                 }
             }
             if (nl > 1) NCK(g, a->GroupEnd());
@@ -742,25 +736,18 @@ static int group_commit(gl_group* g, const uint64_t* const* inputs, bool is_valu
             trace[i].mark("gath" + std::to_string(j), g->r[i].comm_stream);
         }
         if (j > 0)
-            for (uint32_t i = 0; i < nl; i++) {
-                int rc = lde_round(i, j - 1);
-                if (rc != GL_OK) return bail(rc);
-            }
+            for (uint32_t i = 0; i < nl; i++) TRY(lde_round(i, j - 1));
     }
-    for (uint32_t i = 0; i < nl; i++) {
-        int rc = lde_round(i, plan.rounds - 1);
-        if (rc != GL_OK) return bail(rc);
-    }
+    for (uint32_t i = 0; i < nl; i++) TRY(lde_round(i, plan.rounds - 1));
     // ---- trees, then the cap all-gather on the communication stream
     const uint32_t tail = 2 * plan.rounds;
     for (uint32_t i = 0; i < nl; i++) {
         gl_group_rank& rk = g->r[i];
         gl_ctx* ctx = rk.ctx;
-        gl_commit* h = hs[i];
+        gl_commit* h = hs[i].get();
         cudaSetDevice(ctx->device);
         h->cols_added = c;
-        int rc = commit_tree(ctx, h, nullptr, GL_DEVICE, h->stream_hash && h->hashed_cols == h->c);
-        if (rc != GL_OK) return bail(gfail(g, rc, ctx->err));
+        GTRY(g, ctx, commit_tree(ctx, h, nullptr, GL_DEVICE, h->stream_hash && h->hashed_cols == h->c));
         cudaEventRecord(rk.ev[tail], ctx->stream);
         trace[i].mark("tree", ctx->stream);
         cudaStreamWaitEvent(rk.comm_stream, rk.ev[tail], 0);
@@ -770,10 +757,10 @@ static int group_commit(gl_group* g, const uint64_t* const* inputs, bool is_valu
         for (uint32_t i = 0; i < nl; i++) {
             gl_group_rank& rk = g->r[i];
             cudaSetDevice(rk.ctx->device);
-            ncclResult_t r = a->AllGather(hs[i]->cap, rk.cap_all, hs[i]->cap_bytes / 8, ncclUint64, rk.comm, rk.comm_stream);
+            ncclResult_t r = a->AllGather(hs[i]->cap.get(), rk.cap_all, hs[i]->cap.bytes() / 8, ncclUint64, rk.comm, rk.comm_stream);
             if (r != ncclSuccess) {
                 if (nl > 1) a->GroupEnd();
-                return bail(gfail(g, GL_E_NCCL, std::string("ncclAllGather(cap): ") + a->GetErrorString(r)));
+                return gfail(g, GL_E_NCCL, std::string("ncclAllGather(cap): ") + a->GetErrorString(r));
             }
         }
         if (nl > 1) NCK(g, a->GroupEnd());
@@ -782,19 +769,18 @@ static int group_commit(gl_group* g, const uint64_t* const* inputs, bool is_valu
         gl_group_rank& rk = g->r[i];
         gl_ctx* ctx = rk.ctx;
         cudaSetDevice(ctx->device);
-        if (G == 1) cudaMemcpyAsync(rk.cap_all, hs[i]->cap, cap_bytes, cudaMemcpyDeviceToDevice, rk.comm_stream);
+        if (G == 1) cudaMemcpyAsync(rk.cap_all, hs[i]->cap.get(), cap_bytes, cudaMemcpyDeviceToDevice, rk.comm_stream);
         if (cap_out && cap_out[i])
             cudaMemcpyAsync(cap_out[i], rk.cap_all, cap_bytes, space == GL_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost,
                             rk.comm_stream);
         if (space == GL_DEVICE && coeffs_out && coeffs_out[i])
-            cudaMemcpyAsync(coeffs_out[i], hs[i]->coeffs, (size_t)c * n * 8, cudaMemcpyDeviceToDevice, ctx->stream);
+            cudaMemcpyAsync(coeffs_out[i], hs[i]->coeffs.get(), (size_t)c * n * 8, cudaMemcpyDeviceToDevice, ctx->stream);
     }
     // ---- one host synchronisation per commit
     int rc = GL_OK;
     for (uint32_t i = 0; i < nl; i++) {
         gl_group_rank& rk = g->r[i];
         gl_ctx* ctx = rk.ctx;
-        gl_commit* h = hs[i];
         cudaSetDevice(ctx->device);
         cudaError_t e1 = cudaStreamSynchronize(ctx->stream), e2 = cudaStreamSynchronize(rk.comm_stream);
         if (rc == GL_OK && e1 != cudaSuccess) rc = gfail(g, GL_E_CUDA, std::string("commit: ") + cudaGetErrorString(e1));
@@ -805,21 +791,13 @@ static int group_commit(gl_group* g, const uint64_t* const* inputs, bool is_valu
         }
         trace[i].mark("cap+d2h", rk.comm_stream);
         if (trace[i].on) { cudaStreamSynchronize(rk.comm_stream); trace[i].dump(g->rank0 + i, ctx->ev[0]); }
-        if (h->hstate) {
-            dev_release(ctx, h->hstate, h->hstate_bytes);
-            h->hstate = nullptr;
-        }
         if (rc == GL_OK) {
-            for (int p = 0; p < GL_PHASES; p++) cudaEventElapsedTime(&ctx->phase_ms[p], ctx->ev[p], ctx->ev[p + 1]);
-            ctx->ev_valid = true;
+            commit_done(ctx, hs[i].get());
             if (i == 0) memcpy(g->phase_ms, ctx->phase_ms, sizeof g->phase_ms);
         }
     }
-    if (rc != GL_OK) return bail(rc);
-    for (uint32_t i = 0; i < nl; i++) {
-        g->r[i].ctx->live_commits++;
-        handles[i] = hs[i];
-    }
+    if (rc != GL_OK) return rc;
+    for (uint32_t i = 0; i < nl; i++) handles[i] = hs[i].release();
     return GL_OK;
 }
 
@@ -897,7 +875,7 @@ extern "C" int gl_group_commit_open(gl_group* g, gl_commit* const* handles, cons
             GCK(g, cudaStreamSynchronize(ctx->stream));   // `meta` dies with this iteration
             const u64* d_loc = (const u64*)d;
             const u64* d_slot = d_loc + mine;
-            launch_gather_open(h->lde, h->n_local, leaf_len(h), h->digests, L, d_loc, d_slot, mine, rk.open_buf, per, ctx->stream);
+            launch_gather_open(h->lde.get(), h->n_local, leaf_len(h), h->digests.get(), L, d_loc, d_slot, mine, rk.open_buf, per, ctx->stream);
         }
         GCK(g, cudaEventRecord(ctx->dl_ev, ctx->stream));
         GCK(g, cudaStreamWaitEvent(rk.comm_stream, ctx->dl_ev, 0));
