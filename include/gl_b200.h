@@ -429,6 +429,34 @@ int gl_permutation_zs(gl_ctx *ctx, const gl_circuit *circuit, const uint64_t *k_
                       gl_commit *wires, const uint64_t *betas, const uint64_t *gammas, uint64_t *zs_partial_products_out,
                       int space, uint64_t *grand_products_out);
 
+/* ---- N3 in one call: plonky2::plonk::prover::prove from the point where the witness exists ------------------------------
+ * Reached from every data.prove(pw) (44 sites, e.g. src/ecdsa/gadgets/ecdsa.rs:349, src/hash/keccak256.rs:248,
+ * src/smt/gadgets/process/mod.rs:82, src/zkdsa/circuits/mod.rs:326), for circuits built from the gates gl_quotient_polys
+ * evaluates.  Upstream's order, with the Fiat-Shamir sponge on the device:
+ *   public_inputs_hash = hash_no_pad(public_inputs) ([0, 0, 0, 0] without public inputs); wires commit (from_values,
+ *   blinding = false); Challenger::new(), observe circuit_digest, public_inputs_hash, wires cap; betas, gammas
+ *   (get_n_challenges(num_challenges) each); Z and partial products (gl_permutation_zs) and their commit; observe the cap,
+ *   alphas; quotient (gl_quotient_polys) and its commit (from_coeffs); observe the cap, zeta = get_extension_challenge()
+ *   (GL_E_STATE when zeta^(2^degree_bits) == 1, upstream's ensure!); OpeningSet at zeta, plonk_zs_next at g * zeta;
+ *   observe_openings(to_fri_openings()); prove_openings (gl_fri_prove) over the oracles [constants_sigmas, wires,
+ *   zs_partial_products, quotient]: every polynomial at zeta, polynomials 0 .. num_challenges of oracle 2 at g * zeta.
+ * constants_sigmas: the caller's resident prover-data commit ([num_constants | num_routed_wires sigmas], unblinded, unsharded,
+ *   this ctx, degree 2^degree_bits; prm's rate_bits and cap_height); it is read, never modified.  circuit_digest [4]:
+ *   prover_data.circuit_digest (its derivation differs between fork revisions, so it is an input).  Witness: `wires`
+ *   [num_wires][2^degree_bits] in `space` memory, or `wires_cols`, num_wires host arrays (the other pointer NULL), as in
+ *   gl_commit_from_values_ex.  prm->flags and the ctx's compat flags apply as in gl_fri_prove.  public_inputs: host.
+ * proof_out (host, ONE copy at the end), in u64 words: wires cap, zs_partial_products cap, quotient cap ([2^cap_height][4]
+ *   each); the OpeningSet in declaration order, [k][2] per field: constants (num_constants), plonk_sigmas (num_routed_wires),
+ *   wires (num_wires), plonk_zs (nch), plonk_zs_next (nch), partial_products (nch * (ceil(routed / qdf) - 1)),
+ *   quotient_polys (nch * qdf); then the FRI proof word for word as gl_fri_prove writes it.  *proof_words_out is always
+ *   set; a NULL or too small proof_out returns GL_E_ARG.  A witness that breaks a gate or copy constraint still returns
+ *   GL_OK and a proof, as upstream's prover does: the verifier rejects it.  The three commits are internal and freed
+ *   before return. */
+int gl_prove(gl_ctx *ctx, const gl_circuit *circuit, const gl_gate *gates, const uint64_t *k_is, gl_commit *constants_sigmas,
+             const uint64_t circuit_digest[4], const gl_fri_params *prm, const uint64_t *wires, const uint64_t *const *wires_cols,
+             int space, const uint64_t *public_inputs, uint32_t num_public_inputs, uint64_t *proof_out, uint64_t proof_cap_words,
+             uint64_t *proof_words_out);
+
 /* ---- P10: fri_proof_of_work ------------------------------------------------------------------- */
 /* Smallest w >= 0 such that permute(state with state[input_pos] = w)[7] (the last rate lane, as
  * `duplex_state.squeeze().last()`) has >= min_leading_zeros leading zero bits.  Upstream's rayon

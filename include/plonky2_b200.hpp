@@ -656,57 +656,12 @@ inline FriProof prove_openings(const Context& c, const std::vector<FriBatchInfo>
     return fri_proof_resident(c, oracles, coeffs.u64(), values.u64(), n, challenger, fp);
 }
 
-// PolynomialBatch::prove_openings + fri_proof through ONE C-ABI call (gl_fri_prove): the Fiat-Shamir transcript runs on the
-// device from `challenger`'s current state and comes back advanced past the proof; one copy brings the proof back.
-// final_poly_times_x selects the fork form of upstream PR #436 (GL_COMPAT_FRI_FINAL_POLY_TIMES_X).
-inline FriProof prove_openings_device(const Context& c, const std::vector<FriBatchInfo>& instance,
-                                      const std::vector<const PolynomialBatch*>& oracles, Challenger& challenger,
-                                      const FriParams& fp, bool final_poly_times_x = false) {
-    if (fp.reduction_arity_bits.size() > GL_FRI_MAX_LAYERS) throw Panic(GL_E_ARG, "too many FRI reduction layers");
-    std::vector<gl_fri_batch> batches;
-    std::vector<gl_fri_poly> polys;
-    for (auto& b : instance) {
-        gl_fri_batch gb;
-        gb.point[0] = b.point[0];
-        gb.point[1] = b.point[1];
-        gb.first_poly = (uint32_t)polys.size();
-        gb.num_polys = (uint32_t)b.polynomials.size();
-        for (auto& pr : b.polynomials) polys.push_back({pr.first, pr.second});
-        batches.push_back(gb);
-    }
-    gl_fri_params prm;
-    std::memset(&prm, 0, sizeof prm);
-    prm.rate_bits = fp.config.rate_bits;
-    prm.cap_height = fp.config.cap_height;
-    prm.proof_of_work_bits = fp.config.proof_of_work_bits;
-    prm.num_query_rounds = fp.config.num_query_rounds;
-    prm.num_reduction_layers = (uint32_t)fp.reduction_arity_bits.size();
-    for (size_t i = 0; i < fp.reduction_arity_bits.size(); i++) prm.reduction_arity_bits[i] = fp.reduction_arity_bits[i];
-    prm.flags = final_poly_times_x ? GL_COMPAT_FRI_FINAL_POLY_TIMES_X : 0;
-    gl_challenger ch;
-    std::memset(&ch, 0, sizeof ch);
-    for (int i = 0; i < 12; i++) ch.sponge_state[i] = challenger.sponge_state[i];
-    ch.input_len = (uint32_t)challenger.input_buffer.size();
-    ch.output_len = (uint32_t)challenger.output_buffer.size();
-    for (uint32_t i = 0; i < ch.input_len; i++) ch.input_buffer[i] = challenger.input_buffer[i];
-    for (uint32_t i = 0; i < ch.output_len; i++) ch.output_buffer[i] = challenger.output_buffer[i];
-    std::vector<gl_commit*> handles;
-    std::vector<uint32_t> widths;
-    for (auto* o : oracles) {
-        handles.push_back(o->raw_handle());
-        widths.push_back(o->leaf_len);
-    }
-    uint64_t words = 0;
-    c.check(gl_fri_proof_words(&prm, widths.data(), (uint32_t)widths.size(), fp.degree_bits, &words));
-    std::vector<uint64_t> flat(words);
-    c.check(gl_fri_prove(c.raw(), handles.data(), (uint32_t)handles.size(), batches.data(), (uint32_t)batches.size(), polys.data(),
-                         &prm, &ch, flat.data(), words, &words));
-    for (int i = 0; i < 12; i++) challenger.sponge_state[i] = ch.sponge_state[i];
-    challenger.input_buffer.assign(ch.input_buffer, ch.input_buffer + ch.input_len);
-    challenger.output_buffer.assign(ch.output_buffer, ch.output_buffer + ch.output_len);
-    // the word stream -> FriProof (field order of include/gl_b200.h)
+namespace detail {
+// The FRI proof word stream of gl_fri_prove (field order of include/gl_b200.h), starting at flat[at] and running to the end
+// of flat -> FriProof; widths: the leaf width of every initial oracle.
+inline FriProof fri_proof_from_words(const std::vector<uint64_t>& flat, size_t at, const std::vector<uint32_t>& widths,
+                                     const FriParams& fp) {
     FriProof proof;
-    size_t at = 0;
     const uint32_t h = fp.config.cap_height, lgN = fp.degree_bits + fp.config.rate_bits;
     auto take_path = [&](uint32_t len) {
         MerkleProof mp;
@@ -752,6 +707,64 @@ inline FriProof prove_openings_device(const Context& c, const std::vector<FriBat
     return proof;
 }
 
+inline gl_fri_params fri_params_c(const FriParams& fp, bool final_poly_times_x) {
+    if (fp.reduction_arity_bits.size() > GL_FRI_MAX_LAYERS) throw Panic(GL_E_ARG, "too many FRI reduction layers");
+    gl_fri_params prm;
+    std::memset(&prm, 0, sizeof prm);
+    prm.rate_bits = fp.config.rate_bits;
+    prm.cap_height = fp.config.cap_height;
+    prm.proof_of_work_bits = fp.config.proof_of_work_bits;
+    prm.num_query_rounds = fp.config.num_query_rounds;
+    prm.num_reduction_layers = (uint32_t)fp.reduction_arity_bits.size();
+    for (size_t i = 0; i < fp.reduction_arity_bits.size(); i++) prm.reduction_arity_bits[i] = fp.reduction_arity_bits[i];
+    prm.flags = final_poly_times_x ? GL_COMPAT_FRI_FINAL_POLY_TIMES_X : 0;
+    return prm;
+}
+}  // namespace detail
+
+// PolynomialBatch::prove_openings + fri_proof through ONE C-ABI call (gl_fri_prove): the Fiat-Shamir transcript runs on the
+// device from `challenger`'s current state and comes back advanced past the proof; one copy brings the proof back.
+// final_poly_times_x selects the fork form of upstream PR #436 (GL_COMPAT_FRI_FINAL_POLY_TIMES_X).
+inline FriProof prove_openings_device(const Context& c, const std::vector<FriBatchInfo>& instance,
+                                      const std::vector<const PolynomialBatch*>& oracles, Challenger& challenger,
+                                      const FriParams& fp, bool final_poly_times_x = false) {
+    if (fp.reduction_arity_bits.size() > GL_FRI_MAX_LAYERS) throw Panic(GL_E_ARG, "too many FRI reduction layers");
+    std::vector<gl_fri_batch> batches;
+    std::vector<gl_fri_poly> polys;
+    for (auto& b : instance) {
+        gl_fri_batch gb;
+        gb.point[0] = b.point[0];
+        gb.point[1] = b.point[1];
+        gb.first_poly = (uint32_t)polys.size();
+        gb.num_polys = (uint32_t)b.polynomials.size();
+        for (auto& pr : b.polynomials) polys.push_back({pr.first, pr.second});
+        batches.push_back(gb);
+    }
+    const gl_fri_params prm = detail::fri_params_c(fp, final_poly_times_x);
+    gl_challenger ch;
+    std::memset(&ch, 0, sizeof ch);
+    for (int i = 0; i < 12; i++) ch.sponge_state[i] = challenger.sponge_state[i];
+    ch.input_len = (uint32_t)challenger.input_buffer.size();
+    ch.output_len = (uint32_t)challenger.output_buffer.size();
+    for (uint32_t i = 0; i < ch.input_len; i++) ch.input_buffer[i] = challenger.input_buffer[i];
+    for (uint32_t i = 0; i < ch.output_len; i++) ch.output_buffer[i] = challenger.output_buffer[i];
+    std::vector<gl_commit*> handles;
+    std::vector<uint32_t> widths;
+    for (auto* o : oracles) {
+        handles.push_back(o->raw_handle());
+        widths.push_back(o->leaf_len);
+    }
+    uint64_t words = 0;
+    c.check(gl_fri_proof_words(&prm, widths.data(), (uint32_t)widths.size(), fp.degree_bits, &words));
+    std::vector<uint64_t> flat(words);
+    c.check(gl_fri_prove(c.raw(), handles.data(), (uint32_t)handles.size(), batches.data(), (uint32_t)batches.size(), polys.data(),
+                         &prm, &ch, flat.data(), words, &words));
+    for (int i = 0; i < 12; i++) challenger.sponge_state[i] = ch.sponge_state[i];
+    challenger.input_buffer.assign(ch.input_buffer, ch.input_buffer + ch.input_len);
+    challenger.output_buffer.assign(ch.output_buffer, ch.output_buffer + ch.output_len);
+    return detail::fri_proof_from_words(flat, 0, widths, fp);
+}
+
 // plonky2::plonk::prover compute_quotient_polys on the three resident prove-time oracles (gl_quotient_polys): returns
 // quotient_polys.flat_map(|p| p.chunks(degree)), num_challenges * quotient_degree_factor coefficient vectors of 2^degree_bits.
 inline std::vector<std::vector<F>> compute_quotient_polys(const Context& c, const gl_circuit& circuit, const std::vector<gl_gate>& gates,
@@ -791,6 +804,60 @@ inline PermutationZs all_wires_permutation_partial_products(const Context& c, co
     c.check(gl_permutation_zs(c.raw(), &circuit, k_is.data(), constants_sigmas.raw_handle(), wires.raw_handle(), betas.data(),
                               gammas.data(), flat.data(), GL_HOST, out.grand_products.data()));
     for (size_t i = 0; i < cols; i++) out.zs_partial_products.emplace_back(flat.begin() + i * n, flat.begin() + (i + 1) * n);
+    return out;
+}
+
+// plonky2::plonk::prover::prove from the witness on, in one C-ABI call (gl_prove): ProofWithPublicInputs field by field.
+// `words` is the stream gl_prove returns (caps, OpeningSet, FRI proof); the other fields are views of it.
+struct ProofWithPublicInputs {
+    MerkleCap wires_cap, plonk_zs_partial_products_cap, quotient_polys_cap;
+    // OpeningSet in declaration order: constants, plonk_sigmas, wires, plonk_zs, plonk_zs_next, partial_products,
+    // quotient_polys; each entry (a0, a1)
+    std::vector<std::vector<std::array<F, 2>>> openings;
+    FriProof opening_proof;
+    std::vector<F> public_inputs;
+    std::vector<uint64_t> words;
+};
+// wires: num_wires columns of 2^degree_bits values (the witness); constants_sigmas: the resident prover-data commit.
+inline ProofWithPublicInputs prove(const Context& c, const gl_circuit& circuit, const std::vector<gl_gate>& gates,
+                                   const std::vector<F>& k_is, const PolynomialBatch& constants_sigmas, const HashOut& circuit_digest,
+                                   const FriParams& fp, const std::vector<std::vector<F>>& wires, const std::vector<F>& public_inputs,
+                                   bool final_poly_times_x = false) {
+    if (k_is.size() < circuit.num_routed_wires || gates.size() < circuit.num_gates || wires.size() != circuit.num_wires)
+        throw Panic(GL_E_ARG, "prove: fewer k_is than num_routed_wires or gates than num_gates, or a witness without num_wires columns");
+    for (auto& w : wires)   // the library reads 2^degree_bits values of every column and cannot check the caller's sizes
+        if (w.size() != ((size_t)1 << circuit.degree_bits)) throw Panic(GL_E_ARG, "prove: a witness column without 2^degree_bits values");
+    const gl_fri_params prm = detail::fri_params_c(fp, final_poly_times_x);
+    std::vector<const uint64_t*> cols;
+    for (auto& w : wires) cols.push_back(w.data());
+    ProofWithPublicInputs out;
+    uint64_t words = 0;
+    gl_prove(c.raw(), &circuit, gates.data(), k_is.data(), constants_sigmas.raw_handle(), circuit_digest.elements, &prm, nullptr,
+             cols.data(), GL_HOST, public_inputs.data(), (uint32_t)public_inputs.size(), nullptr, 0, &words);   // size only
+    out.words.resize(words);
+    c.check(gl_prove(c.raw(), &circuit, gates.data(), k_is.data(), constants_sigmas.raw_handle(), circuit_digest.elements, &prm,
+                     nullptr, cols.data(), GL_HOST, public_inputs.data(), (uint32_t)public_inputs.size(), out.words.data(), words,
+                     &words));
+    size_t at = 0;
+    const size_t cap_len = (size_t)1 << fp.config.cap_height;
+    for (MerkleCap* cap : {&out.wires_cap, &out.plonk_zs_partial_products_cap, &out.quotient_polys_cap}) {
+        cap->resize(cap_len);
+        for (auto& d : *cap)
+            for (int e = 0; e < 4; e++) d.elements[e] = out.words[at++];
+    }
+    const uint32_t nch = circuit.num_challenges, qdf = circuit.quotient_degree_factor;
+    const uint32_t zcols = nch * ((circuit.num_routed_wires + qdf - 1) / qdf);
+    for (uint32_t k : {circuit.num_constants, circuit.num_routed_wires, circuit.num_wires, nch, nch, zcols - nch, nch * qdf}) {
+        std::vector<std::array<F, 2>> field(k);
+        for (auto& v : field) {
+            v[0] = out.words[at++];
+            v[1] = out.words[at++];
+        }
+        out.openings.push_back(std::move(field));
+    }
+    const std::vector<uint32_t> widths = {constants_sigmas.leaf_len, circuit.num_wires, zcols, nch * qdf};
+    out.opening_proof = detail::fri_proof_from_words(out.words, at, widths, fp);
+    out.public_inputs = public_inputs;
     return out;
 }
 

@@ -143,6 +143,7 @@ SIGNATURES = {
     "gl_fri_prove": (cint, [vp, vp, u32, vp, u32, vp, vp, vp, vp, u64, C.POINTER(u64)]),
     "gl_quotient_polys": (cint, [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, cint]),
     "gl_permutation_zs": (cint, [vp, vp, vp, vp, vp, vp, vp, vp, cint, vp]),
+    "gl_prove": (cint, [vp, vp, vp, vp, vp, vp, vp, vp, vp, cint, vp, u32, vp, u64, C.POINTER(u64)]),
     "gl_group_unique_id": (cint, [vp]),
     "gl_group_create": (cint, [vp, u32, u32, u32, vp, C.POINTER(vp)]),
     "gl_group_destroy": (None, [vp]),

@@ -1416,19 +1416,16 @@ static int commit_build(gl_ctx* ctx, gl_commit* h, const HostCols& input, bool i
     return finish(ctx);
 }
 
-static int commit_common(gl_ctx* ctx, const HostCols& input, bool is_values, uint32_t log_n, uint32_t c,
-                         uint32_t rate_bits, uint32_t cap_height, const HostCols& coeffs_out, uint64_t* cap_out,
-                         gl_commit** handle, int space, const char* name, bool blinding = false) {
-    if (!ctx) return GL_E_ARG;
-    if (!handle || !input) return fail(ctx, GL_E_ARG, std::string(name) + ": NULL argument");
-    *handle = nullptr;
+// A whole polynomial commit with the ctx held (Guard): checks, allocation, build.  *out is set only on success.
+static int commit_make(gl_ctx* ctx, const HostCols& input, bool is_values, uint32_t log_n, uint32_t c, uint32_t rate_bits,
+                       uint32_t cap_height, const HostCols& coeffs_out, uint64_t* cap_out, int space, const char* name,
+                       bool blinding, std::unique_ptr<gl_commit>* out) {
     TRY(commit_check(ctx, log_n, c, rate_bits, cap_height, name));
     if (input.cols || coeffs_out.cols) {
         for (uint32_t j = 0; j < c; j++)
             if ((input.cols && !input.cols[j]) || (coeffs_out.cols && !coeffs_out.cols[j]))
                 return fail(ctx, GL_E_ARG, std::string(name) + ": NULL polynomial pointer");
     }
-    Guard g(ctx);
     std::unique_ptr<gl_commit> h;
     int rc = commit_new(ctx, log_n, c, rate_bits, cap_height, blinding ? GL_SALT_SIZE : 0, c, &h);
     if (rc == GL_OK) rc = commit_build(ctx, h.get(), input, is_values, coeffs_out, cap_out, space);
@@ -1441,6 +1438,19 @@ static int commit_common(gl_ctx* ctx, const HostCols& input, bool is_values, uin
         return rc;
     }
     commit_done(ctx, h.get());
+    *out = std::move(h);
+    return GL_OK;
+}
+
+static int commit_common(gl_ctx* ctx, const HostCols& input, bool is_values, uint32_t log_n, uint32_t c,
+                         uint32_t rate_bits, uint32_t cap_height, const HostCols& coeffs_out, uint64_t* cap_out,
+                         gl_commit** handle, int space, const char* name, bool blinding = false) {
+    if (!ctx) return GL_E_ARG;
+    if (!handle || !input) return fail(ctx, GL_E_ARG, std::string(name) + ": NULL argument");
+    *handle = nullptr;
+    Guard g(ctx);
+    std::unique_ptr<gl_commit> h;
+    TRY(commit_make(ctx, input, is_values, log_n, c, rate_bits, cap_height, coeffs_out, cap_out, space, name, blinding, &h));
     *handle = h.release();
     return GL_OK;
 }
@@ -1610,6 +1620,23 @@ extern "C" int gl_commit_coeffs(gl_commit* h, uint64_t* coeffs_out, int space) {
     return finish(ctx);
 }
 
+// Polynomials [col0, col0 + ncols) of the commit at one extension point -> values_out [ncols][2], with the ctx held
+static int commit_eval(gl_ctx* ctx, const gl_commit* h, uint32_t col0, uint32_t ncols, const uint64_t point[2],
+                       uint64_t* values_out, int space) {
+    const u64 n = (u64)1 << h->log_n;
+    const u64 chunks = (n + FRI_EVAL_CHUNK - 1) / FRI_EVAL_CHUNK;
+    const glh::ext z = {glh::canon(point[0]), glh::canon(point[1])};
+    const glh::ext z256 = glh::ext_pow(z, 256), zc = glh::ext_pow(z, FRI_EVAL_CHUNK);
+    const u64 zz[2] = {z.a, z.b}, z2[2] = {z256.a, z256.b}, z3[2] = {zc.a, zc.b};
+    void* d;
+    TRY(scratch_get(ctx, 0, ((size_t)ncols * chunks + ncols) * 16, &d));
+    u64* partial = (u64*)d;
+    u64* d_out = space == GL_DEVICE ? values_out : partial + 2 * (size_t)ncols * chunks;
+    launch_eval_at(h->coeffs.get() + (size_t)col0 * n, n, ncols, zz, z2, z3, partial, d_out, ctx->stream);
+    if (space == GL_HOST) TRY(copy_out(ctx, values_out, d_out, (size_t)ncols * 16, GL_HOST));
+    return GL_OK;
+}
+
 // OpeningSet::new: every polynomial of the commit at one extension point, without bringing the coefficients back
 extern "C" int gl_commit_eval(gl_commit* h, const uint64_t point[2], uint64_t* values_out, int space) {
     if (!h || !point || !values_out) return GL_E_ARG;
@@ -1617,17 +1644,7 @@ extern "C" int gl_commit_eval(gl_commit* h, const uint64_t point[2], uint64_t* v
     if (!h->coeffs.get()) return fail(ctx, GL_E_STATE, "gl_commit_eval: this handle has no polynomials (FRI layer tree)");
     if (!h->finished && h->cols_added != h->c) return fail(ctx, GL_E_STATE, "gl_commit_eval: not every polynomial has been added");
     Guard g(ctx);
-    const u64 n = (u64)1 << h->log_n;
-    const u64 chunks = (n + FRI_EVAL_CHUNK - 1) / FRI_EVAL_CHUNK;
-    const glh::ext z = {glh::canon(point[0]), glh::canon(point[1])};
-    const glh::ext z256 = glh::ext_pow(z, 256), zc = glh::ext_pow(z, FRI_EVAL_CHUNK);
-    const u64 zz[2] = {z.a, z.b}, z2[2] = {z256.a, z256.b}, z3[2] = {zc.a, zc.b};
-    void* d;
-    TRY(scratch_get(ctx, 0, ((size_t)h->c * chunks + h->c) * 16, &d));
-    u64* partial = (u64*)d;
-    u64* d_out = space == GL_DEVICE ? values_out : partial + 2 * (size_t)h->c * chunks;
-    launch_eval_at(h->coeffs.get(), n, h->c, zz, z2, z3, partial, d_out, ctx->stream);
-    if (space == GL_HOST) TRY(copy_out(ctx, values_out, d_out, (size_t)h->c * 16, GL_HOST));
+    TRY(commit_eval(ctx, h, 0, h->c, point, values_out, space));
     return finish(ctx);
 }
 
@@ -1971,6 +1988,17 @@ extern "C" int gl_fri_proof_words(const gl_fri_params* prm, const uint32_t* orac
     return GL_OK;
 }
 
+static int fri_params_check(gl_ctx* ctx, const gl_fri_params* prm, const char* name) {
+    if (prm->num_reduction_layers > GL_FRI_MAX_LAYERS || prm->num_query_rounds == 0 || prm->num_query_rounds > 1024 ||
+        prm->proof_of_work_bits > 48)
+        return fail(ctx, GL_E_ARG, std::string(name) + ": unsupported FRI parameters");
+    return GL_OK;
+}
+
+static int fri_prove_body(gl_ctx* ctx, gl_commit* const* oracles, uint32_t num_oracles, const gl_fri_batch* batches,
+                          uint32_t num_batches, const gl_fri_poly* polys, const gl_fri_params* prm, gl_challenger* challenger,
+                          uint64_t words, u64* d_proof, uint64_t* host_out, const u64* host_src, uint64_t host_words);
+
 extern "C" int gl_fri_prove(gl_ctx* ctx, gl_commit* const* oracles, uint32_t num_oracles, const gl_fri_batch* batches,
                             uint32_t num_batches, const gl_fri_poly* polys, const gl_fri_params* prm, gl_challenger* challenger,
                             uint64_t* proof_out, uint64_t proof_cap_words, uint64_t* proof_words_out) {
@@ -1978,32 +2006,40 @@ extern "C" int gl_fri_prove(gl_ctx* ctx, gl_commit* const* oracles, uint32_t num
     if (!oracles || !num_oracles || !prm || !challenger || !proof_words_out)
         return fail(ctx, GL_E_ARG, "gl_fri_prove: NULL argument");
     if (challenger->input_len > 8 || challenger->output_len > 8) return fail(ctx, GL_E_ARG, "gl_fri_prove: bad challenger state");
-    if (prm->num_reduction_layers > GL_FRI_MAX_LAYERS || prm->num_query_rounds == 0 || prm->num_query_rounds > 1024 ||
-        prm->proof_of_work_bits > 48)
-        return fail(ctx, GL_E_ARG, "gl_fri_prove: unsupported FRI parameters");
+    TRY(fri_params_check(ctx, prm, "gl_fri_prove"));
     for (uint32_t i = 0; i < num_oracles; i++)
         if (!oracles[i] || oracles[i]->ctx != ctx || !oracles[i]->coeffs.get() || !oracles[i]->finished || oracles[i]->shard_count != 1 ||
             oracles[i]->rate_bits != prm->rate_bits || oracles[i]->cap_height != prm->cap_height || oracles[i]->log_n != oracles[0]->log_n)
             return fail(ctx, GL_E_STATE, "gl_fri_prove: every oracle must be a finished, unsharded polynomial commit of this ctx with the FRI config's rate_bits / cap_height");
-    const uint32_t degree_bits = oracles[0]->log_n, rate_bits = prm->rate_bits, h = prm->cap_height, rounds = prm->num_query_rounds;
-    const unsigned lgN = degree_bits + rate_bits;
     std::vector<uint32_t> ocols(num_oracles);
     for (uint32_t i = 0; i < num_oracles; i++) ocols[i] = leaf_len(oracles[i]);
     uint64_t words = 0;
-    if (gl_fri_proof_words(prm, ocols.data(), num_oracles, degree_bits, &words) != GL_OK)
+    if (gl_fri_proof_words(prm, ocols.data(), num_oracles, oracles[0]->log_n, &words) != GL_OK)
         return fail(ctx, GL_E_ARG, "gl_fri_prove: reduction_arity_bits do not fit the degree / cap_height");
     *proof_words_out = words;
     if (!proof_out || proof_cap_words < words) return fail(ctx, GL_E_ARG, "gl_fri_prove: proof buffer too small (see *proof_words_out)");
     Guard g(ctx);
+    PoolBuf proof;
+    TRY(proof.alloc(ctx, words * 8));
+    return fri_prove_body(ctx, oracles, num_oracles, batches, num_batches, polys, prm, challenger, words, proof.get(), proof_out,
+                          proof.get(), words);
+}
+
+// The body of gl_fri_prove, with the ctx held and the arguments checked: the proof's `words` words go to the device buffer
+// d_proof, *challenger advances past the proof, and host_words words from host_src reach host_out with the final
+// synchronisation (the proof itself, or a larger buffer that holds it).
+static int fri_prove_body(gl_ctx* ctx, gl_commit* const* oracles, uint32_t num_oracles, const gl_fri_batch* batches,
+                          uint32_t num_batches, const gl_fri_poly* polys, const gl_fri_params* prm, gl_challenger* challenger,
+                          uint64_t words, u64* d_proof, uint64_t* host_out, const u64* host_src, uint64_t host_words) {
+    const uint32_t degree_bits = oracles[0]->log_n, rate_bits = prm->rate_bits, h = prm->cap_height, rounds = prm->num_query_rounds;
+    const unsigned lgN = degree_bits + rate_bits;
     const u64 N = (u64)1 << lgN;
     const uint32_t layers = prm->num_reduction_layers;
     // device state: challenger | alpha/beta scratch [2] | query challenges [rounds] | pow state [12] | pow best | response |
     // cumulative arity bits | query indices [(layers + 1)][rounds]
-    PoolBuf state, proof;
+    PoolBuf state;
     TRY(state.alloc(ctx, (32 + 2 + rounds + 12 + 2 + GL_FRI_MAX_LAYERS + (size_t)(layers + 1) * rounds) * 8));
-    TRY(proof.alloc(ctx, words * 8));
     u64* d_state = state.get();
-    u64* d_proof = proof.get();
     std::vector<std::unique_ptr<gl_commit>> trees;
     static_assert(sizeof(gl_challenger) == 29 * 8, "gl_challenger layout");
     gl_challenger* d_ch = (gl_challenger*)d_state;
@@ -2119,7 +2155,7 @@ extern "C" int gl_fri_prove(gl_ctx* ctx, gl_commit* const* oracles, uint32_t num
     off += query_stride * rounds;
     if (off != words) return fail(ctx, GL_E_STATE, "gl_fri_prove: internal size mismatch");
     u64 response = 0;
-    CK(cudaMemcpyAsync(proof_out, d_proof, words * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(host_out, host_src, host_words * 8, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(challenger, d_ch, sizeof(gl_challenger), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(&response, d_resp, 8, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
@@ -2140,18 +2176,47 @@ extern "C" int gl_ctx_set_compat(gl_ctx* ctx, uint32_t flags) {
 // ------------------------------------------------------------------------------------------------
 // N3: compute_quotient_polys
 // ------------------------------------------------------------------------------------------------
-extern "C" int gl_quotient_polys(gl_ctx* ctx, const gl_circuit* cd, const gl_gate* gates, const uint64_t* k_is,
-                                 gl_commit* constants_sigmas, gl_commit* wires, gl_commit* zs_pp,
-                                 const uint64_t* public_inputs_hash, const uint64_t* betas, const uint64_t* gammas,
-                                 const uint64_t* alphas, uint64_t* chunks_out, int space) {
-    if (!ctx) return GL_E_ARG;
-    if (!cd || !gates || !k_is || !constants_sigmas || !wires || !zs_pp || !public_inputs_hash || !betas || !gammas || !alphas ||
-        !chunks_out)
-        return fail(ctx, GL_E_ARG, "gl_quotient_polys: NULL argument");
+// The circuit geometry compute_quotient_polys supports (independent of the oracles)
+static int quotient_geometry_check(gl_ctx* ctx, const gl_circuit* cd) {
     const uint32_t nch = cd->num_challenges, R = cd->num_routed_wires, deg = cd->quotient_degree_factor;
     if (nch == 0 || nch > QUOTIENT_MAX_CHALLENGES || cd->num_gates == 0 || cd->num_gates > QUOTIENT_MAX_GATES || R == 0 ||
         R > cd->num_wires || !is_pow2(deg) || cd->num_selectors == 0 || cd->num_selectors > cd->num_constants)
         return fail(ctx, GL_E_ARG, "gl_quotient_polys: unsupported circuit geometry");
+    return GL_OK;
+}
+static int quotient_rate_check(gl_ctx* ctx, const gl_circuit* cd, uint32_t rate_bits) {
+    const uint32_t qdb = ilog2(cd->quotient_degree_factor);
+    if (qdb > rate_bits || qdb > 5)
+        return fail(ctx, GL_E_ARG, "compute_quotient_polys: having constraints of degree higher than the rate is not supported");
+    return GL_OK;
+}
+// gates[i] of a circuit that passed quotient_geometry_check
+static int quotient_gate_check(gl_ctx* ctx, const gl_circuit* cd, const gl_gate& g, uint32_t i) {
+    if (g.kind > GL_GATE_UNINTERLEAVE_TO_B32 || g.selector_index >= cd->num_selectors || g.group_start > i || g.group_end <= i ||
+        g.group_end > cd->num_gates)
+        return fail(ctx, GL_E_ARG, "gl_quotient_polys: bad gate descriptor");
+    uint32_t need = 0;
+    switch (g.kind) {
+        case GL_GATE_CONSTANT: need = g.num_ops; if (cd->num_selectors + g.num_ops > cd->num_constants) need = ~0u; break;
+        case GL_GATE_PUBLIC_INPUT: need = 4; break;
+        case GL_GATE_U32_INTERLEAVE: need = g.num_ops * 34; break;
+        case GL_GATE_UNINTERLEAVE_TO_U32:
+        case GL_GATE_UNINTERLEAVE_TO_B32: need = g.num_ops * 67; break;
+        default: break;
+    }
+    if (need > cd->num_wires) return fail(ctx, GL_E_ARG, "gl_quotient_polys: gate does not fit the wires / constants");
+    return GL_OK;
+}
+
+// compute_quotient_polys with the ctx held (the body of gl_quotient_polys)
+static int quotient_polys(gl_ctx* ctx, const gl_circuit* cd, const gl_gate* gates, const uint64_t* k_is,
+                          gl_commit* constants_sigmas, gl_commit* wires, gl_commit* zs_pp, const uint64_t* public_inputs_hash,
+                          const uint64_t* betas, const uint64_t* gammas, const uint64_t* alphas, uint64_t* chunks_out, int space) {
+    if (!cd || !gates || !k_is || !constants_sigmas || !wires || !zs_pp || !public_inputs_hash || !betas || !gammas || !alphas ||
+        !chunks_out)
+        return fail(ctx, GL_E_ARG, "gl_quotient_polys: NULL argument");
+    const uint32_t nch = cd->num_challenges, R = cd->num_routed_wires, deg = cd->quotient_degree_factor;
+    TRY(quotient_geometry_check(ctx, cd));
     const uint32_t qdb = ilog2(deg), lg_n = cd->degree_bits;
     gl_commit* cm[3] = {constants_sigmas, wires, zs_pp};
     for (auto* h : cm) {
@@ -2160,8 +2225,7 @@ extern "C" int gl_quotient_polys(gl_ctx* ctx, const gl_circuit* cd, const gl_gat
         if (h->shard_count != 1) return fail(ctx, GL_E_ARG, "gl_quotient_polys: sharded oracles are not supported");
     }
     const uint32_t rate_bits = wires->rate_bits;
-    if (qdb > rate_bits || qdb > 5)
-        return fail(ctx, GL_E_ARG, "compute_quotient_polys: having constraints of degree higher than the rate is not supported");
+    TRY(quotient_rate_check(ctx, cd, rate_bits));
     const uint32_t chunks = (R + deg - 1) / deg, num_prods = chunks - 1;
     if (constants_sigmas->c != cd->num_constants + R || wires->c != cd->num_wires || zs_pp->c != nch * chunks)
         return fail(ctx, GL_E_ARG, "gl_quotient_polys: column counts do not match the circuit description");
@@ -2170,23 +2234,10 @@ extern "C" int gl_quotient_polys(gl_ctx* ctx, const gl_circuit* cd, const gl_gat
     uint32_t ngc = 0;
     for (uint32_t i = 0; i < cd->num_gates; i++) {
         const gl_gate& g = gates[i];
-        if (g.kind > GL_GATE_UNINTERLEAVE_TO_B32 || g.selector_index >= cd->num_selectors || g.group_start > i || g.group_end <= i ||
-            g.group_end > cd->num_gates)
-            return fail(ctx, GL_E_ARG, "gl_quotient_polys: bad gate descriptor");
-        uint32_t need = 0;
-        switch (g.kind) {
-            case GL_GATE_CONSTANT: need = g.num_ops; if (cd->num_selectors + g.num_ops > cd->num_constants) need = ~0u; break;
-            case GL_GATE_PUBLIC_INPUT: need = 4; break;
-            case GL_GATE_U32_INTERLEAVE: need = g.num_ops * 34; break;
-            case GL_GATE_UNINTERLEAVE_TO_U32:
-            case GL_GATE_UNINTERLEAVE_TO_B32: need = g.num_ops * 67; break;
-            default: break;
-        }
-        if (need > cd->num_wires) return fail(ctx, GL_E_ARG, "gl_quotient_polys: gate does not fit the wires / constants");
+        TRY(quotient_gate_check(ctx, cd, g, i));
         a.gates[i] = g;
         ngc = std::max(ngc, quotient_gate_constraints(g));
     }
-    Guard g(ctx);
     const u64 n = (u64)1 << lg_n, lde_size = n << qdb;
     const uint32_t nterms = nch * (1 + chunks) + ngc;
     // tables: alpha powers [nch][nterms], k_is [R]
@@ -2236,22 +2287,38 @@ extern "C" int gl_quotient_polys(gl_ctx* ctx, const gl_circuit* cd, const gl_gat
     return finish(ctx);
 }
 
+extern "C" int gl_quotient_polys(gl_ctx* ctx, const gl_circuit* cd, const gl_gate* gates, const uint64_t* k_is,
+                                 gl_commit* constants_sigmas, gl_commit* wires, gl_commit* zs_pp,
+                                 const uint64_t* public_inputs_hash, const uint64_t* betas, const uint64_t* gammas,
+                                 const uint64_t* alphas, uint64_t* chunks_out, int space) {
+    if (!ctx) return GL_E_ARG;
+    Guard g(ctx);
+    return quotient_polys(ctx, cd, gates, k_is, constants_sigmas, wires, zs_pp, public_inputs_hash, betas, gammas, alphas,
+                          chunks_out, space);
+}
+
 // ------------------------------------------------------------------------------------------------
 // all_wires_permutation_partial_products: Z and the partial products, from the coefficients the two commits hold
 // ------------------------------------------------------------------------------------------------
-extern "C" int gl_permutation_zs(gl_ctx* ctx, const gl_circuit* cd, const uint64_t* k_is, gl_commit* constants_sigmas,
-                                 gl_commit* wires, const uint64_t* betas, const uint64_t* gammas,
-                                 uint64_t* zs_partial_products_out, int space, uint64_t* grand_products_out) {
-    if (!ctx) return GL_E_ARG;
+static int permutation_geometry_check(gl_ctx* ctx, const gl_circuit* cd) {
+    const uint32_t nch = cd->num_challenges, R = cd->num_routed_wires, deg = cd->quotient_degree_factor;
+    if (nch == 0 || nch > PERM_MAX_CHALLENGES || R == 0 || R > cd->num_wires || !is_pow2(deg))
+        return fail(ctx, GL_E_ARG, "gl_permutation_zs: unsupported circuit geometry");
+    if (nch * ((R + deg - 1) / deg) > PERM_MAX_SLOTS)
+        return fail(ctx, GL_E_ARG, "gl_permutation_zs: num_challenges * ceil(num_routed_wires / quotient_degree_factor) > 64");
+    return GL_OK;
+}
+
+// the body of gl_permutation_zs, with the ctx held
+static int permutation_zs(gl_ctx* ctx, const gl_circuit* cd, const uint64_t* k_is, gl_commit* constants_sigmas, gl_commit* wires,
+                          const uint64_t* betas, const uint64_t* gammas, uint64_t* zs_partial_products_out, int space,
+                          uint64_t* grand_products_out) {
     if (!cd || !k_is || !constants_sigmas || !wires || !betas || !gammas || !zs_partial_products_out)
         return fail(ctx, GL_E_ARG, "gl_permutation_zs: NULL argument");
     if (space != GL_HOST && space != GL_DEVICE) return fail(ctx, GL_E_ARG, "gl_permutation_zs: bad space");
     const uint32_t nch = cd->num_challenges, R = cd->num_routed_wires, deg = cd->quotient_degree_factor;
-    if (nch == 0 || nch > PERM_MAX_CHALLENGES || R == 0 || R > cd->num_wires || !is_pow2(deg))
-        return fail(ctx, GL_E_ARG, "gl_permutation_zs: unsupported circuit geometry");
+    TRY(permutation_geometry_check(ctx, cd));
     const uint32_t chunks = (R + deg - 1) / deg;
-    if (nch * chunks > PERM_MAX_SLOTS)
-        return fail(ctx, GL_E_ARG, "gl_permutation_zs: num_challenges * ceil(num_routed_wires / quotient_degree_factor) > 64");
     for (gl_commit* h : {constants_sigmas, wires}) {
         if (h->ctx != ctx || !h->finished || !h->coeffs.get())
             return fail(ctx, GL_E_STATE, "gl_permutation_zs: oracle is not a finished polynomial commit of this ctx");
@@ -2261,7 +2328,6 @@ extern "C" int gl_permutation_zs(gl_ctx* ctx, const gl_circuit* cd, const uint64
         return fail(ctx, GL_E_ARG, "gl_permutation_zs: column counts do not match the circuit description");
     if (wires->log_n != constants_sigmas->log_n || wires->log_n != cd->degree_bits)
         return fail(ctx, GL_E_ARG, "gl_permutation_zs: oracles of different degree");
-    Guard g(ctx);
     const uint32_t lg_n = cd->degree_bits;
     const u64 n = (u64)1 << lg_n;
     const uint32_t nblocks = (uint32_t)((n + PERM_BLOCK - 1) / PERM_BLOCK);
@@ -2311,6 +2377,175 @@ extern "C" int gl_permutation_zs(gl_ctx* ctx, const gl_circuit* cd, const uint64
     if (grand_products_out)
         for (uint32_t c = 0; c < nch; c++) grand_products_out[c] = grand[c];
     return GL_OK;
+}
+
+extern "C" int gl_permutation_zs(gl_ctx* ctx, const gl_circuit* cd, const uint64_t* k_is, gl_commit* constants_sigmas,
+                                 gl_commit* wires, const uint64_t* betas, const uint64_t* gammas,
+                                 uint64_t* zs_partial_products_out, int space, uint64_t* grand_products_out) {
+    if (!ctx) return GL_E_ARG;
+    Guard g(ctx);
+    return permutation_zs(ctx, cd, k_is, constants_sigmas, wires, betas, gammas, zs_partial_products_out, space,
+                          grand_products_out);
+}
+
+// ------------------------------------------------------------------------------------------------
+// plonky2::plonk::prover::prove from the witness on: the stages above chained by the Fiat-Shamir transcript
+// ------------------------------------------------------------------------------------------------
+// The prover's three commits; they die (back to the pool) when gl_prove returns, on every path.
+struct ProveOracles {
+    std::unique_ptr<gl_commit> wires, zs, quotient;
+};
+
+// Pops `n` challenges from the device challenger into host memory (one small copy and a synchronisation).
+static int draw_challenges(gl_ctx* ctx, gl_challenger* d_ch, const u64* observe, uint32_t n_obs, u64* d_out, uint32_t n,
+                           u64* host_out) {
+    launch_challenger_step(d_ch, observe, n_obs, d_out, n, nullptr, ctx->stream);
+    CK(cudaMemcpyAsync(host_out, d_out, (size_t)n * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    return finish(ctx);
+}
+
+static int prove_body(gl_ctx* ctx, const gl_circuit* cd, const gl_gate* gates, const uint64_t* k_is, gl_commit* cs,
+                      const uint64_t circuit_digest[4], const gl_fri_params* prm, const HostCols& witness, int space,
+                      const uint64_t* public_inputs, uint32_t num_public_inputs, uint64_t* proof_out, uint64_t fri_words,
+                      uint64_t total_words, ProveOracles& o) {
+    const uint32_t lg_n = cd->degree_bits, nch = cd->num_challenges, R = cd->num_routed_wires, qdf = cd->quotient_degree_factor;
+    const uint32_t rate_bits = prm->rate_bits, h = prm->cap_height, zcols = nch * ((R + qdf - 1) / qdf), qcols = nch * qdf;
+    const u64 n = (u64)1 << lg_n, cap_words = 4ull << h;
+    // the proof as it goes back: caps [3][2^h][4] | OpeningSet | FRI proof
+    PoolBuf out, st;
+    TRY(out.alloc(ctx, total_words * 8));
+    u64* d_caps = out.get();
+    u64* d_open = d_caps + 3 * cap_words;
+    u64* d_cs_open = d_open;                                   // constants | plonk_sigmas
+    u64* d_w_open = d_cs_open + 2 * (size_t)cs->c;             // wires
+    u64* d_z_open = d_w_open + 2 * (size_t)cd->num_wires;      // plonk_zs
+    u64* d_znext_open = d_z_open + 2 * (size_t)nch;            // plonk_zs_next
+    u64* d_pp_open = d_znext_open + 2 * (size_t)nch;           // partial_products
+    u64* d_q_open = d_pp_open + 2 * (size_t)(zcols - nch);     // quotient_polys
+    u64* d_fri = d_q_open + 2 * (size_t)qcols;
+    // transcript state: challenger [32] | circuit digest [4] | public-inputs hash [4] | challenges [max(2 nch, 2)] | public inputs
+    static_assert(sizeof(gl_challenger) == 29 * 8, "gl_challenger layout");
+    TRY(st.alloc(ctx, (32 + 8 + 2 * (size_t)nch + 2 + num_public_inputs) * 8));
+    gl_challenger* d_ch = (gl_challenger*)st.get();
+    u64* d_digest = st.get() + 32;
+    u64* d_pih = d_digest + 4;
+    u64* d_chal = d_pih + 4;
+    u64* d_pi = d_chal + 2 * (size_t)nch + 2;
+    CK(cudaMemsetAsync(d_ch, 0, sizeof(gl_challenger), ctx->stream));   // Challenger::new()
+    CK(cudaMemcpyAsync(d_digest, circuit_digest, 32, cudaMemcpyHostToDevice, ctx->stream));
+    if (num_public_inputs)
+        CK(cudaMemcpyAsync(d_pi, public_inputs, (size_t)num_public_inputs * 8, cudaMemcpyHostToDevice, ctx->stream));
+    launch_hash_no_pad_rows(d_pi, num_public_inputs, 1, d_pih, ctx->stream);   // no inputs: [0, 0, 0, 0]
+    // wires commit, then observe digest, pih, wires cap and draw betas, gammas
+    TRY(commit_make(ctx, witness, true, lg_n, cd->num_wires, rate_bits, h, HostCols(), nullptr, space, "gl_prove: wires commit",
+                    false, &o.wires));
+    CK(cudaMemcpyAsync(d_caps, o.wires->cap.get(), cap_words * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+    launch_challenger_step(d_ch, d_digest, 8, nullptr, 0, nullptr, ctx->stream);
+    std::vector<u64> bg(2 * (size_t)nch + 4);
+    u64 *betas = bg.data(), *gammas = betas + nch, *pih = gammas + nch;
+    CK(cudaMemcpyAsync(pih, d_pih, 32, cudaMemcpyDeviceToHost, ctx->stream));
+    TRY(draw_challenges(ctx, d_ch, d_caps, (uint32_t)cap_words, d_chal, 2 * nch, betas));
+    // Z and the partial products, resident, and their commit; observe the cap, draw alphas
+    {
+        PoolBuf zs;
+        TRY(zs.alloc(ctx, (size_t)zcols * n * 8));
+        TRY(permutation_zs(ctx, cd, k_is, cs, o.wires.get(), betas, gammas, zs.get(), GL_DEVICE, nullptr));
+        HostCols zin;
+        zin.flat = zs.get();
+        TRY(commit_make(ctx, zin, true, lg_n, zcols, rate_bits, h, HostCols(), nullptr, GL_DEVICE, "gl_prove: Z commit", false, &o.zs));
+    }
+    CK(cudaMemcpyAsync(d_caps + cap_words, o.zs->cap.get(), cap_words * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+    std::vector<u64> alphas(nch);
+    TRY(draw_challenges(ctx, d_ch, d_caps + cap_words, (uint32_t)cap_words, d_chal, nch, alphas.data()));
+    // the quotient chunks, resident, and their commit; observe the cap, draw zeta
+    {
+        PoolBuf q;
+        TRY(q.alloc(ctx, (size_t)qcols * n * 8));
+        TRY(quotient_polys(ctx, cd, gates, k_is, cs, o.wires.get(), o.zs.get(), pih, betas, gammas, alphas.data(), q.get(), GL_DEVICE));
+        HostCols qin;
+        qin.flat = q.get();
+        TRY(commit_make(ctx, qin, false, lg_n, qcols, rate_bits, h, HostCols(), nullptr, GL_DEVICE, "gl_prove: quotient commit", false,
+                        &o.quotient));
+    }
+    CK(cudaMemcpyAsync(d_caps + 2 * cap_words, o.quotient->cap.get(), cap_words * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+    u64 zeta[2];
+    TRY(draw_challenges(ctx, d_ch, d_caps + 2 * cap_words, (uint32_t)cap_words, d_chal, 2, zeta));
+    const glh::ext z = {zeta[0], zeta[1]};
+    const glh::ext zn = glh::ext_pow(z, n);
+    if (zn.a == 1 && zn.b == 0)
+        return fail(ctx, GL_E_STATE, "gl_prove: Opening point is in the subgroup.");
+    const glh::ext gz = glh::ext_mul(z, glh::ext{glh::root_of_unity(lg_n), 0});
+    const u64 zeta_next[2] = {gz.a, gz.b};
+    // OpeningSet::new, written in place in the proof buffer
+    TRY(commit_eval(ctx, cs, 0, cs->c, zeta, d_cs_open, GL_DEVICE));
+    TRY(commit_eval(ctx, o.wires.get(), 0, o.wires->c, zeta, d_w_open, GL_DEVICE));
+    TRY(commit_eval(ctx, o.zs.get(), 0, nch, zeta, d_z_open, GL_DEVICE));
+    TRY(commit_eval(ctx, o.zs.get(), 0, nch, zeta_next, d_znext_open, GL_DEVICE));
+    if (zcols > nch) TRY(commit_eval(ctx, o.zs.get(), nch, zcols - nch, zeta, d_pp_open, GL_DEVICE));
+    TRY(commit_eval(ctx, o.quotient.get(), 0, qcols, zeta, d_q_open, GL_DEVICE));
+    // observe_openings(to_fri_openings()): [constants, plonk_sigmas, wires, plonk_zs, partial_products, quotient_polys], then
+    // [plonk_zs_next]
+    launch_challenger_step(d_ch, d_open, (uint32_t)(d_znext_open - d_open), nullptr, 0, nullptr, ctx->stream);
+    launch_challenger_step(d_ch, d_pp_open, (uint32_t)(d_fri - d_pp_open), nullptr, 0, nullptr, ctx->stream);
+    launch_challenger_step(d_ch, d_znext_open, 2 * nch, nullptr, 0, nullptr, ctx->stream);
+    gl_challenger ch;
+    CK(cudaMemcpyAsync(&ch, d_ch, sizeof ch, cudaMemcpyDeviceToHost, ctx->stream));
+    TRY(finish(ctx));
+    // prove_openings over get_fri_instance(zeta): every polynomial at zeta, the Z polynomials at g * zeta
+    gl_commit* oracles[4] = {cs, o.wires.get(), o.zs.get(), o.quotient.get()};
+    std::vector<gl_fri_poly> polys;
+    for (uint32_t i = 0; i < 4; i++)
+        for (uint32_t j = 0; j < oracles[i]->c; j++) polys.push_back({i, j});
+    const uint32_t at_zeta = (uint32_t)polys.size();
+    for (uint32_t j = 0; j < nch; j++) polys.push_back({2, j});
+    gl_fri_batch batches[2] = {{{zeta[0], zeta[1]}, 0, at_zeta}, {{zeta_next[0], zeta_next[1]}, at_zeta, nch}};
+    return fri_prove_body(ctx, oracles, 4, batches, 2, polys.data(), prm, &ch, fri_words, d_fri, proof_out, out.get(), total_words);
+}
+
+extern "C" int gl_prove(gl_ctx* ctx, const gl_circuit* cd, const gl_gate* gates, const uint64_t* k_is, gl_commit* constants_sigmas,
+                        const uint64_t circuit_digest[4], const gl_fri_params* prm, const uint64_t* wires,
+                        const uint64_t* const* wires_cols, int space, const uint64_t* public_inputs, uint32_t num_public_inputs,
+                        uint64_t* proof_out, uint64_t proof_cap_words, uint64_t* proof_words_out) {
+    if (!ctx) return GL_E_ARG;
+    if (!cd || !gates || !k_is || !constants_sigmas || !circuit_digest || !prm || !proof_words_out ||
+        (num_public_inputs && !public_inputs))
+        return fail(ctx, GL_E_ARG, "gl_prove: NULL argument");
+    if ((wires != nullptr) == (wires_cols != nullptr))
+        return fail(ctx, GL_E_ARG, "gl_prove: pass the witness either as one array or as one array per wire");
+    if ((space != GL_HOST && space != GL_DEVICE) || (wires_cols && space != GL_HOST))
+        return fail(ctx, GL_E_ARG, "gl_prove: bad space (per-wire arrays are host memory)");
+    const gl_commit* cs = constants_sigmas;
+    const uint32_t nch = cd->num_challenges, R = cd->num_routed_wires, qdf = cd->quotient_degree_factor;
+    // every geometry check of the two stage calls, before any work is done
+    TRY(permutation_geometry_check(ctx, cd));
+    TRY(quotient_geometry_check(ctx, cd));
+    TRY(quotient_rate_check(ctx, cd, prm->rate_bits));
+    for (uint32_t i = 0; i < cd->num_gates; i++) TRY(quotient_gate_check(ctx, cd, gates[i], i));
+    if (ctx->shard_count != 1) return fail(ctx, GL_E_ARG, "gl_prove: sharded proving is not supported");
+    if (cs->ctx != ctx || !cs->finished || !cs->coeffs.get() || cs->salt || cs->shard_count != 1)
+        return fail(ctx, GL_E_ARG, "gl_prove: constants_sigmas must be a finished, unblinded, unsharded polynomial commit of this ctx");
+    if (cs->log_n != cd->degree_bits || cs->c != cd->num_constants + R)
+        return fail(ctx, GL_E_ARG, "gl_prove: constants_sigmas does not have the circuit's degree and num_constants + num_routed_wires columns");
+    if (cs->rate_bits != prm->rate_bits || cs->cap_height != prm->cap_height)
+        return fail(ctx, GL_E_ARG, "gl_prove: the FRI config's rate_bits / cap_height differ from constants_sigmas'");
+    TRY(fri_params_check(ctx, prm, "gl_prove"));
+    const uint32_t zcols = nch * ((R + qdf - 1) / qdf), qcols = nch * qdf;
+    const uint32_t ocols[4] = {cs->c, cd->num_wires, zcols, qcols};
+    uint64_t fri_words = 0;
+    if (gl_fri_proof_words(prm, ocols, 4, cd->degree_bits, &fri_words) != GL_OK)
+        return fail(ctx, GL_E_ARG, "gl_prove: reduction_arity_bits do not fit the degree / cap_height");
+    const uint64_t total = 3 * (4ull << prm->cap_height) + 2ull * (cs->c + cd->num_wires + 2 * nch + (zcols - nch) + qcols) + fri_words;
+    *proof_words_out = total;
+    if (!proof_out || proof_cap_words < total) return fail(ctx, GL_E_ARG, "gl_prove: proof buffer too small (see *proof_words_out)");
+    Guard g(ctx);
+    HostCols witness;
+    witness.flat = const_cast<uint64_t*>(wires);
+    witness.cols = const_cast<uint64_t* const*>(wires_cols);
+    ProveOracles o;
+    int rc = prove_body(ctx, cd, gates, k_is, constants_sigmas, circuit_digest, prm, witness, space, public_inputs, num_public_inputs,
+                        proof_out, fri_words, total, o);
+    if (rc != GL_OK) quiesce(ctx);   // nothing of a failed call is still running when its commits go back to the pool
+    return rc;
 }
 
 extern "C" int gl_pow_grind(gl_ctx* ctx, const uint64_t state[12], uint32_t input_pos, uint32_t min_leading_zeros,

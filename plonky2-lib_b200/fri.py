@@ -330,13 +330,8 @@ def parse_flat_proof(flat: np.ndarray, oracle_columns: Sequence[int], fri_params
     return {"commit_phase_merkle_caps": caps, "query_round_proofs": rounds, "final_poly": final, "pow_witness": pow_witness}
 
 
-def prove_openings_device(oracles, batches, challenger: Challenger, fri_params: FriParams, ctx: Optional[Context] = None,
-                          flat: bool = False):
-    """PolynomialBatch::prove_openings through ONE C-ABI call (gl_fri_prove): the transcript runs on the device from the
-    Challenger's current state and comes back advanced past the proof; three host synchronisations in total."""
-    import ctypes as C
-
-    ctx = _ctx(ctx)
+def c_params(fri_params: FriParams) -> N.FriParams:
+    """gl_fri_params of FriParams (FriConfig, reduction_arity_bits, the GL_COMPAT_FRI_FINAL_POLY_TIMES_X form)."""
     cfg = fri_params.config
     prm = N.FriParams()
     prm.rate_bits, prm.cap_height, prm.proof_of_work_bits, prm.num_query_rounds = cfg.rate_bits, cfg.cap_height, cfg.proof_of_work_bits, cfg.num_query_rounds
@@ -344,6 +339,17 @@ def prove_openings_device(oracles, batches, challenger: Challenger, fri_params: 
     for i, ab in enumerate(fri_params.reduction_arity_bits):
         prm.reduction_arity_bits[i] = ab
     prm.flags = N.GL_COMPAT_FRI_FINAL_POLY_TIMES_X if fri_params.final_poly_times_x else 0
+    return prm
+
+
+def prove_openings_device(oracles, batches, challenger: Challenger, fri_params: FriParams, ctx: Optional[Context] = None,
+                          flat: bool = False):
+    """PolynomialBatch::prove_openings through ONE C-ABI call (gl_fri_prove): the transcript runs on the device from the
+    Challenger's current state and comes back advanced past the proof; three host synchronisations in total."""
+    import ctypes as C
+
+    ctx = _ctx(ctx)
+    prm = c_params(fri_params)
     ch = N.Challenger()
     for i in range(12):
         ch.sponge_state[i] = int(challenger.sponge_state[i])

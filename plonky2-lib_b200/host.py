@@ -21,6 +21,7 @@ from typing import List, Optional, Sequence
 import numpy as np
 
 from . import _native as N
+from . import wire
 
 P = 0xFFFFFFFF00000001
 
@@ -677,6 +678,73 @@ def permutation_zs(circuit, k_is, constants_sigmas: "PolynomialBatch", wires: "P
     ctx.check(ctx._lib.gl_permutation_zs(ctx._h, C.byref(cd), k.ctypes.data, constants_sigmas._h, wires._h, b.ctypes.data,
                                          g.ctypes.data, o.ptr, o.space, grand.ctypes.data))
     return out, grand[:nch]
+
+
+def opening_set_lengths(circuit) -> dict:
+    """OpeningSet field -> number of extension values, for a circuit tuple as compute_quotient_polys takes it."""
+    cd = N.Circuit(*[int(v) for v in circuit])
+    nch, qdf = cd.num_challenges, cd.quotient_degree_factor
+    num_prods = -(-cd.num_routed_wires // qdf) - 1
+    return dict(zip(wire.OPENING_SET_FIELDS, (cd.num_constants, cd.num_routed_wires, cd.num_wires, nch, nch, nch * num_prods, nch * qdf)))
+
+
+def prove(circuit, gates, k_is, constants_sigmas: "PolynomialBatch", circuit_digest, fri_params, wires, public_inputs=(),
+          ctx=None) -> dict:
+    """plonky2::plonk::prover::prove from the witness on, in one call (gl_prove): the wires, Z and quotient commits, the
+    transcript, the OpeningSet and the opening proof all on the device; one copy brings the proof back.  circuit / gates /
+    k_is as compute_quotient_polys takes them; constants_sigmas: the resident prover-data commit; circuit_digest: the four
+    elements of prover_data.circuit_digest; fri_params: fri.FriParams.  wires: the witness [num_wires][n] as a numpy array, a
+    list of 1-D numpy arrays (one per wire), a torch CUDA tensor or a DeviceBuffer.  Returns dict(caps=(wires_cap,
+    plonk_zs_partial_products_cap, quotient_polys_cap), openings={OpeningSet field: [k][2]}, opening_proof=FriProof as
+    fri.parse_flat_proof gives it, public_inputs, words=the stream gl_prove wrote); wire.proof_with_public_inputs_to_bytes
+    turns it into ProofWithPublicInputs bytes."""
+    from .fri import c_params, parse_flat_proof
+
+    ctx = _ctx(ctx)
+    cd = N.Circuit(*[int(v) for v in circuit])
+    arr = (N.Gate * len(gates))(*[N.Gate(*[int(v) for v in tuple(g)[:5]], 0) for g in gates])
+    k, digest, pis = _h(k_is), _h(circuit_digest), _h(public_inputs).reshape(-1)
+    if len(k) < cd.num_routed_wires or digest.shape != (4,) or len(gates) < cd.num_gates:
+        raise GlPanic(N.GL_E_ARG, "prove: fewer k_is than num_routed_wires or gates than num_gates, or a circuit digest that is "
+                                  "not four elements")
+    prm = c_params(fri_params)
+    # the library reads num_wires x 2^degree_bits words of witness and cannot check the caller's sizes: they are checked here
+    n = 1 << cd.degree_bits
+    flat, cols, space, keep = None, None, N.GL_HOST, None
+    if isinstance(wires, (list, tuple)):
+        keep = [_h(w) for w in wires]
+        if len(keep) != cd.num_wires or any(w.shape != (n,) for w in keep):
+            raise GlPanic(N.GL_E_ARG, f"prove: the witness must be num_wires = {cd.num_wires} columns of 2^degree_bits = {n} values")
+        cols = (C.c_void_p * len(keep))(*[w.ctypes.data for w in keep])
+    else:
+        dev = isinstance(wires, DeviceBuffer) or _is_torch(wires)
+        b = _Buf(wires if dev else _h(wires))
+        if (b.nbytes < cd.num_wires * n * 8) if dev else (b.keep.shape != (cd.num_wires, n)):
+            raise GlPanic(N.GL_E_ARG, f"prove: the witness must be [num_wires = {cd.num_wires}][2^degree_bits = {n}]")
+        flat, space, keep = b.ptr, b.space, b
+    words = C.c_uint64(0)
+    args = (ctx._h, C.byref(cd), arr, k.ctypes.data, constants_sigmas._h, digest.ctypes.data, C.byref(prm), flat, cols, space,
+            pis.ctypes.data, pis.size)
+    rc = ctx._lib.gl_prove(*args, None, 0, C.byref(words))     # the size: a NULL buffer is rejected after it is set
+    if words.value == 0:
+        ctx.check(rc)
+    out = np.empty(words.value, dtype=np.uint64)
+    ctx.check(ctx._lib.gl_prove(*args, out.ctypes.data, out.size, C.byref(words)))
+    del keep
+    h = fri_params.config.cap_height
+    at = 0
+    caps = []
+    for _ in range(3):
+        caps.append(out[at:at + (4 << h)].reshape(-1, 4))
+        at += 4 << h
+    lens = opening_set_lengths(circuit)
+    openings = {}
+    for f, cnt in lens.items():
+        openings[f] = out[at:at + 2 * cnt].reshape(-1, 2)
+        at += 2 * cnt
+    widths = [constants_sigmas.leaf_len, cd.num_wires, lens["plonk_zs"] + lens["partial_products"], lens["quotient_polys"]]
+    return {"caps": tuple(caps), "openings": openings, "opening_proof": parse_flat_proof(out[at:], widths, fri_params),
+            "public_inputs": pis.copy(), "words": out}
 
 
 # ------------------------------------------------------------------------------------------------

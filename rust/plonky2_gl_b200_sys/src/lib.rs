@@ -113,6 +113,11 @@ extern "C" {
     pub fn gl_permutation_zs(ctx: *mut gl_ctx, circuit: *const gl_circuit, k_is: *const u64, constants_sigmas: *mut gl_commit,
                              wires: *mut gl_commit, betas: *const u64, gammas: *const u64, zs_partial_products_out: *mut u64,
                              space: c_int, grand_products_out: *mut u64) -> c_int;
+    // plonk/prover.rs::prove from the witness on: every stage above chained by the transcript, one proof stream back
+    pub fn gl_prove(ctx: *mut gl_ctx, circuit: *const gl_circuit, gates: *const gl_gate, k_is: *const u64,
+                    constants_sigmas: *mut gl_commit, circuit_digest: *const u64, prm: *const gl_fri_params, wires: *const u64,
+                    wires_cols: *const *const u64, space: c_int, public_inputs: *const u64, num_public_inputs: u32,
+                    proof_out: *mut u64, proof_cap_words: u64, proof_words_out: *mut u64) -> c_int;
     // N1 in one call: prove_openings + fri_proof with the transcript on the device; fork-version switches
     pub fn gl_ctx_set_compat(ctx: *mut gl_ctx, flags: u32) -> c_int;
     pub fn gl_fri_proof_words(prm: *const gl_fri_params, oracle_columns: *const u32, num_oracles: u32, degree_bits: u32,
