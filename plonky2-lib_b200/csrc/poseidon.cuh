@@ -18,8 +18,9 @@
 //   * The next round's constants are the addend of the first DFMA of each row (a constant-bank
 //     operand), so "add round constants" costs nothing.
 //   * The 22 partial rounds run as 11 fused pairs (poseidon_partial_pair): two linear layers minus the
-//     lane-0 path are one matrix N = M M' with entries < 2^14, still exact in FP64.
-// The 12-lane state lives in 24 registers of one thread.  Measured: 1.39 G permutations/s on one B200.
+//     lane-0 path are one matrix N = M M' with entries < 2^14, still exact in FP64.  Between two pairs lanes 1..11
+//     stay two doubles (poseidon_renorm), only lane 0 is folded to a 64-bit element for its S-box.
+// The 12-lane state lives in 24 registers of one thread (46 during the partial rounds).  Measured: 1.39 G permutations/s on one B200.
 #pragma once
 #include "gl_field.cuh"
 
@@ -68,8 +69,8 @@ GL_D void poseidon_sbox_split(u64 x, double& dl, double& dh) {
 }
 // (exactness: every operand is an integer multiple of 2^-1074, so FP64 sums and products are exact while they stay below
 // 2^53 in magnitude.  A full round's layer sees inputs in [0, 3 * 2^32); the fused pair's CIRC^2 form sees lane 0 in
-// [0, 3 * 2^32) and the other lanes in [0, 2^32).  tests/test_poseidon_schedule_model_cpu.py bounds every intermediate
-// exactly: all stay below 2^51.)
+// [0, 3 * 2^32) and the other lanes in [0, 2^33) (poseidon_renorm's L and H).  tests/test_poseidon_schedule_model_cpu.py
+// and tests/test_poseidon_split_pairs_model_cpu.py bound every intermediate exactly: all stay below 2^50.)
 
 // MDS entries: M[r][j] = CIRC[(j - r) mod 12] + (r == j ? DIAG[r] : 0)
 __host__ __device__ constexpr int poseidon_mds_entry(int r, int j) {
@@ -92,7 +93,8 @@ __constant__ double2 c_poseidon_pair_k[(POSEIDON_PARTIAL / 2) * POSEIDON_WIDTH];
 //   A + 2^32 B = (A - bh) + 2^32 (bh + b0)  (mod p),
 // one carry chain without a multiply.  A - bh does not borrow: the tables keep A >= 2^40 (their positive offsets).  The sum
 // is below 2^64 + 2^51, so it wraps at most once; the wrap c is folded back as c * (2^32 - 1) = c * 2^32 - c, which cannot
-// wrap again (the wrapped sum is below 2^51).
+// wrap again (the wrapped sum is below 2^51).  After the last fused pair it takes poseidon_renorm's (L, H) as they are:
+// L >= 2^32 - 2^18 > H >> 32.
 GL_D u64 poseidon_fold(double al, double ah) {
     const u64 A = double_bits(al), B = double_bits(ah);
     u32 y0, y1;
@@ -116,7 +118,7 @@ GL_D u64 poseidon_fold(double al, double ah) {
 // of round a's S-box (constants already added).  With x~ = state after that S-box (lane 0 only):
 //   y0 = M[0] . x~ + rc[a+1][0]                     -> S-box of round a + 1 -> sigma
 //   z  = N x~ + K + M[.][0] * sigma                 (N = M M' without the lane-0 path)
-// 336 DFMA instead of 576, 13 folds instead of 24; every partial sum stays below 2^50 (exact).
+// 2 folds (y0 and lane 0 of z) and 11 renormalisations instead of 24 folds; every partial sum stays below 2^50 (exact).
 // ------------------------------------------------------------------------------------------------------------
 // Circulant products through a 4 x 3 Good-Thomas FFT (exact, FP64 pipe).
 //
@@ -128,8 +130,11 @@ GL_D u64 poseidon_fold(double al, double ah) {
 // units of 2^-1074 (signed: differences can be negative denormals), so the arithmetic is exact and the final,
 // non-negative results are again integer bit patterns.  SQ = 1 applies the circulant twice (kernel convolved with
 // itself), which is what the fused partial-round pair needs.
-template <int SQ>
-GL_D void poseidon_circ12(const double x[12], double y[12]) {
+// E0 adds CIRC (e e_0) = e col0(CIRC) to the result (the pair's rank-one lane-0 term): the forward FFT of e_0 is 1 in
+// U0, U2 and UR of residue class b = 0, so its image after the single circulant's kernel is e {K0, K2, KR, KI}[0][b] in
+// (v0, v2, vr, vi) of class b -- 12 FMAs after the kernel multiply instead of 12 multiply-adds per output lane.
+template <int SQ, bool E0 = false>
+GL_D void poseidon_circ12(const double x[12], double y[12], double e = 0.) {
     constexpr double K0[2][3] = {{16., 32., 16.}, {5120., 5120., 6144.}};
     constexpr double K2[2][3] = {{-1., 8., 2.}, {132., -48., 240.}};
     constexpr double KR[2][3] = {{2., -1., -16.}, {54., 486., -162.}};
@@ -148,8 +153,8 @@ GL_D void poseidon_circ12(const double x[12], double y[12]) {
 #pragma unroll
     for (int b = 0; b < 3; b++) {
         const int b1 = (b + 2) % 3, b2 = (b + 1) % 3;        // (b - 1) mod 3, (b - 2) mod 3
-        const double v0 = __fma_rn(K0[SQ][2], U0[b2], __fma_rn(K0[SQ][1], U0[b1], K0[SQ][0] * U0[b]));
-        const double v2 = __fma_rn(K2[SQ][2], U2[b2], __fma_rn(K2[SQ][1], U2[b1], K2[SQ][0] * U2[b]));
+        double v0 = __fma_rn(K0[SQ][2], U0[b2], __fma_rn(K0[SQ][1], U0[b1], K0[SQ][0] * U0[b]));
+        double v2 = __fma_rn(K2[SQ][2], U2[b2], __fma_rn(K2[SQ][1], U2[b1], K2[SQ][0] * U2[b]));
         double vr = KR[SQ][0] * UR[b], vi = KR[SQ][0] * UI[b];
         vr = __fma_rn(-KI[SQ][0], UI[b], vr);
         vi = __fma_rn(KI[SQ][0], UR[b], vi);
@@ -161,6 +166,12 @@ GL_D void poseidon_circ12(const double x[12], double y[12]) {
         vi = __fma_rn(KR[SQ][2], UI[b2], vi);
         vr = __fma_rn(-KI[SQ][2], UI[b2], vr);
         vi = __fma_rn(KI[SQ][2], UR[b2], vi);
+        if (E0) {
+            v0 = __fma_rn(K0[0][b], e, v0);
+            v2 = __fma_rn(K2[0][b], e, v2);
+            vr = __fma_rn(KR[0][b], e, vr);
+            vi = __fma_rn(KI[0][b], e, vi);
+        }
         const double sm = v0 + v2, df = v0 - v2;
         y[IDX[0][b]] = sm + vr;
         y[IDX[2][b]] = sm - vr;
@@ -191,44 +202,65 @@ GL_D void poseidon_full_round(u64 s[12], const double2* __restrict__ rc) {
     }
 }
 
+// Lanes 1..11 between two fused pairs: the pair's accumulators A = a0 + 2^32 a1, B = b0 + 2^32 b1 (A in [2^32, 2^50),
+// B < 2^50) are not folded to a field element, only brought back to two doubles the next pair's layers can read.
+// 2^64 = 2^32 - 1 (mod p):
+//   A + 2^32 B = (a0 - b1 + 2^32) + 2^32 (a1 - 1 + b0 + b1)  (mod p),
+// L = a0 - b1 + 2^32 in [2^32 - 2^18, 2^33) (b1 < 2^18), H = a1 - 1 + b0 + b1 in [0, 2^32 + 2^19) (a1 >= 1).  The 2^32 in L
+// is paid for by the -1 in H, so the value is congruent without any table offset.  Five two-input carry-chain
+// instructions instead of the fold's eight plus the next pair's two zero-extensions.
+GL_D void poseidon_renorm(double al, double ah, double& l, double& h) {
+    const u64 A = double_bits(al), B = double_bits(ah);
+    u32 l0, l1, h0, h1;
+    asm("{\n\t"
+        ".reg .u32 t;\n\t"
+        "sub.cc.u32 %0, %4, %7;\n\t"      // L = 2^32 + a0 - b1
+        "subc.u32 %1, 1, 0;\n\t"
+        "add.u32 t, %5, %7;\n\t"          // a1 + b1 - 1 < 2^19
+        "sub.u32 t, t, 1;\n\t"
+        "add.cc.u32 %2, t, %6;\n\t"       // H = (a1 + b1 - 1) + b0
+        "addc.u32 %3, 0, 0;\n\t"
+        "}"
+        : "=&r"(l0), "=&r"(l1), "=&r"(h0), "=&r"(h1)
+        : "r"((u32)A), "r"((u32)(A >> 32)), "r"((u32)B), "r"((u32)(B >> 32)));
+    l = __longlong_as_double((long long)gl_pack(l0, l1));
+    h = __longlong_as_double((long long)gl_pack(h0, h1));
+}
+
 // Two consecutive partial rounds in FFT form.  With M = CIRC + 8 e0 e0^T and M' = M without its row 0,
 //   N x~ = M M' x~ = CIRC^2 x~ + col0(CIRC) * (8 x~_0 - Yraw),   Yraw = M[0] . x~  (the unfolded y0 without its constant)
-// so z = CIRC^2 x~ (90 operations through poseidon_circ12<1>) + col0(CIRC) * w + M[.][0] * sigma + K: 280 FP64
-// operations per pair instead of 336, 13 folds.
-GL_D void poseidon_partial_pair(u64 s[12], int pair) {
-    double dl[12], dh[12];
-#pragma unroll
-    for (int i = 1; i < 12; i++) {
-        dl[i] = u32_as_denormal((u32)s[i]);
-        dh[i] = u32_as_denormal((u32)(s[i] >> 32));
-    }
+// and M[.][0] = col0(CIRC) + 8 e0, so
+//   z = N x~ + M[.][0] sigma + K = CIRC (CIRC x~ + (w + sigma) e0) + 8 sigma e0 + K,   w = 8 x~_0 - Yraw:
+// the rank-one lane-0 terms go into the frequency domain of poseidon_circ12<1, true>, 258 FP64 operations per pair.
+// s0 is lane 0 as a 64-bit integer (the next S-box's input); lanes 1..11 enter and leave in split form, (xl, xh)[i] with
+// value xl + 2^32 xh: the halves of a folded lane for the first pair, poseidon_renorm's (L, H) after that.
+GL_D void poseidon_partial_pair(u64& s0, double xl[12], double xh[12], int pair) {
     // everything that does not depend on lane 0 first: the FP64 pipe works while lane 0 goes through its S-box
-    double yl = (double)poseidon_mds_entry(0, 1) * dl[1], yh = (double)poseidon_mds_entry(0, 1) * dh[1];
+    double yl = (double)poseidon_mds_entry(0, 1) * xl[1], yh = (double)poseidon_mds_entry(0, 1) * xh[1];
 #pragma unroll
     for (int j = 2; j < 12; j++) {
-        yl = __fma_rn((double)poseidon_mds_entry(0, j), dl[j], yl);
-        yh = __fma_rn((double)poseidon_mds_entry(0, j), dh[j], yh);
+        yl = __fma_rn((double)poseidon_mds_entry(0, j), xl[j], yl);
+        yh = __fma_rn((double)poseidon_mds_entry(0, j), xh[j], yh);
     }
-    poseidon_sbox_split(s[0], dl[0], dh[0]);
-    yl = __fma_rn((double)poseidon_mds_entry(0, 0), dl[0], yl);      // Yraw
-    yh = __fma_rn((double)poseidon_mds_entry(0, 0), dh[0], yh);
+    poseidon_sbox_split(s0, xl[0], xh[0]);
+    yl = __fma_rn((double)poseidon_mds_entry(0, 0), xl[0], yl);      // Yraw
+    yh = __fma_rn((double)poseidon_mds_entry(0, 0), xh[0], yh);
     const double2 ky = c_poseidon_rc_split[(POSEIDON_FULL_HALF + 2 * pair + 1) * 12];
+    // w before sigma: across sigma's S-box only (wl, wh) stay live, not (x~_0, Yraw) as well
+    const double wl = __fma_rn(8., xl[0], -yl), wh = __fma_rn(8., xh[0], -yh);
     double gl, gh;
     poseidon_sbox_split(poseidon_fold(yl + ky.x, yh + ky.y), gl, gh);
+    const double el = wl + gl, eh = wh + gh;
     double zl[12], zh[12];
-    poseidon_circ12<1>(dl, zl);
-    poseidon_circ12<1>(dh, zh);
-    const double wl = __fma_rn(8., dl[0], -yl), wh = __fma_rn(8., dh[0], -yh);
+    poseidon_circ12<1, true>(xl, zl, el);
+    poseidon_circ12<1, true>(xh, zh, eh);
     const double2* kk = c_poseidon_pair_k + pair * 12;
 #pragma unroll
     for (int r = 0; r < 12; r++) {
         const double2 k = kk[r];
-        const double c0 = (double)(poseidon_mds_entry(r, 0) - (r == 0 ? 8 : 0));   // col0(CIRC)
-        double tl = __fma_rn((double)poseidon_mds_entry(r, 0), gl, k.x);
-        double th = __fma_rn((double)poseidon_mds_entry(r, 0), gh, k.y);
-        tl = __fma_rn(c0, wl, tl);
-        th = __fma_rn(c0, wh, th);
-        s[r] = poseidon_fold(zl[r] + tl, zh[r] + th);
+        const double al = zl[r] + k.x, ah = zh[r] + k.y;
+        if (r == 0) s0 = poseidon_fold(__fma_rn(8., gl, al), __fma_rn(8., gh, ah));
+        else poseidon_renorm(al, ah, xl[r], xh[r]);
     }
 }
 
@@ -243,8 +275,17 @@ GL_D void poseidon_permute(u64 s[12]) {
 #pragma unroll 1
         for (int r = 0; r < POSEIDON_FULL_HALF; r++, rc += 12) poseidon_full_round(s, rc);
         if (phase == 0) {
+            double xl[12], xh[12];
+#pragma unroll
+            for (int i = 1; i < 12; i++) {
+                xl[i] = u32_as_denormal((u32)s[i]);
+                xh[i] = u32_as_denormal((u32)(s[i] >> 32));
+            }
 #pragma unroll 1
-            for (int pair = 0; pair < POSEIDON_PARTIAL / 2; pair++) poseidon_partial_pair(s, pair);
+            for (int pair = 0; pair < POSEIDON_PARTIAL / 2; pair++) poseidon_partial_pair(s[0], xl, xh, pair);
+            // the full rounds take 64-bit lanes: L + 2^32 H with L >= 2^32 - 2^18 > H >> 32, inside the fold's domain
+#pragma unroll
+            for (int i = 1; i < 12; i++) s[i] = poseidon_fold(xl[i], xh[i]);
         }
     }
 }

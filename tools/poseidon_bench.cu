@@ -29,8 +29,19 @@ __device__ __forceinline__ void poseidon_permute2(u64 s[12], u64 t[12]) {
 #pragma unroll 1
         for (int r = 0; r < POSEIDON_FULL_HALF; r++, rc += 12) { poseidon_full_round(s, rc); poseidon_full_round(t, rc); }
         if (phase == 0) {
+            double sl[12], sh[12], tl[12], th[12];
+#pragma unroll
+            for (int i = 1; i < 12; i++) {
+                sl[i] = u32_as_denormal((u32)s[i]); sh[i] = u32_as_denormal((u32)(s[i] >> 32));
+                tl[i] = u32_as_denormal((u32)t[i]); th[i] = u32_as_denormal((u32)(t[i] >> 32));
+            }
 #pragma unroll 1
-            for (int pair = 0; pair < POSEIDON_PARTIAL / 2; pair++) { poseidon_partial_pair(s, pair); poseidon_partial_pair(t, pair); }
+            for (int pair = 0; pair < POSEIDON_PARTIAL / 2; pair++) {
+                poseidon_partial_pair(s[0], sl, sh, pair);
+                poseidon_partial_pair(t[0], tl, th, pair);
+            }
+#pragma unroll
+            for (int i = 1; i < 12; i++) { s[i] = poseidon_fold(sl[i], sh[i]); t[i] = poseidon_fold(tl[i], th[i]); }
         }
     }
 }
@@ -94,8 +105,10 @@ __global__ void k_circ_extremes(const u64* halves, int cases, int* bad) {
 }
 
 // The same check for the inputs the S-box hand-off gives the layers: lanes in [0, 3 * 2^32) (dl = r0 - r2 - r3 + 2^33) for one
-// layer (SQ = 0); lane 0 in that range and lanes 1..11 in [0, 2^32) for the fused pair (SQ = 1).  ab[t][i] = (a, b): the
-// lane is a + 2 b, formed as an integer bit pattern the way poseidon_sbox_split forms it.
+// layer (SQ = 0); lane 0 in that range and lanes 1..11 in [0, 2^33) for the fused pair (SQ = 1, the range of poseidon_renorm's
+// (L, H)), with the rank-one term e e0 (e = 8 x_0 - M[0] . x + sigma, signed) applied in the frequency domain.
+// ab[t][i] = (a, b): lane 0 (and every lane of SQ = 0) is a + 2 b, formed as an integer bit pattern the way
+// poseidon_sbox_split forms it; lanes 1..11 of SQ = 1 are a + 2^32 (b >> 31).
 __global__ void k_circ_handoff(const u32* ab, int cases, int* bad) {
     int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= cases) return;
@@ -105,11 +118,13 @@ __global__ void k_circ_handoff(const u32* ab, int cases, int* bad) {
         double x[12], y[12];
         u64 xi[12], c1[12], c2[12];
         for (int i = 0; i < 12; i++) {
-            xi[i] = (sq == 0 || i == 0) ? (u64)h[2 * i] + 2 * (u64)h[2 * i + 1] : (u64)h[2 * i];
+            xi[i] = (sq == 0 || i == 0) ? (u64)h[2 * i] + 2 * (u64)h[2 * i + 1] : (u64)h[2 * i] + ((u64)(h[2 * i + 1] >> 31) << 32);
             x[i] = __longlong_as_double((long long)xi[i]);
         }
+        long long e = 8 * (long long)xi[0] + (long long)(xi[1] ^ xi[5]);   // + sigma, any value in the lanes' range
+        for (int j = 0; j < 12; j++) e -= (long long)(C[j] + (j == 0 ? 8 : 0)) * (long long)xi[j];
         if (sq == 0) poseidon_circ12<0>(x, y);
-        else poseidon_circ12<1>(x, y);
+        else poseidon_circ12<1, true>(x, y, e < 0 ? -__longlong_as_double(-e) : __longlong_as_double(e));
         for (int r = 0; r < 12; r++) {
             u64 acc = 0;
             for (int i = 0; i < 12; i++) acc += (u64)C[i] * xi[(i + r) % 12];
@@ -120,8 +135,11 @@ __global__ void k_circ_handoff(const u32* ab, int cases, int* bad) {
             for (int i = 0; i < 12; i++) acc += (u64)C[i] * c1[(i + r) % 12];
             c2[r] = acc;
         }
-        for (int r = 0; r < 12; r++)
-            if (double_bits(y[r]) != (sq ? c2[r] : c1[r])) atomicAdd(bad, 1);
+        for (int r = 0; r < 12; r++) {
+            // without the pair's table offsets z can be negative: compare signed integers
+            const long long got = y[r] < 0 ? -(long long)double_bits(-y[r]) : (long long)double_bits(y[r]);
+            if (got != (sq ? (long long)c2[r] + C[(12 - r) % 12] * e : (long long)c1[r])) atomicAdd(bad, 1);
+        }
     }
 }
 
@@ -141,6 +159,21 @@ __global__ void k_forms(const u64* w, int cases, int* bad) {
     if ((u64)(((u128)l + ((u128)h << 32) + (u128)GL_P * 4 - POSEIDON_HANDOFF_BIAS) % GL_P) != x7) atomicAdd(bad, 1);
     const u64 y = poseidon_fold(__longlong_as_double((long long)A), __longlong_as_double((long long)B));
     if (y % GL_P != (u64)(((u128)A + ((u128)B << 32)) % GL_P)) atomicAdd(bad, 1);
+}
+
+// poseidon_renorm at its extremes against 128-bit arithmetic: A in [2^32, 2^50), B in [0, 2^50) give L in [2^32 - 2^18, 2^33),
+// H < 2^32 + 2^19 with L + 2^32 H = A + 2^32 B (mod p), and the fold after the last pair takes (L, H).  w[t] = (A, B).
+__global__ void k_renorm(const u64* w, int cases, int* bad) {
+    int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= cases) return;
+    typedef unsigned __int128 u128;
+    const u64 A = w[2 * t], B = w[2 * t + 1];
+    double dl, dh;
+    poseidon_renorm(__longlong_as_double((long long)A), __longlong_as_double((long long)B), dl, dh);
+    const u64 l = double_bits(dl), h = double_bits(dh), want = (u64)(((u128)A + ((u128)B << 32)) % GL_P);
+    if (l < (1ULL << 32) - (1ULL << 18) || l >= (1ULL << 33) || h >= (1ULL << 32) + (1ULL << 19)) atomicAdd(bad, 1);
+    if ((u64)(((u128)l + ((u128)h << 32)) % GL_P) != want) atomicAdd(bad, 1);
+    if (poseidon_fold(dl, dh) % GL_P != want) atomicAdd(bad, 1);
 }
 
 int main() {
@@ -252,6 +285,36 @@ int main() {
         k_forms<<<cases / 128, 128>>>(dw, cases, dbad);
         cudaMemcpy(&hbad, dbad, 4, cudaMemcpyDeviceToHost);
         printf("{\"handoff_fold_cases\": %d, \"mismatches\": %d}\n", cases, hbad);
+        ok &= hbad == 0;
+        free(hw);
+    }
+    {
+        const int cases = 1 << 16;
+        u64* hw = (u64*)malloc((size_t)cases * 16);
+        u64 st = 0x6A09E667F3BCC909ULL;
+        const u64 AMIN = 1ULL << 32, AMAX = (1ULL << 50) - 1, BMAX = (1ULL << 50) - 1;
+        for (int t = 0; t < cases; t++) {
+            u64 r[2];
+            for (int k = 0; k < 2; k++) { st ^= st << 13; st ^= st >> 7; st ^= st << 17; r[k] = st; }
+            const int mode = t & 7;   // b1 at its maximum, a0 = 0, b0 = 0xffffffff, a1 = 1, A and B at their ends, then random
+            u64 A = AMIN + r[0] % (AMAX - AMIN + 1), B = r[1] & BMAX;
+            if (mode == 0) { A &= ~0xFFFFFFFFULL; B = BMAX; }
+            else if (mode == 1) { A = AMIN; B = BMAX; }
+            else if (mode == 2) { A = AMAX; B = 0; }
+            else if (mode == 3) { A = AMIN; B = 0xFFFFFFFFULL; }
+            else if (mode == 4) { A &= ~0xFFFFFFFFULL; B |= 0xFFFFFFFFULL; }
+            else if (mode == 5) B |= 0xFFFFFFFFULL;
+            hw[2 * t] = A; hw[2 * t + 1] = B;
+        }
+        u64* dw;
+        int *dbad, hbad = 0;
+        cudaMalloc(&dw, (size_t)cases * 16);
+        cudaMalloc(&dbad, 4);
+        cudaMemcpy(dw, hw, (size_t)cases * 16, cudaMemcpyHostToDevice);
+        cudaMemset(dbad, 0, 4);
+        k_renorm<<<cases / 128, 128>>>(dw, cases, dbad);
+        cudaMemcpy(&hbad, dbad, 4, cudaMemcpyDeviceToHost);
+        printf("{\"renorm_cases\": %d, \"mismatches\": %d}\n", cases, hbad);
         ok &= hbad == 0;
         free(hw);
     }
