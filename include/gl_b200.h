@@ -15,6 +15,10 @@
  *  - `space` says where the caller's buffers live: GL_HOST (pageable or pinned host memory; the
  *    library stages the copies) or GL_DEVICE (device pointers on the ctx's device; used by callers
  *    that keep data resident, e.g. bench.py's `value` leg).
+ *  - GL_DEVICE buffers go to the kernels as they are: every GL_DEVICE buffer of 16 bytes or more must be 16-byte
+ *    aligned, a smaller one (a single element) 8-byte aligned.  A violation returns GL_E_ARG, naming the entry point
+ *    and the argument, before any copy or launch.  Allocations of cudaMalloc, torch and gl_dev_alloc qualify; a view
+ *    at an odd element offset does not.  GL_HOST buffers have no alignment rule (the library stages them).
  *  - every function returns 0 on success or a GL_E_* code; gl_last_error() gives the text.  The
  *    upstream functions are infallible and panic on contract violation (log2_strict on a
  *    non-power-of-two, `cap_height <= log2(leaves.len())`, inconsistent polynomial degrees): those

@@ -313,6 +313,18 @@ static int downloads_wait(gl_ctx* ctx) {
     return GL_OK;
 }
 
+// A GL_DEVICE buffer goes to the kernels as it is, and they read and write it in 16-byte pairs (Poseidon states,
+// digests, NTT outputs) or through TMA descriptors, whose base must be 16-byte aligned.  So a device buffer of 16 bytes
+// or more must be 16-byte aligned, a smaller one 8-byte aligned; GL_E_ARG otherwise, before any copy or launch.
+// Host buffers are staged into pool blocks and need nothing.  `what` names the entry point and the argument.
+static int check_device_ptr(gl_ctx* ctx, int space, const void* p, size_t bytes, const char* what) {
+    if (space != GL_DEVICE || !p || !bytes) return GL_OK;
+    const uintptr_t align = bytes >= 16 ? 16 : 8;
+    if (((uintptr_t)p & (align - 1)) == 0) return GL_OK;
+    return fail(ctx, GL_E_ARG, std::string(what) + ": GL_DEVICE buffer is not " + std::to_string(align) +
+                                   "-byte aligned (device buffers of 16 bytes or more need 16-byte alignment)");
+}
+
 // caller buffer -> device pointer (no copy when the caller already is on the device)
 static int stage_in(gl_ctx* ctx, const void* src, size_t bytes, int space, int slot, const u64** out) {
     if (space == GL_DEVICE) {
@@ -798,6 +810,7 @@ extern "C" void gl_host_free(void* p) {
 extern "C" int gl_poseidon_permute_batch(gl_ctx* ctx, uint64_t* states, uint64_t m, int space) {
     if (!ctx) return GL_E_ARG;
     if (m && !states) return fail(ctx, GL_E_ARG, "gl_poseidon_permute_batch: NULL states");
+    TRY(check_device_ptr(ctx, space, states, m * 96, "gl_poseidon_permute_batch: states"));
     Guard g(ctx);
     const u64* d;
     TRY(stage_in(ctx, states, m * 96, space, 0, &d));
@@ -826,6 +839,9 @@ extern "C" int gl_poseidon_two_to_one_batch(gl_ctx* ctx, const uint64_t* l, cons
                                             uint64_t m, int space) {
     if (!ctx) return GL_E_ARG;
     if (m && (!l || !r || !out)) return fail(ctx, GL_E_ARG, "gl_poseidon_two_to_one_batch: NULL buffer");
+    TRY(check_device_ptr(ctx, space, l, m * 32, "gl_poseidon_two_to_one_batch: l"));
+    TRY(check_device_ptr(ctx, space, r, m * 32, "gl_poseidon_two_to_one_batch: r"));
+    TRY(check_device_ptr(ctx, space, out, m * 32, "gl_poseidon_two_to_one_batch: out"));
     Guard g(ctx);
     const u64 *dl, *dr;
     TRY(stage_in(ctx, l, m * 32, space, 0, &dl));
@@ -845,6 +861,8 @@ extern "C" int gl_poseidon_hash_no_pad_batch(gl_ctx* ctx, const uint64_t* in, ui
                                              uint64_t* out, int space) {
     if (!ctx) return GL_E_ARG;
     if (m && (!out || (len_each && !in))) return fail(ctx, GL_E_ARG, "gl_poseidon_hash_no_pad_batch: NULL buffer");
+    TRY(check_device_ptr(ctx, space, in, (size_t)m * len_each * 8, "gl_poseidon_hash_no_pad_batch: in"));
+    TRY(check_device_ptr(ctx, space, out, m * 32, "gl_poseidon_hash_no_pad_batch: out"));
     Guard g(ctx);
     const u64* din;
     TRY(stage_in(ctx, in, (size_t)m * len_each * 8, space, 0, &din));
@@ -863,6 +881,9 @@ extern "C" int gl_smt_leaf_hash_batch(gl_ctx* ctx, const uint64_t* keys, const u
                                       uint64_t m, int space) {
     if (!ctx) return GL_E_ARG;
     if (m && (!keys || !values || !out)) return fail(ctx, GL_E_ARG, "gl_smt_leaf_hash_batch: NULL buffer");
+    TRY(check_device_ptr(ctx, space, keys, m * 32, "gl_smt_leaf_hash_batch: keys"));
+    TRY(check_device_ptr(ctx, space, values, m * 32, "gl_smt_leaf_hash_batch: values"));
+    TRY(check_device_ptr(ctx, space, out, m * 32, "gl_smt_leaf_hash_batch: out"));
     Guard g(ctx);
     const u64 *dk, *dv;
     TRY(stage_in(ctx, keys, m * 32, space, 0, &dk));
@@ -883,6 +904,11 @@ extern "C" int gl_smt_verify_process_batch(gl_ctx* ctx, const gl_smt_proof_hdr* 
     if (!ctx) return GL_E_ARG;
     if (m == 0) return GL_OK;
     if (!proofs || !sib_off || !status) return fail(ctx, GL_E_ARG, "gl_smt_verify_process_batch: NULL buffer");
+    TRY(check_device_ptr(ctx, space, proofs, m * sizeof(gl_smt_proof_hdr), "gl_smt_verify_process_batch: proofs"));
+    // the pool's length is sib_off[m], which lies on the device: any non-empty pool holds 32-byte siblings
+    TRY(check_device_ptr(ctx, space, sib_pool, 32, "gl_smt_verify_process_batch: sib_pool"));
+    TRY(check_device_ptr(ctx, space, sib_off, (m + 1) * 8, "gl_smt_verify_process_batch: sib_off"));
+    TRY(check_device_ptr(ctx, space, status, m * 4, "gl_smt_verify_process_batch: status"));
     Guard g(ctx);
     if (space == GL_DEVICE) {
         launch_smt_verify_process(proofs, sib_pool, sib_off, m, status, ctx->stream);
@@ -912,6 +938,11 @@ extern "C" int gl_smt_build(gl_ctx* ctx, const uint64_t* keys, const uint64_t* v
     if (!ctx) return GL_E_ARG;
     if (!root_out || (m && (!keys || !values))) return fail(ctx, GL_E_ARG, "gl_smt_build: NULL buffer");
     if (m >= ((uint64_t)1 << 31)) return fail(ctx, GL_E_ARG, "gl_smt_build: at most 2^31 - 1 entries");
+    TRY(check_device_ptr(ctx, space, keys, m * 32, "gl_smt_build: keys"));
+    TRY(check_device_ptr(ctx, space, values, m * 32, "gl_smt_build: values"));
+    TRY(check_device_ptr(ctx, space, root_out, 32, "gl_smt_build: root_out"));
+    TRY(check_device_ptr(ctx, space, nodes_out, nodes_cap * 96, "gl_smt_build: nodes_out"));
+    TRY(check_device_ptr(ctx, space, leaf_hashes_out, m * 32, "gl_smt_build: leaf_hashes_out"));
     Guard g(ctx);
     if (m == 0) {
         if (num_nodes_out) *num_nodes_out = 0;
@@ -1074,6 +1105,11 @@ extern "C" int gl_smt_set_proofs(gl_ctx* ctx, const uint64_t* keys, const uint64
     if (m >= ((uint64_t)1 << 31)) return fail(ctx, GL_E_ARG, "gl_smt_set_proofs: at most 2^31 - 1 entries");
     *num_siblings_out = 0;
     if (m == 0) return GL_OK;
+    TRY(check_device_ptr(ctx, space, keys, m * 32, "gl_smt_set_proofs: keys"));
+    TRY(check_device_ptr(ctx, space, values, m * 32, "gl_smt_set_proofs: values"));
+    TRY(check_device_ptr(ctx, space, proofs_out, m * sizeof(gl_smt_proof_hdr), "gl_smt_set_proofs: proofs_out"));
+    TRY(check_device_ptr(ctx, space, sib_pool_out, sib_cap * 32, "gl_smt_set_proofs: sib_pool_out"));
+    TRY(check_device_ptr(ctx, space, sib_off_out, (m + 1) * 8, "gl_smt_set_proofs: sib_off_out"));
     Guard g(ctx);
     const u64 *dk, *dv;
     TRY(stage_in(ctx, keys, m * 32, space, 0, &dk));
@@ -1092,6 +1128,12 @@ extern "C" int gl_smt_find_batch(gl_ctx* ctx, const uint64_t* keys, const uint64
     if (m + nq >= ((uint64_t)1 << 31)) return fail(ctx, GL_E_ARG, "gl_smt_find_batch: at most 2^31 - 1 entries and queries");
     *num_siblings_out = 0;
     if (nq == 0) return GL_OK;
+    TRY(check_device_ptr(ctx, space, keys, m * 32, "gl_smt_find_batch: keys"));
+    TRY(check_device_ptr(ctx, space, values, m * 32, "gl_smt_find_batch: values"));
+    TRY(check_device_ptr(ctx, space, queries, nq * 32, "gl_smt_find_batch: queries"));
+    TRY(check_device_ptr(ctx, space, proofs_out, nq * sizeof(gl_smt_inclusion_hdr), "gl_smt_find_batch: proofs_out"));
+    TRY(check_device_ptr(ctx, space, sib_pool_out, sib_cap * 32, "gl_smt_find_batch: sib_pool_out"));
+    TRY(check_device_ptr(ctx, space, sib_off_out, (nq + 1) * 8, "gl_smt_find_batch: sib_off_out"));
     Guard g(ctx);
     // one event list on the device: the sets, then the queries (their values are not looked at)
     const uint64_t all = m + nq;
@@ -1119,6 +1161,11 @@ extern "C" int gl_merkle_verify_batch(gl_ctx* ctx, const uint64_t* leaves, uint3
         return fail(ctx, GL_E_ARG, "gl_merkle_verify_batch: NULL buffer");
     if (leaf_len == 0 || cap_height > 30 || path_len > 64) return fail(ctx, GL_E_ARG, "gl_merkle_verify_batch: bad shape");
     if (k == 0) return GL_OK;
+    TRY(check_device_ptr(ctx, space, leaves, k * leaf_len * 8, "gl_merkle_verify_batch: leaves"));
+    TRY(check_device_ptr(ctx, space, leaf_indices, k * 8, "gl_merkle_verify_batch: leaf_indices"));
+    TRY(check_device_ptr(ctx, space, paths, k * (size_t)path_len * 32, "gl_merkle_verify_batch: paths"));
+    TRY(check_device_ptr(ctx, space, cap, ((size_t)32) << cap_height, "gl_merkle_verify_batch: cap"));
+    TRY(check_device_ptr(ctx, space, ok, k * 4, "gl_merkle_verify_batch: ok"));
     Guard g(ctx);
     const u64 *dl, *di, *dp, *dc;
     TRY(stage_in(ctx, leaves, k * leaf_len * 8, space, 0, &dl));
@@ -1147,6 +1194,9 @@ extern "C" int gl_merkle_build(gl_ctx* ctx, const uint64_t* leaves, uint64_t num
     if (cap_height > lg)
         return fail(ctx, GL_E_ARG, "MerkleTree::new: cap_height must be at most log2(leaves.len())");
     if (!cap_out || (leaf_len && !leaves)) return fail(ctx, GL_E_ARG, "gl_merkle_build: NULL buffer");
+    TRY(check_device_ptr(ctx, space, leaves, (size_t)num_leaves * leaf_len * 8, "gl_merkle_build: leaves"));
+    TRY(check_device_ptr(ctx, space, digests_out, 2 * (num_leaves - ((uint64_t)1 << cap_height)) * 32, "gl_merkle_build: digests_out"));
+    TRY(check_device_ptr(ctx, space, cap_out, ((size_t)32 << cap_height), "gl_merkle_build: cap_out"));
     Guard g(ctx);
     const u64* dl;
     TRY(stage_in(ctx, leaves, (size_t)num_leaves * leaf_len * 8, space, 0, &dl));
@@ -1169,8 +1219,9 @@ static int fft_entry(gl_ctx* ctx, uint64_t* data, uint32_t log_n, uint32_t c, in
     if (log_n > 30) return fail(ctx, GL_E_ARG, std::string(name) + ": log_n > 30 not supported");
     if (c == 0) return GL_OK;
     if (!data) return fail(ctx, GL_E_ARG, std::string(name) + ": NULL data");
-    Guard g(ctx);
     size_t bytes = ((size_t)c << log_n) * 8;
+    TRY(check_device_ptr(ctx, space, data, bytes, (std::string(name) + ": data").c_str()));
+    Guard g(ctx);
     const u64* d;
     TRY(stage_in(ctx, data, bytes, space, 0, &d));
     const u64 *pre = nullptr, *post = nullptr;
@@ -1448,6 +1499,12 @@ static int commit_common(gl_ctx* ctx, const HostCols& input, bool is_values, uin
     if (!ctx) return GL_E_ARG;
     if (!handle || !input) return fail(ctx, GL_E_ARG, std::string(name) + ": NULL argument");
     *handle = nullptr;
+    TRY(commit_check(ctx, log_n, c, rate_bits, cap_height, name));   // the buffer sizes below need a valid geometry
+    const size_t bytes = ((size_t)c << log_n) * 8;
+    const std::string nm(name);
+    TRY(check_device_ptr(ctx, space, input.flat, bytes, (nm + (is_values ? ": values" : ": coeffs")).c_str()));
+    TRY(check_device_ptr(ctx, space, coeffs_out.flat, bytes, (nm + ": coeffs_out").c_str()));
+    TRY(check_device_ptr(ctx, space, cap_out, (size_t)32 << cap_height, (nm + ": cap_out").c_str()));
     Guard g(ctx);
     std::unique_ptr<gl_commit> h;
     TRY(commit_make(ctx, input, is_values, log_n, c, rate_bits, cap_height, coeffs_out, cap_out, space, name, blinding, &h));
@@ -1560,8 +1617,9 @@ extern "C" int gl_commit_add_coeffs(gl_commit* h, uint32_t col0, uint32_t ncols,
     gl_ctx* ctx = h->ctx;
     if (h->finished) return fail(ctx, GL_E_STATE, "gl_commit_add_coeffs: the commit is already finished");
     if (!coeffs || ncols == 0 || col0 + (uint64_t)ncols > h->c) return fail(ctx, GL_E_ARG, "gl_commit_add_coeffs: bad column range");
-    Guard g(ctx);
     const u64 n = (u64)1 << h->log_n;
+    TRY(check_device_ptr(ctx, space, coeffs, (size_t)ncols * n * 8, "gl_commit_add_coeffs: coeffs"));
+    Guard g(ctx);
     CK(cudaMemcpyAsync(h->coeffs.get() + (size_t)col0 * n, coeffs, (size_t)ncols * n * 8,
                        space == GL_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, ctx->stream));
     TRY(commit_lde_columns(ctx, h, col0, ncols));
@@ -1574,6 +1632,7 @@ extern "C" int gl_commit_finish(gl_commit* h, uint64_t* cap_out, int space) {
     gl_ctx* ctx = h->ctx;
     if (h->finished) return fail(ctx, GL_E_STATE, "gl_commit_finish: the commit is already finished");
     if (h->cols_added != h->c) return fail(ctx, GL_E_STATE, "gl_commit_finish: not every polynomial has been added");
+    TRY(check_device_ptr(ctx, space, cap_out, (size_t)32 << h->cap_height, "gl_commit_finish: cap_out"));
     Guard g(ctx);
     TRY(commit_tree(ctx, h, cap_out, space, h->stream_hash && h->hashed_cols == h->c));
     TRY(finish(ctx));
@@ -1615,6 +1674,7 @@ extern "C" int gl_commit_coeffs(gl_commit* h, uint64_t* coeffs_out, int space) {
     if (!h || !coeffs_out) return GL_E_ARG;
     gl_ctx* ctx = h->ctx;
     if (!h->coeffs.get()) return fail(ctx, GL_E_STATE, "gl_commit_coeffs: this handle has no polynomials (FRI layer tree)");
+    TRY(check_device_ptr(ctx, space, coeffs_out, ((size_t)h->c << h->log_n) * 8, "gl_commit_coeffs: coeffs_out"));
     Guard g(ctx);
     TRY(copy_out(ctx, coeffs_out, h->coeffs.get(), ((size_t)h->c << h->log_n) * 8, space));
     return finish(ctx);
@@ -1643,6 +1703,7 @@ extern "C" int gl_commit_eval(gl_commit* h, const uint64_t point[2], uint64_t* v
     gl_ctx* ctx = h->ctx;
     if (!h->coeffs.get()) return fail(ctx, GL_E_STATE, "gl_commit_eval: this handle has no polynomials (FRI layer tree)");
     if (!h->finished && h->cols_added != h->c) return fail(ctx, GL_E_STATE, "gl_commit_eval: not every polynomial has been added");
+    TRY(check_device_ptr(ctx, space, values_out, (size_t)h->c * 16, "gl_commit_eval: values_out"));
     Guard g(ctx);
     TRY(commit_eval(ctx, h, 0, h->c, point, values_out, space));
     return finish(ctx);
@@ -1652,6 +1713,8 @@ extern "C" int gl_commit_download(gl_commit* h, uint64_t* leaves_out, uint64_t* 
     if (!h) return GL_E_ARG;
     gl_ctx* ctx = h->ctx;
     if (!h->finished) return fail(ctx, GL_E_STATE, "gl_commit_download: gl_commit_finish has not run yet");
+    TRY(check_device_ptr(ctx, space, leaves_out, (size_t)h->n_local * leaf_len(h) * 8, "gl_commit_download: leaves_out"));
+    TRY(check_device_ptr(ctx, space, digests_out, h->num_digests * 32, "gl_commit_download: digests_out"));
     Guard g(ctx);
     if (digests_out) TRY(copy_out(ctx, digests_out, h->digests.get(), h->num_digests * 32, space));
     if (leaves_out) {
@@ -1700,6 +1763,10 @@ extern "C" int gl_commit_open(gl_commit* h, const uint64_t* leaf_indices, uint32
     if (!h->finished) return fail(ctx, GL_E_STATE, "gl_commit_open: gl_commit_finish has not run yet");
     if (k == 0) return GL_OK;
     if (!leaf_indices) return fail(ctx, GL_E_ARG, "gl_commit_open: NULL indices");
+    const unsigned sub_bits = h->log_n + h->rate_bits - h->cap_height;
+    TRY(check_device_ptr(ctx, space, leaf_indices, (size_t)k * 8, "gl_commit_open: leaf_indices"));
+    TRY(check_device_ptr(ctx, space, rows_out, (size_t)k * leaf_len(h) * 8, "gl_commit_open: rows_out"));
+    TRY(check_device_ptr(ctx, space, paths_out, (size_t)k * sub_bits * 32, "gl_commit_open: paths_out"));
     Guard g(ctx);
     std::vector<u64> idx;
     TRY(fetch_indices(ctx, leaf_indices, k, space, idx));
@@ -1710,7 +1777,6 @@ extern "C" int gl_commit_open(gl_commit* h, const uint64_t* leaf_indices, uint32
     }
     const u64* d_idx;
     TRY(upload_indices(ctx, h, idx, &d_idx));
-    const unsigned sub_bits = h->log_n + h->rate_bits - h->cap_height;
     if (rows_out) {
         u64* d_rows = rows_out;
         if (space == GL_HOST) {
@@ -1741,6 +1807,8 @@ extern "C" int gl_commit_get_lde_values(gl_commit* h, const uint64_t* indices, u
     if (!h->finished) return fail(ctx, GL_E_STATE, "gl_commit_get_lde_values: gl_commit_finish has not run yet");
     if (k == 0) return GL_OK;
     if (!indices || !rows_out) return fail(ctx, GL_E_ARG, "gl_commit_get_lde_values: NULL buffer");
+    TRY(check_device_ptr(ctx, space, indices, (size_t)k * 8, "gl_commit_get_lde_values: indices"));
+    TRY(check_device_ptr(ctx, space, rows_out, (size_t)k * h->c * 8, "gl_commit_get_lde_values: rows_out"));
     Guard g(ctx);
     std::vector<u64> idx;
     TRY(fetch_indices(ctx, indices, k, space, idx));
@@ -1778,6 +1846,10 @@ extern "C" int gl_fri_layer_tree(gl_ctx* ctx, const uint64_t* values_ext, uint64
     if (cap_height > lg - arity_bits)
         return fail(ctx, GL_E_ARG, "MerkleTree::new: cap_height must be at most log2(leaves.len())");
     if (!values_ext || !cap_out) return fail(ctx, GL_E_ARG, "gl_fri_layer_tree: NULL buffer");
+    TRY(check_device_ptr(ctx, space, values_ext, len * 16, "gl_fri_layer_tree: values_ext"));
+    TRY(check_device_ptr(ctx, space, digests_out, 2 * ((len >> arity_bits) - ((uint64_t)1 << cap_height)) * 32,
+                         "gl_fri_layer_tree: digests_out"));
+    TRY(check_device_ptr(ctx, space, cap_out, (size_t)32 << cap_height, "gl_fri_layer_tree: cap_out"));
     Guard g(ctx);
     const u64* dv;
     TRY(stage_in(ctx, values_ext, len * 16, space, 0, &dv));
@@ -1824,6 +1896,8 @@ extern "C" int gl_fri_layer_commit(gl_ctx* ctx, const uint64_t* values_ext, uint
     if (cap_height > lg - arity_bits)
         return fail(ctx, GL_E_ARG, "MerkleTree::new: cap_height must be at most log2(leaves.len())");
     if (!values_ext) return fail(ctx, GL_E_ARG, "gl_fri_layer_commit: NULL buffer");
+    TRY(check_device_ptr(ctx, space, values_ext, len * 16, "gl_fri_layer_commit: values_ext"));
+    TRY(check_device_ptr(ctx, space, cap_out, (size_t)32 << cap_height, "gl_fri_layer_commit: cap_out"));
     Guard g(ctx);
     const u64* dv;
     TRY(stage_in(ctx, values_ext, len * 16, space, 0, &dv));
@@ -1843,6 +1917,9 @@ extern "C" int gl_fri_fold(gl_ctx* ctx, const uint64_t* coeffs_ext, uint64_t len
     unsigned lg = ilog2(len);
     if (arity_bits > lg) return fail(ctx, GL_E_ARG, "fri fold: arity larger than the polynomial");
     if (!coeffs_ext || !beta) return fail(ctx, GL_E_ARG, "gl_fri_fold: NULL buffer");
+    TRY(check_device_ptr(ctx, space, coeffs_ext, len * 16, "gl_fri_fold: coeffs_ext"));
+    TRY(check_device_ptr(ctx, space, folded_coeffs_out, (len >> arity_bits) * 16, "gl_fri_fold: folded_coeffs_out"));
+    TRY(check_device_ptr(ctx, space, next_values_out, (len >> arity_bits) * 16, "gl_fri_fold: next_values_out"));
     Guard g(ctx);
     const u64* dcf;
     TRY(stage_in(ctx, coeffs_ext, len * 16, space, 0, &dcf));
@@ -1950,6 +2027,9 @@ extern "C" int gl_fri_final_poly(gl_ctx* ctx, gl_commit* const* oracles, uint32_
                                  uint32_t num_batches, const gl_fri_poly* polys, const uint64_t alpha[2],
                                  uint32_t rate_bits, uint64_t* lde_coeffs_out, uint64_t* lde_values_out, int space) {
     if (!ctx) return GL_E_ARG;
+    // both outputs are [N][2] extension elements, N >= 1: 16 bytes at least
+    TRY(check_device_ptr(ctx, space, lde_coeffs_out, 16, "gl_fri_final_poly: lde_coeffs_out"));
+    TRY(check_device_ptr(ctx, space, lde_values_out, 16, "gl_fri_final_poly: lde_values_out"));
     Guard g(ctx);
     u64 *dc, *dv;
     TRY(fri_final_poly_device(ctx, oracles, num_oracles, batches, num_batches, polys, alpha, rate_bits,
@@ -2239,6 +2319,7 @@ static int quotient_polys(gl_ctx* ctx, const gl_circuit* cd, const gl_gate* gate
         ngc = std::max(ngc, quotient_gate_constraints(g));
     }
     const u64 n = (u64)1 << lg_n, lde_size = n << qdb;
+    TRY(check_device_ptr(ctx, space, chunks_out, (size_t)nch * lde_size * 8, "gl_quotient_polys: chunks_out"));
     const uint32_t nterms = nch * (1 + chunks) + ngc;
     // tables: alpha powers [nch][nterms], k_is [R]
     std::vector<u64> tab((size_t)nch * nterms + R);
@@ -2330,6 +2411,8 @@ static int permutation_zs(gl_ctx* ctx, const gl_circuit* cd, const uint64_t* k_i
         return fail(ctx, GL_E_ARG, "gl_permutation_zs: oracles of different degree");
     const uint32_t lg_n = cd->degree_bits;
     const u64 n = (u64)1 << lg_n;
+    const size_t out_bytes = (size_t)nch * chunks * n * 8;
+    TRY(check_device_ptr(ctx, space, zs_partial_products_out, out_bytes, "gl_permutation_zs: zs_partial_products_out"));
     const uint32_t nblocks = (uint32_t)((n + PERM_BLOCK - 1) / PERM_BLOCK);
     // small device state (scratch slot 0): k_is [R] | CTA products [nch][nblocks] | grand products [4] | zero flag
     std::vector<u64> kt(R);
@@ -2346,7 +2429,6 @@ static int permutation_zs(gl_ctx* ctx, const gl_circuit* cd, const uint64_t* k_i
     const u64* xtab;
     TRY(pow_table(ctx, glh::root_of_unity(lg_n), &xtab));
     void* d_out = zs_partial_products_out;
-    const size_t out_bytes = (size_t)nch * chunks * n * 8;
     if (space == GL_HOST) TRY(scratch_get(ctx, 4, out_bytes, &d_out));
     // the routed wire and sigma values: forward transforms of the coefficient columns (the salt of a blinded commit
     // lives only in its leaves).  The transforms run through scratch slot 1.
@@ -2537,6 +2619,7 @@ extern "C" int gl_prove(gl_ctx* ctx, const gl_circuit* cd, const gl_gate* gates,
     const uint64_t total = 3 * (4ull << prm->cap_height) + 2ull * (cs->c + cd->num_wires + 2 * nch + (zcols - nch) + qcols) + fri_words;
     *proof_words_out = total;
     if (!proof_out || proof_cap_words < total) return fail(ctx, GL_E_ARG, "gl_prove: proof buffer too small (see *proof_words_out)");
+    TRY(check_device_ptr(ctx, space, wires, ((size_t)cd->num_wires << cd->degree_bits) * 8, "gl_prove: wires"));
     Guard g(ctx);
     HostCols witness;
     witness.flat = const_cast<uint64_t*>(wires);

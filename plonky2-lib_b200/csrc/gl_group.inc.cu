@@ -551,6 +551,11 @@ static int group_commit(gl_group* g, const uint64_t* const* inputs, bool is_valu
         if (!inputs[i]) return gfail(g, GL_E_ARG, std::string(name) + ": NULL polynomials");
         gl_ctx* ctx = g->r[i].ctx;
         GTRY(g, ctx, commit_check(ctx, log_n, c, rate_bits, cap_height, name));
+        const std::string nm(name), rank = "[" + std::to_string(i) + "]";
+        const size_t bytes = ((size_t)c << log_n) * 8;
+        GTRY(g, ctx, check_device_ptr(ctx, space, inputs[i], bytes, (nm + (is_values ? ": values" : ": coeffs") + rank).c_str()));
+        if (coeffs_out) GTRY(g, ctx, check_device_ptr(ctx, space, coeffs_out[i], bytes, (nm + ": coeffs_out" + rank).c_str()));
+        if (cap_out) GTRY(g, ctx, check_device_ptr(ctx, space, cap_out[i], (size_t)32 << cap_height, (nm + ": cap_out" + rank).c_str()));
     }
     const u64 n = (u64)1 << log_n;
     const GroupPlan plan = group_plan(c, G);
